@@ -2,6 +2,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # our arm (CUDA path through the C ABI)
     python bench.py --impl reference --steps K --warmup W    # the reference's CPU path (torch.stft) on the host cores
+    python bench.py --steps K --dump-outputs bench_outputs   # also write the last timed step's features (see dump_outputs)
 
 Workload at every N: BASELINE.json configs[1] -- a batch of 256 x 30 s synthetic 16 kHz clips per GPU ->
 scalar-normalised log-mel fp32 [256, 80, 1876].  A "step" is one pass of the fused kernel over one batch; at N > 1 every
@@ -247,6 +248,25 @@ def pin_to_gpu_cpus(local_rank: int, world_local: int):
     return info
 
 
+DUMP_BYTES = 64 * 10**6          # cap on what --dump-outputs writes, .npy header included
+
+
+def dump_outputs(out: torch.Tensor, directory: str) -> dict:
+    """Writes the features the timed path returned in its last step as ``directory/logmel.npy`` (float32, [k, n_mels, T]), so that two
+    builds run with the same arguments (hence the same seeded inputs) can be compared output for output.  When the whole batch is larger
+    than DUMP_BYTES, k clips drawn by a fixed seed stand for it, in batch order; their batch indices are returned with the file's shape."""
+    B = out.shape[0]
+    per_clip = out[0].numel() * 4
+    keep = min(B, (DUMP_BYTES - 4096) // per_clip)                 # 4096: room for the .npy header
+    if keep < 1:
+        raise ValueError(f"--dump-outputs: one clip's features ({per_clip} bytes) exceed the {DUMP_BYTES}-byte cap")
+    clips = np.arange(B) if keep == B else np.sort(np.random.default_rng(0).choice(B, size=keep, replace=False))
+    sample = out[torch.from_numpy(clips).to(out.device)].float().cpu().numpy()
+    os.makedirs(directory, exist_ok=True)
+    np.save(os.path.join(directory, "logmel.npy"), sample)
+    return {"dir": directory, "files": {"logmel.npy": list(sample.shape)}, "clips": clips.tolist()}
+
+
 def max_over_ranks(dist, value: float, device) -> float:
     if dist is None:
         return value
@@ -378,8 +398,14 @@ def main() -> None:
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip config1 / config4 / the Whisper-style preset")
     ap.add_argument("--no-whisper", action="store_true", help="skip the extra line of the tensor-core route (Whisper-style preset)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write rank 0's features of the last step to DIR/logmel.npy (float32, <= 64 MB)")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 0)
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the CUDA path's features; the reference arm has none to write")
 
     if args.impl == "reference":
         run_reference(args)
@@ -441,6 +467,7 @@ def main() -> None:
     clocks = sampler.stop()
     fe.check()
     launches = fe.launches - launches0
+    dumped = dump_outputs(out, args.dump_outputs) if args.dump_outputs and rank == 0 else None   # before e2e reuses `out` as staging
     total_ms = max_over_ranks(dist, t_start.elapsed_time(t_end), device)
     kernel_ms = float(np.mean([a.elapsed_time(b) for a, b in ev]))
     audio_s_per_step = B * args.seconds * world
@@ -619,6 +646,8 @@ def main() -> None:
             "sustained": sustained, "sustained_ms_per_step": None if sustained is None else sustained["ms_per_step"],
             "stats_pass": stats, "config1": config1, "config4": config4, "whisper_preset": whisper,
         }
+        if dumped is not None:
+            line["outputs"] = dumped
         sys.stdout.flush()
         os.write(json_fd, (json.dumps(line) + "\n").encode())
     if dist is not None:

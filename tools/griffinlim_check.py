@@ -1,12 +1,13 @@
 import numpy as np, torch, sys
-sys.path.insert(0,'/root/repo')
 import os
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT)
 import audio_calm_b200 as _acb
 if os.environ.get("ACB_LIB"):
     _acb._lib.LIB_PATH = os.environ["ACB_LIB"]
 from audio_calm_b200 import spectral
 from oracle import spectral_oracle as so
-g=np.load('/root/repo/tests/golden/griffinlim_cases.npz')
+g=np.load(os.path.join(ROOT, 'tests', 'golden', 'griffinlim_cases.npz'))
 init=torch.from_numpy(g["init_angles"]).cuda(); mag=torch.from_numpy(g["mag"]).cuda()
 for n in (2,8,32):
     w=spectral.griffin_lim(mag,n_iter=n,init_angles=init).cpu().numpy()
