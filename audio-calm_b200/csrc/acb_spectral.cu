@@ -398,10 +398,22 @@ __global__ void __launch_bounds__(kThreads) stft_mag_backward_kernel(const float
         const int row_a = valid ? qa / n_frames : 0, fa = valid ? qa - row_a * n_frames : 0;
         const int row_b = valid_b ? qb / n_frames : 0, fb = valid_b ? qb - row_b * n_frames : 0;
         float2 pr[16], pi[16];
+        bool live_a = false, live_b = false;            // this lane holds a nonzero windowed sample of frame a / b
         if (valid) {                                    // forward transform of the pair, as in stft_mag_kernel
             load_pair_windowed<R>(s_x, row_a * T + fa * hop, row_b * T + fb * hop, valid_b, blocked, r, wreg, pr, pi);
+#pragma unroll
+            for (int q = 0; q < 16; ++q) {
+                live_a |= pr[q].x != 0.f || pr[q].y != 0.f;
+                live_b |= pi[q].x != 0.f || pi[q].y != 0.f;
+            }
             group_fft_stage1<R>(pr, pi, buf, s_tw, r);
         }
+        // A silent frame (every windowed sample 0) has X = 0 exactly and passes no gradient, as in torch.  Packed with a sounding
+        // frame, the separation below leaves that frame's rounding noise in its X instead, and g conj(X) / |X| of noise is a
+        // unit-sized direction: such a frame is zeroed by the group's vote rather than by |X| = 0.
+        const unsigned group_bits = (R == 32 ? 0xffffffffu : (1u << (R & 31)) - 1u) << ((tid & 31) & ~(R - 1));
+        const bool silent_a = (__ballot_sync(0xffffffffu, live_a) & group_bits) == 0u;
+        const bool silent_b = (__ballot_sync(0xffffffffu, live_b) & group_bits) == 0u;
         __syncwarp();
         if (valid) group_fft_stage2<R>(buf, r);
         __syncwarp();
@@ -414,8 +426,8 @@ __global__ void __launch_bounds__(kThreads) stft_mag_backward_kernel(const float
                 const float xar = 0.5f * (z.x + zc.x), xai = 0.5f * (z.y - zc.y);          // X_A[k]
                 const float xbr = 0.5f * (z.y + zc.y), xbi = -0.5f * (z.x - zc.x);         // X_B[k]
                 const float pa = fmaf(xar, xar, xai * xai), pb = fmaf(xbr, xbr, xbi * xbi);   // |X|^2; g / |X| = g * rsqrt(|X|^2)
-                const float sa = pa > 0.f ? ga[(size_t)k * n_frames] * rsqrtf(pa) : 0.f;
-                const float sb = (valid_b && pb > 0.f) ? gb[(size_t)k * n_frames] * rsqrtf(pb) : 0.f;
+                const float sa = (!silent_a && pa > 0.f) ? ga[(size_t)k * n_frames] * rsqrtf(pa) : 0.f;
+                const float sb = (valid_b && !silent_b && pb > 0.f) ? gb[(size_t)k * n_frames] * rsqrtf(pb) : 0.f;
                 const float har = sa * xar, hai = -sa * xai;                                // h_A = g conj(X_A) / |X_A|
                 const float hbr = sb * xbr, hbi = -sb * xbi;
                 if (k == 0 || 2 * k == N) {
@@ -441,13 +453,14 @@ __global__ void __launch_bounds__(kThreads) stft_mag_backward_kernel(const float
         __syncwarp();
         if (valid) group_fft_stage2<R>(buf, r);
         __syncwarp();
-        if (valid) {                                    // windowed overlap-add into the rows' gradients
+        if (valid) {                                    // windowed overlap-add into the rows' gradients (a silent frame adds exactly 0,
+                                                        // not the partner's rounding noise in its half of the transform)
             const int base_a = row_a * T + fa * hop, base_b = row_b * T + fb * hop;
             for (int n = r; n < N; n += R) {
                 const float2 y = buf[buf_index(n)];
                 const float w = s_win[n];
-                atomicAdd(s_gx + Swz<R>::at(base_a + n), w * y.x);
-                if (valid_b) atomicAdd(s_gx + Swz<R>::at(base_b + n), w * y.y);
+                if (!silent_a) atomicAdd(s_gx + Swz<R>::at(base_a + n), w * y.x);
+                if (valid_b && !silent_b) atomicAdd(s_gx + Swz<R>::at(base_b + n), w * y.y);
             }
         }
         __syncwarp();

@@ -165,6 +165,11 @@ def griffin_lim(specgram: torch.Tensor, n_fft: int = 1024, hop_length: Optional[
     else:
         angles = torch.ones(mag.shape, dtype=torch.complex64, device=mag.device)
     L = int(length) if length is not None else hop * (frames - 1)
+    if 1 + L // hop != frames:
+        # every iteration re-analyses the L-sample estimate into 1 + L // hop frames; torchaudio fails on the shape mismatch, and the
+        # complex STFT here would write a spectrum of another shape over `spec`
+        raise ValueError(f"griffin_lim: length {L} gives {1 + L // hop} frames at hop {hop}, the spectrogram has {frames} "
+                         f"(length must lie in [{hop * (frames - 1)}, {hop * frames}))")
     spec = (mag * angles).contiguous()
     prev = torch.zeros_like(spec)
     wave = torch.empty((rows, L), dtype=torch.float32, device=mag.device)

@@ -96,9 +96,28 @@ def test_training_batch_size():
         assert float(((got - ref).abs() / ref.abs().clamp(min=1.0)).max()) < 1e-4
 
 
+@pytest.mark.parametrize("n_fft,hop,T", [(64, 16, 272), (128, 32, 300), (256, 64, 700), (512, 100, 1500), (1024, 256, 2048)])
+def test_oracle_adjoint_matches_float64_autograd(n_fft, hop, T):
+    """The fp64 adjoint of the oracle against torch autograd through torch.stft(center=False).abs() in float64 on the CPU, with an
+    all-zero first frame (|X| = 0 at every bin: both pass no gradient there)."""
+    rng = np.random.default_rng(n_fft + T)
+    x = rng.normal(-6.0, 3.0, (2, 3, T))
+    x[0, 0, :n_fft] = 0.0
+    frames = 1 + (T - n_fft) // hop
+    up = rng.normal(0.0, 1.0, (2, 3, n_fft // 2 + 1, frames))
+    xt = torch.from_numpy(x).requires_grad_(True)
+    X = torch.stft(xt.reshape(-1, T), n_fft=n_fft, hop_length=hop, win_length=n_fft, window=torch.hann_window(n_fft, dtype=torch.float64),
+                   return_complex=True, normalized=False, center=False)
+    (X.abs().view(up.shape) * torch.from_numpy(up)).sum().backward()
+    ref = xt.grad.numpy()
+    got = so.stft_mag_backward(x, up, n_fft, hop)
+    assert got.shape == ref.shape
+    assert float(np.max(np.abs(got - ref))) < 1e-12 * float(np.max(np.abs(ref))), float(np.max(np.abs(got - ref)))
+
+
 @pytest.mark.gpu
 @pytest.mark.parametrize("n_fft,hop,T", [(64, 16, 256), (128, 32, 256), (256, 64, 256), (256, 64, 700), (512, 128, 777), (64, 7, 100),
-                                         (512, 128, 1024), (64, 16, 272)])
+                                         (512, 128, 1024), (64, 16, 272), (1024, 256, 2048)])
 def test_backward_matches_autograd_through_torch_stft(n_fft, hop, T):
     """The adjoint kernel against torch's own autograd through torch.stft(...).abs() (what stft_loss differentiates in the reference)."""
     g = torch.Generator(device="cuda").manual_seed(n_fft + T)
