@@ -171,9 +171,6 @@ struct LogmelParams {
     const float* bin_std;
     double* moments_partial;   // [gridDim.x * G][2][n_mels] or nullptr
     int* error_flag;           // set to 1 when a sample-tile barrier timed out (results invalid)
-    // warp-specialised variant (logmel_tc_kernel): filterbank blocks for the tensor-core mel projection
-    const float4* tc_w;        // [mel warp][step][lane] (W_hi, W_hi', W_lo, W_lo') of the lane's two fragment elements
-    const int* tc_meta;        // [mel warp][2 + 3 * kTcMaxBlocks]: n_blocks, n_steps, then (steps, first bin, first band) per band block
 };
 
 struct SmemLayout {
@@ -745,359 +742,6 @@ __global__ void __launch_bounds__(G * kGroupThreads, G == 4 ? 1 : 2) logmel_fuse
     }
 }
 
-// --------------------------------------------------------------------------------------------
-// warp-specialised variant: FFT warps + tensor-core mel warps
-// --------------------------------------------------------------------------------------------
-// One 512-thread CTA per SM.  Twelve FFT warps each own one frame pair at a time: private sample buffer (one 5 KB bulk copy per
-// pair), the packed-FFMA2 32 x 32 FFT of the fused kernel above, and the pair's two power spectra written as fp32 planes into a
-// ring of tile slots in shared memory.  Four mel warps (one per SM sub-partition) consume whole 8-frame tiles from the ring and
-// do the banded mel projection on the TENSOR pipe: mma.sync.m16n8k8 TF32 with the filterbank weights resident in registers for
-// the whole kernel.  fp32 accuracy comes from splitting both operands into TF32 pairs (hi = top 19 bits, lo = x - hi): the 16
-// rows of an A fragment are the hi halves (rows 0-7) and the lo halves (rows 8-15) of the tile's 8 frames, so ONE MMA against
-// W_hi yields P_hi W_hi and P_lo W_hi, a second against W_lo the two remaining products; the accumulator rows g and g + 8 of a lane
-// are summed in the epilogue (measured |d ln mel| ~ 2e-7, the same as the fp32 CUDA-core projection).  Each (8 bands x 8 bins)
-// block of the filterbank with a non-zero weight is one step: 79 steps for the 80-band slaney bank, dealt to the four mel warps
-// longest-first.  Every hand-off is an mbarrier (ring slot full / empty, sample tile landed); only the mel warps share a named barrier.
-#if !defined(ACB_DEV) || !defined(ACB_TC_ABLATE)
-#undef ACB_TC_ABLATE
-#define ACB_TC_ABLATE 0      // development (-DACB_DEV): bit 0 = no MMA phase, bit 1 = no epilogue (results are wrong)
-#endif
-#if ACB_TC_ABLATE & 4        // development: FFT warps only (16 of them), nothing consumes the power spectra
-constexpr int kTcFftWarps = 16;
-constexpr int kTcMelLaunched = 0;
-#else
-constexpr int kTcFftWarps = 12;                       // three tiles in flight, four pairs each
-constexpr int kTcMelLaunched = 4;
-#endif
-constexpr int kTcMelWarps = 4;
-constexpr int kTcThreads = (kTcFftWarps + kTcMelLaunched) * 32;
-constexpr int kTcRing = (ACB_TC_ABLATE & 4) ? 2 : 4;  // tile slots of the power ring
-constexpr int kTcPlane = kBins + 8;                   // floats per frame plane: == 8 (mod 32) -> conflict-free 8-byte fragment loads
-constexpr int kTcSlotFloats = kTileFrames * kTcPlane;
-constexpr int kTcPairSamples = kNfft + kHop;          // 1280 samples feed one frame pair
-constexpr int kTcWarpFloats = kPlaneFloats + kTcPairSamples;   // transpose plane A + (sample buffer == transpose plane B)
-constexpr int kTcMaxSteps = 22;                       // (8 bands x 8 bins) weight blocks per mel warp (4 registers per lane each)
-constexpr int kTcMaxBlocks = 8;                       // band blocks per mel warp
-static_assert(kTcPairSamples >= kPlaneFloats, "the sample buffer doubles as the second transpose plane");
-static_assert(kTcFftWarps % 4 == 0, "a warp keeps its pair slot from tile to tile");
-
-// pitch of the staged [frame][band] tile: >= n_mels and == 8 (mod 32), so that the accumulator flush (8-byte stores, lanes =
-// 8 frames x 4 band pairs) is conflict-free and aligned
-__host__ __device__ inline int tc_row_stride(int n_mels) { return n_mels + ((40 - (n_mels & 31)) & 31); }
-
-struct TcSmemLayout {
-    int warp_buf, ring, raw, twiddle, window, affine, meta, mbar, moments, total_bytes;
-};
-
-__host__ __device__ inline TcSmemLayout make_tc_smem_layout(int n_mels, bool with_moments) {
-    TcSmemLayout L;
-    int off = 0;   // 4-byte words
-    L.warp_buf = off; off += kTcFftWarps * kTcWarpFloats;
-    L.ring = off; off += kTcRing * kTcSlotFloats;
-    L.raw = off; off += 2 * kTileFrames * tc_row_stride(n_mels);                        // two staged mel tiles [frame][band]
-    L.twiddle = off; off += 5 * 32 * 4;
-    L.window = off; off += kNfft / 2;
-    L.affine = off; off += 2 * ((n_mels + 1) & ~1);
-    L.meta = off; off += kTcMelWarps * (2 + 3 * kTcMaxBlocks);                          // per mel warp: n_blocks, n_steps, then (steps, first bin, first band) per block
-    off = (off + 3) & ~3;
-    L.mbar = off; off += 2 * (kTcFftWarps + 2 * kTcRing);                               // 8-byte mbarriers: samples[12], full[ring], empty[ring]
-    L.moments = off; if (with_moments) off += 4 * n_mels;                               // float2 [2][n_mels]
-    L.total_bytes = off * 4;
-    return L;
-}
-
-__device__ __forceinline__ void mma_tf32_16x8x8(float (&d)[4], unsigned a0, unsigned a1, unsigned a2, unsigned a3, unsigned b0, unsigned b1) {
-    asm volatile("mma.sync.aligned.m16n8k8.row.col.f32.tf32.tf32.f32 {%0, %1, %2, %3}, {%4, %5, %6, %7}, {%8, %9}, {%0, %1, %2, %3};"
-                 : "+f"(d[0]), "+f"(d[1]), "+f"(d[2]), "+f"(d[3]) : "r"(a0), "r"(a1), "r"(a2), "r"(a3), "r"(b0), "r"(b1));
-}
-
-// Stage the 1280 samples of one frame pair in the warp's buffer; the warp's mbarrier completes a phase when they have landed.
-// Interior pairs are one bulk async copy issued by lane 0; pairs that touch a clip end (reflection) or an unaligned address
-// are gathered by the warp.
-__device__ __forceinline__ void tc_load_pair(const LogmelParams& p, const ClipCursor& t, int pair_slot, float* buf, int lane,
-                                             unsigned long long* bar) {
-    const long long g0 = (long long)(t.tile_in_clip * kTileFrames + 2 * pair_slot) * kHop - kNfft / 2;
-    const float* src = p.wav + t.wav_base;
-    const bool interior = (g0 >= 0) && (g0 + kTcPairSamples <= t.length);
-    if (interior && (reinterpret_cast<uintptr_t>(src + g0) & 15) == 0) {   // warp-uniform
-        if (lane == 0) {
-            asm volatile("fence.proxy.async.shared::cta;" ::: "memory");  // the buffer was read / written through the generic proxy (transpose plane B)
-            mbar_arrive_expect_tx(bar, kTcPairSamples * (unsigned)sizeof(float));
-            bulk_copy_g2s(buf, src + g0, kTcPairSamples * (unsigned)sizeof(float), bar);
-        }
-        return;
-    }
-    float v[kTcPairSamples / 32];
-#pragma unroll
-    for (int k = 0; k < kTcPairSamples / 32; ++k) {
-        long long idx = g0 + lane + 32 * k;
-        if (idx < 0) idx = -idx;
-        if (idx >= t.length) idx = 2 * (t.length - 1) - idx;
-        v[k] = (idx >= 0 && idx < t.length) ? __ldg(src + idx) : 0.f;
-    }
-#pragma unroll
-    for (int k = 0; k < kTcPairSamples / 32; ++k) buf[lane + 32 * k] = v[k];
-    __syncwarp();
-    if (lane == 0) mbar_arrive(bar);
-}
-
-template <bool kMoments, typename OutT>
-__global__ void __launch_bounds__(kTcThreads, 1) logmel_tc_kernel(const LogmelParams p) {
-    extern __shared__ __align__(16) float smem[];
-    const TcSmemLayout L = make_tc_smem_layout(p.n_mels, kMoments);
-    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    const int n_mels = p.n_mels;
-    const int S = tc_row_stride(n_mels);
-    float4* s_tw4 = reinterpret_cast<float4*>(smem + L.twiddle);
-    float* s_win = smem + L.window;
-    float2* s_aff = reinterpret_cast<float2*>(smem + L.affine);
-    int* s_meta = reinterpret_cast<int*>(smem + L.meta);
-    float* s_ring = smem + L.ring;
-    unsigned long long* s_bar = reinterpret_cast<unsigned long long*>(smem + L.mbar);
-    unsigned long long* s_full = s_bar + kTcFftWarps;
-    unsigned long long* s_empty = s_full + kTcRing;
-    float2* s_mom = reinterpret_cast<float2*>(smem + L.moments);
-
-    for (int i = tid; i < 5 * 32; i += kTcThreads) s_tw4[i] = p.twiddle[i];
-    for (int i = tid; i < kNfft / 2; i += kTcThreads) s_win[i] = p.window[i];
-    for (int i = tid; i < kTcMelWarps * (2 + 3 * kTcMaxBlocks); i += kTcThreads) s_meta[i] = p.tc_meta[i];
-    for (int i = tid; i < n_mels; i += kTcThreads) {
-        float sc = 1.f, sh = 0.f;
-        if (p.affine == 1) { sc = p.affine_inv_std; sh = -p.affine_mean * p.affine_inv_std; }
-        else if (p.affine == 2) { sc = 1.f / __ldg(p.bin_std + i); sh = -__ldg(p.bin_mean + i) * sc; }
-        s_aff[i] = make_float2(sc, sh);
-    }
-    if (kMoments)
-        for (int i = tid; i < 2 * n_mels; i += kTcThreads) s_mom[i] = make_float2(0.f, 0.f);
-    if (tid == 0) {
-        for (int i = 0; i < kTcFftWarps; ++i) mbar_init(s_bar + i, 1);
-        for (int i = 0; i < kTcRing; ++i) { mbar_init(s_full + i, 4); mbar_init(s_empty + i, kTcMelWarps); }
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    __syncthreads();
-
-    // this CTA's contiguous tile range
-    const long long t_begin = (long long)p.n_tiles * blockIdx.x / gridDim.x;
-    const int n_local = (int)((long long)p.n_tiles * (blockIdx.x + 1) / gridDim.x - t_begin);
-
-    if (warp >= kTcMelLaunched) {
-        // =========================================== FFT warps ===========================================
-        const int fw = warp - kTcMelLaunched;
-        const int slot_in_tile = fw & 3;              // this warp's frame pair of every tile it visits
-        float* buf_a = smem + L.warp_buf + fw * kTcWarpFloats;        // transpose plane A
-        float* buf_b = buf_a + kPlaneFloats;                            // sample buffer, then transpose plane B
-        unsigned long long* my_bar = s_bar + fw;
-        unsigned parity = 0;
-        int tau = fw >> 2;                            // tile index inside the CTA's range; advances by kTcFftWarps / 4
-        ClipCursor cur;
-        bool staged = false;
-        if (tau < n_local) {
-            cursor_init(p, cur, t_begin + tau);
-            staged = cur.tile_in_clip * kTileFrames + 2 * slot_in_tile < cur.frames;
-            if (staged) tc_load_pair(p, cur, slot_in_tile, buf_b, lane, my_bar);
-        }
-        for (; tau < n_local; tau += kTcFftWarps / 4) {
-            const bool active = staged;
-            float2 pr[16], pi[16];
-            if (active) {
-                if (!mbar_wait(my_bar, parity) && lane == 0) atomicExch(p.error_flag, 1);
-                parity ^= 1;
-                {
-                    const float* sp = buf_b + lane;
-                    float2 v[20];
-#pragma unroll
-                    for (int r = 0; r < 20; ++r) v[r] = make_float2(sp[32 * (2 * r)], sp[32 * (2 * r + 1)]);
-#pragma unroll
-                    for (int j = 0; j < 8; ++j) {
-                        const int t = brev5(2 * j) >> 1;
-                        const float2 wa = make_float2(s_win[32 * (2 * t) + lane], s_win[32 * (2 * t + 1) + lane]);
-                        const float2 wb = __fadd2_rn(bcast2(1.f), neg2(wa));
-                        const float2 ar = __fmul2_rn(v[t], wa), br = __fmul2_rn(v[t + 8], wb);
-                        const float2 ai = __fmul2_rn(v[t + 4], wa), bi = __fmul2_rn(v[t + 12], wb);
-                        pr[2 * j] = __fadd2_rn(ar, br);
-                        pr[2 * j + 1] = __fadd2_rn(ar, neg2(br));
-                        pi[2 * j] = __fadd2_rn(ai, bi);
-                        pi[2 * j + 1] = __fadd2_rn(ai, neg2(bi));
-                    }
-                }
-                __syncwarp();   // every lane has its samples in registers: the sample buffer may now serve as transpose plane B
-                fft32_packed_from_stage2(pr, pi);
-                {
-                    float* pre = buf_a + lane;
-                    float* pim = buf_b + lane;
-                    float2 tr[4], ti[4];
-#pragma unroll
-                    for (int c = 0; c < 4; ++c) {
-                        const float4 sd = s_tw4[c * 32 + lane];
-                        tr[c] = make_float2(sd.x, sd.y);
-                        ti[c] = make_float2(sd.z, sd.w);
-                    }
-                    const float4 w4 = s_tw4[4 * 32 + lane];
-                    const float2 w4r = bcast2(w4.x), w4i = bcast2(w4.y);
-#pragma unroll
-                    for (int k = 0; k < 16; ++k) {
-                        const int c = k & 3;
-                        const float2 yr = __ffma2_rn(neg2(pi[k]), ti[c], __fmul2_rn(pr[k], tr[c]));
-                        const float2 yi = __ffma2_rn(pr[k], ti[c], __fmul2_rn(pi[k], tr[c]));
-                        pre[k * kRowStride] = yr.x;
-                        pre[(k + 16) * kRowStride] = yr.y;
-                        pim[k * kRowStride] = yi.x;
-                        pim[(k + 16) * kRowStride] = yi.y;
-                        if (k + 4 < 16) {
-                            const float2 nr = __ffma2_rn(neg2(ti[c]), w4i, __fmul2_rn(tr[c], w4r));
-                            ti[c] = __ffma2_rn(tr[c], w4i, __fmul2_rn(ti[c], w4r));
-                            tr[c] = nr;
-                        }
-                    }
-                }
-                __syncwarp();
-                {
-                    const float4* re4 = reinterpret_cast<const float4*>(buf_a + lane * kRowStride);
-                    const float4* im4 = reinterpret_cast<const float4*>(buf_b + lane * kRowStride);
-#pragma unroll
-                    for (int h = 0; h < 8; ++h) {
-                        const float4 zr = re4[h], zi = im4[h];
-                        pr[brev3(h)] = make_float2(zr.x, zr.y);
-                        pr[brev3(h) + 8] = make_float2(zr.z, zr.w);
-                        pi[brev3(h)] = make_float2(zi.x, zi.y);
-                        pi[brev3(h) + 8] = make_float2(zi.z, zi.w);
-                    }
-                }
-                __syncwarp();   // plane B has been read: the next pair's samples may land in it
-            }
-            // prefetch the samples of this warp's next pair while the second FFT runs
-            staged = false;
-            if (tau + kTcFftWarps / 4 < n_local) {
-#pragma unroll
-                for (int s = 0; s < kTcFftWarps / 4; ++s) cursor_advance(p, cur);
-                staged = cur.tile_in_clip * kTileFrames + 2 * slot_in_tile < cur.frames;
-                if (staged) tc_load_pair(p, cur, slot_in_tile, buf_b, lane, my_bar);
-            }
-            if (active) fft32_packed(pr, pi);
-            // the ring slot of this tile must have been drained by the mel warps (one round of the ring ago)
-            const int ring_slot = tau % kTcRing, round = tau / kTcRing;
-            if (!(ACB_TC_ABLATE & 4) && round > 0 && !mbar_wait(s_empty + ring_slot, (unsigned)(round - 1) & 1u) && lane == 0) atomicExch(p.error_flag, 1);
-            if (active) {
-                float* plane_a = s_ring + ring_slot * kTcSlotFloats + (2 * slot_in_tile) * kTcPlane + lane;
-                const int src_lane = (32 - lane) & 31;
-#pragma unroll
-                for (int m = 0; m < 16; ++m) {
-                    const float alt_r = (m == 0) ? pr[0].x : pr[16 - m].y;
-                    const float alt_i = (m == 0) ? pi[0].x : pi[16 - m].y;
-                    const float offer_r = (lane == 0) ? alt_r : pr[15 - m].y;
-                    const float offer_i = (lane == 0) ? alt_i : pi[15 - m].y;
-                    const float c = __shfl_sync(0xffffffffu, offer_r, src_lane);
-                    const float d = __shfl_sync(0xffffffffu, offer_i, src_lane);
-                    const float a = pr[m].x, b = pi[m].x;
-                    const float apc = a + c, bmd = b - d, amc = a - c, bpd = b + d;
-                    plane_a[32 * m] = fmaf(apc, apc, bmd * bmd);
-                    plane_a[kTcPlane + 32 * m] = fmaf(amc, amc, bpd * bpd);
-                }
-            }
-            __syncwarp();
-            if (!(ACB_TC_ABLATE & 4) && lane == 0) mbar_arrive(s_full + ring_slot);
-        }
-        return;
-    }
-    if (ACB_TC_ABLATE & 4) return;
-
-    // =========================================== mel warps ===========================================
-    const int mw = warp, gid = lane >> 2, tig = lane & 3, gt = tid;   // gt: thread index inside the 128-thread mel group
-    const int* meta = s_meta + mw * (2 + 3 * kTcMaxBlocks);
-    const int n_blocks = meta[0], n_steps = meta[1];
-    float4 w[kTcMaxSteps];                            // (W_hi[k0+2tig][n0+gid], W_hi[k0+2tig+1][.], W_lo ..., W_lo ...) per step
-#pragma unroll
-    for (int i = 0; i < kTcMaxSteps; ++i) w[i] = __ldg(p.tc_w + ((size_t)mw * kTcMaxSteps + i) * 32 + lane);
-    ClipCursor cur;
-    if (n_local > 0) cursor_init(p, cur, t_begin);
-    for (int tau = 0; tau < n_local; ++tau) {
-        const int ring_slot = tau % kTcRing, round = tau / kTcRing;
-        float* s_raw = smem + L.raw + (tau & 1) * (kTileFrames * S);
-        const int f0 = cur.tile_in_clip * kTileFrames;
-        const bool has_frames = f0 < cur.frames;
-        if (!mbar_wait(s_full + ring_slot, (unsigned)round & 1u) && lane == 0) atomicExch(p.error_flag, 1);
-        if (has_frames && !(ACB_TC_ABLATE & 1)) {
-            const float* P = s_ring + ring_slot * kTcSlotFloats + gid * kTcPlane + 2 * tig;
-            float acc[4] = {0.f, 0.f, 0.f, 0.f};
-            int blk = 0, left = meta[2], off = meta[3], band0 = meta[4];
-#pragma unroll
-            for (int i = 0; i < kTcMaxSteps; ++i) {
-                if (i < n_steps) {   // warp-uniform
-                    const float2 pv = *reinterpret_cast<const float2*>(P + off);
-                    const unsigned h0 = __float_as_uint(pv.x) & 0xffffe000u, h1 = __float_as_uint(pv.y) & 0xffffe000u;
-                    const unsigned l0 = __float_as_uint(pv.x - __uint_as_float(h0)) & 0xffffe000u;
-                    const unsigned l1 = __float_as_uint(pv.y - __uint_as_float(h1)) & 0xffffe000u;
-                    mma_tf32_16x8x8(acc, h0, l0, h1, l1, __float_as_uint(w[i].x), __float_as_uint(w[i].y));
-                    mma_tf32_16x8x8(acc, h0, l0, h1, l1, __float_as_uint(w[i].z), __float_as_uint(w[i].w));
-                    off += 8;
-                    if (--left == 0) {   // the band block is complete: rows g (hi) and g + 8 (lo) of the accumulator add up to the mel power
-                        *reinterpret_cast<float2*>(s_raw + gid * S + band0 + 2 * tig) = make_float2(acc[0] + acc[2], acc[1] + acc[3]);
-                        acc[0] = acc[1] = acc[2] = acc[3] = 0.f;
-                        ++blk;
-                        if (blk < n_blocks) { left = meta[2 + 3 * blk]; off = meta[3 + 3 * blk]; band0 = meta[4 + 3 * blk]; }
-                    }
-                }
-            }
-        }
-        __syncwarp();
-        if (lane == 0) mbar_arrive(s_empty + ring_slot);          // this warp has read the slot's power for the last time
-        asm volatile("bar.sync 1, %0;" ::"n"(kTcMelWarps * 32) : "memory");   // the raw mel tile is complete
-
-        const int pad = cur.frames_padded - cur.frames;
-        const bool direct = !p.time_major && (f0 + kTileFrames - 1 <= cur.frames - 2 - pad);
-        const bool write_out = p.out != nullptr;
-        if (has_frames && !(ACB_TC_ABLATE & 2)) {
-            OutT* out_clip = reinterpret_cast<OutT*>(p.out) + cur.out_base;
-            const int f = gt & (kTileFrames - 1);
-            const int fr = f0 + f;
-            for (int b = gt >> 3; b < ((n_mels + 15) & ~15); b += kTcMelWarps * 32 / kTileFrames) {   // whole warps stay in the loop for the shuffles
-                const bool valid = b < n_mels;
-                const float m = (valid ? s_raw[f * S + b] : 1.f) * cur.gain;
-                float v = (m > p.clamp_min) ? lg2_normal(m) * p.log_scale : p.log_floor;
-                if (kMoments) {
-                    float s = 0.f, s2 = 0.f;
-                    if (valid && fr < cur.frames) {
-                        const float c = (fr <= cur.frames - 2 && fr > cur.frames - 2 - pad) ? 2.f : 1.f;
-                        s = c * v;
-                        s2 = s * v;
-                    }
-#pragma unroll
-                    for (int o = 4; o >= 1; o >>= 1) {       // the 8 frames of a band are 8 consecutive lanes
-                        s += __shfl_xor_sync(0xffffffffu, s, o);
-                        s2 += __shfl_xor_sync(0xffffffffu, s2, o);
-                    }
-                    if (f == 0 && valid) {
-                        two_sum_add(s_mom[b], s);
-                        two_sum_add(s_mom[n_mels + b], s2);
-                    }
-                }
-                if (valid) {
-                    const float2 af = s_aff[b];
-                    v = fmaf(v, af.x, af.y);
-                    if (direct) {
-                        if (write_out) out_clip[(size_t)((unsigned)b * (unsigned)cur.cap) + fr] = to_out<OutT>(v);
-                    } else {
-                        s_raw[f * S + b] = v;
-                    }
-                }
-            }
-        }
-        if (!direct) {   // group-uniform
-            asm volatile("bar.sync 1, %0;" ::"n"(kTcMelWarps * 32) : "memory");
-            if (write_out) {
-                store_tile<OutT>(p, cur, s_raw, n_mels, S, gt);
-                if (p.fill_tail && p.tile_start != nullptr && cur.tile_in_clip == cur.tiles_in_clip - 1) fill_row_tail<OutT>(p, cur, n_mels, gt);
-            }
-        }
-        if (tau + 1 < n_local) cursor_advance(p, cur);
-    }
-    if (kMoments) {
-        asm volatile("bar.sync 1, %0;" ::"n"(kTcMelWarps * 32) : "memory");
-        for (int i = gt; i < 2 * n_mels; i += kTcMelWarps * 32)
-            p.moments_partial[(size_t)blockIdx.x * 2 * n_mels + i] = (double)s_mom[i].x + (double)s_mom[i].y;
-    }
-}
-
 // Sum the per-group partials in a fixed order (deterministic) and add into the running accumulators: one warp per value,
 // lanes stride over the partials (independent loads), then a shuffle tree.
 __global__ void __launch_bounds__(256) moments_reduce_kernel(const double* __restrict__ partial, int n_parts, int n_vals, double* __restrict__ acc) {
@@ -1571,12 +1215,6 @@ struct acb_frontend {
     const short* d_plan_astart = nullptr;
     int n_plan_w = 0;
     int* d_err = nullptr;  // in-kernel barrier timeout flag
-    // warp-specialised tensor-core variant (logmel_tc_kernel)
-    bool tc_ok = false;    // the filterbank fits the mel warps' register-resident block plan
-    int kernel_kind = 0;   // 0 = automatic (tc when it fits), 1 = CUDA-core kernel, 2 = tensor-core kernel
-    const float4* d_tc_w = nullptr;
-    const int* d_tc_meta = nullptr;
-    int tc_smem_bytes = 0, tc_smem_bytes_moments = 0, tc_grid = 0;
     // host-path streams/events (created lazily)
     cudaStream_t s_in = nullptr, s_out = nullptr;
     std::vector<cudaEvent_t> ev;
@@ -1739,70 +1377,10 @@ int acb_frontend_create(acb_frontend** out, int device, int n_fft, int hop, int 
         tw[4 * 32 + l] = make_float4(wre(4), wim(4), 0.f, 0.f);
     }
 
-    // Tensor-core plan: the bank as (8 bands x 8 bins) blocks.  A band block covers the bin blocks from its first to its last
-    // non-zero weight; blocks are dealt to the four mel warps longest-first (whole band blocks, so no partial sums cross warps).
-    // Within a block lane (gid, tig) holds the weights of bins k0 + 2 tig, k0 + 2 tig + 1 for band n0 + gid, split into TF32
-    // pairs (hi rounded to nearest, lo = tf32(w - hi)); the 1/4 of the packed-pair power spectrum is folded in.
-    std::vector<float> tc_w((size_t)kTcMelWarps * kTcMaxSteps * 32 * 4, 0.f);
-    std::vector<int> tc_meta((size_t)kTcMelWarps * (2 + 3 * kTcMaxBlocks), 0);
-    bool tc_ok = true;
-    {
-        auto tf32_rn = [](float x) {
-            unsigned u; memcpy(&u, &x, 4);
-            u = (u + 0x0fffu + ((u >> 13) & 1u)) & 0xffffe000u;
-            float y; memcpy(&y, &u, 4);
-            return y;
-        };
-        const int n_nb = (n_mels + 7) / 8;
-        std::vector<int> kb0(n_nb, 0), cnt(n_nb, 0);
-        for (int nb = 0; nb < n_nb; ++nb) {
-            int lo = -1, hi = -1;
-            for (int m = 8 * nb; m < std::min(n_mels, 8 * nb + 8); ++m)
-                if (len[m] > 0) { lo = lo < 0 ? start[m] : std::min(lo, start[m]); hi = std::max(hi, start[m] + len[m] - 1); }
-            if (lo >= 0) { kb0[nb] = lo / 8; cnt[nb] = std::min(hi, kBins - 1) / 8 - lo / 8 + 1; }
-            else { kb0[nb] = 0; cnt[nb] = 1; }   // a block of silent bands still writes its (zero) mel powers
-        }
-        std::vector<int> order_nb(n_nb);
-        std::iota(order_nb.begin(), order_nb.end(), 0);
-        std::stable_sort(order_nb.begin(), order_nb.end(), [&](int a, int b) { return cnt[a] > cnt[b]; });
-        std::vector<int> steps(kTcMelWarps, 0), blocks(kTcMelWarps, 0);
-        for (int nb : order_nb) {
-            int best = 0;
-            for (int w = 1; w < kTcMelWarps; ++w)
-                if (steps[w] < steps[best]) best = w;
-            if (steps[best] + cnt[nb] > kTcMaxSteps || blocks[best] >= kTcMaxBlocks) { tc_ok = false; break; }
-            int* meta = tc_meta.data() + (size_t)best * (2 + 3 * kTcMaxBlocks);
-            meta[2 + 3 * blocks[best]] = cnt[nb];
-            meta[3 + 3 * blocks[best]] = kb0[nb] * 8;
-            meta[4 + 3 * blocks[best]] = nb * 8;
-            for (int s = 0; s < cnt[nb]; ++s) {
-                const int k0 = (kb0[nb] + s) * 8;
-                for (int lane = 0; lane < 32; ++lane) {
-                    const int gid = lane >> 2, tig = lane & 3, m = nb * 8 + gid;
-                    float wv[2] = {0.f, 0.f};
-                    for (int e = 0; e < 2; ++e) {
-                        const int f = k0 + 2 * tig + e;
-                        if (m < n_mels && f < kBins) wv[e] = fb_host[(size_t)f * n_mels + m] * 0.25f;
-                    }
-                    float* dst = tc_w.data() + (((size_t)best * kTcMaxSteps + steps[best] + s) * 32 + lane) * 4;
-                    dst[0] = tf32_rn(wv[0]); dst[1] = tf32_rn(wv[1]);
-                    dst[2] = tf32_rn(wv[0] - dst[0]); dst[3] = tf32_rn(wv[1] - dst[1]);
-                }
-            }
-            steps[best] += cnt[nb];
-            blocks[best]++;
-        }
-        for (int w = 0; w < kTcMelWarps; ++w) {
-            tc_meta[(size_t)w * (2 + 3 * kTcMaxBlocks)] = blocks[w];
-            tc_meta[(size_t)w * (2 + 3 * kTcMaxBlocks) + 1] = steps[w];
-        }
-    }
-
     int prev = 0;
     ACB_CUDA(cudaGetDevice(&prev));
     ACB_CUDA(cudaSetDevice(device));
     auto* fe = new acb_frontend();
-    fe->tc_ok = tc_ok;
     fe->device = device; fe->n_fft = n_fft; fe->hop = hop; fe->n_mels = n_mels; fe->n_weights = (int)weights.size();
     fe->n_plan_w = (int)plan_w.size();
     fe->log_kind = log_kind; fe->clamp_min = clamp_min;
@@ -1813,8 +1391,7 @@ int acb_frontend_create(acb_frontend** out, int device, int n_fft, int hop, int 
     const size_t o_win = take(sizeof(float) * kNfft), o_tw = take(sizeof(float4) * 160),
                  o_pw = take(sizeof(float) * std::max<size_t>(plan_w.size(), 1)), o_po = take(sizeof(int) * plan_woff.size()),
                  o_pt = take(sizeof(short) * plan_trip.size()), o_pb = take(sizeof(short) * plan_band.size()),
-                 o_pa = take(sizeof(short) * plan_astart.size()), o_err = take(16),
-                 o_tcw = take(sizeof(float) * tc_w.size()), o_tcm = take(sizeof(int) * tc_meta.size());
+                 o_pa = take(sizeof(short) * plan_astart.size()), o_err = take(16);
     std::vector<unsigned char> host(o, 0);
     memcpy(host.data() + o_win, window_host, sizeof(float) * kNfft);
     memcpy(host.data() + o_tw, tw.data(), sizeof(float4) * 160);
@@ -1823,8 +1400,6 @@ int acb_frontend_create(acb_frontend** out, int device, int n_fft, int hop, int 
     memcpy(host.data() + o_pt, plan_trip.data(), sizeof(short) * plan_trip.size());
     memcpy(host.data() + o_pb, plan_band.data(), sizeof(short) * plan_band.size());
     memcpy(host.data() + o_pa, plan_astart.data(), sizeof(short) * plan_astart.size());
-    memcpy(host.data() + o_tcw, tc_w.data(), sizeof(float) * tc_w.size());
-    memcpy(host.data() + o_tcm, tc_meta.data(), sizeof(int) * tc_meta.size());
     cudaError_t e = cudaMalloc(&fe->d_blob, o);
     if (e == cudaSuccess) e = cudaMemcpy(fe->d_blob, host.data(), o, cudaMemcpyHostToDevice);
     cudaDeviceProp prop;
@@ -1860,16 +1435,6 @@ int acb_frontend_create(acb_frontend** out, int device, int n_fft, int hop, int 
         prepare(logmel_fused_kernel<2, true, float>, 2 * kGroupThreads);
         prepare(logmel_fused_kernel<2, true, __nv_bfloat16>, 2 * kGroupThreads);
     }
-    fe->tc_smem_bytes = make_tc_smem_layout(n_mels, false).total_bytes;
-    fe->tc_smem_bytes_moments = make_tc_smem_layout(n_mels, true).total_bytes;
-    if (fe->tc_smem_bytes_moments > optin) fe->tc_ok = false;
-    if (fe->tc_ok) {
-        auto prep = [&](auto kernel) { if (e == cudaSuccess) e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, optin); };
-        prep(logmel_tc_kernel<false, float>);
-        prep(logmel_tc_kernel<false, __nv_bfloat16>);
-        prep(logmel_tc_kernel<true, float>);
-        prep(logmel_tc_kernel<true, __nv_bfloat16>);
-    }
     if (e != cudaSuccess) {
         if (fe->d_blob) cudaFree(fe->d_blob);
         delete fe;
@@ -1877,7 +1442,6 @@ int acb_frontend_create(acb_frontend** out, int device, int n_fft, int hop, int 
         return cuda_fail(e, "acb_frontend_create");
     }
     fe->num_sms = prop.multiProcessorCount;
-    fe->tc_grid = prop.multiProcessorCount;
     fe->grid = fe->num_sms * std::max(occ, 1);
     auto* base = static_cast<unsigned char*>(fe->d_blob);
     fe->d_window = reinterpret_cast<const float*>(base + o_win);
@@ -1888,8 +1452,6 @@ int acb_frontend_create(acb_frontend** out, int device, int n_fft, int hop, int 
     fe->d_plan_band = reinterpret_cast<const short*>(base + o_pb);
     fe->d_plan_astart = reinterpret_cast<const short*>(base + o_pa);
     fe->d_err = reinterpret_cast<int*>(base + o_err);
-    fe->d_tc_w = reinterpret_cast<const float4*>(base + o_tcw);
-    fe->d_tc_meta = reinterpret_cast<const int*>(base + o_tcm);
     cudaSetDevice(prev);
     *out = fe;
     return ACB_OK;
@@ -1911,7 +1473,7 @@ int acb_frontend_destroy(acb_frontend* fe) {
 
 int64_t acb_moments_workspace_bytes(const acb_frontend* fe) {
     if (!fe) return fail(ACB_ERR_INVALID, "acb_moments_workspace_bytes: null handle");
-    return (int64_t)std::max(fe->grid * fe->groups, fe->tc_grid) * 2 * fe->n_mels * (int64_t)sizeof(double);
+    return (int64_t)fe->grid * fe->groups * 2 * fe->n_mels * (int64_t)sizeof(double);
 }
 
 int acb_logmel_forward(const acb_frontend* fe, const acb_logmel_args* a, void* stream) {
@@ -1985,35 +1547,22 @@ int acb_logmel_forward(const acb_frontend* fe, const acb_logmel_args* a, void* s
     if (prev != fe->device) ACB_CUDA(cudaSetDevice(fe->device));
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     const int grid = fe->grid;  // persistent: every CTA takes a contiguous share of the tiles (possibly empty)
-    // "automatic" is the CUDA-core kernel: measured on B200 (256 x 30 s) it runs 0.466 ms against 1.80 ms for the warp-specialised
-    // tensor-core variant, whose twelve FFT warps alone need 0.437 ms (profiles/r02_tc_variant.txt) -- the FFT phase, not the mel
-    // projection, bounds this path.  The tensor-core variant stays selectable (acb_frontend_set_kernel) and parity-tested.
-    const bool use_tc = fe->tc_ok && fe->kernel_kind == 2;
-    p.tc_w = fe->d_tc_w; p.tc_meta = fe->d_tc_meta;
-    int n_parts = 0;
-    if (use_tc) {
-        // warp-specialised kernel: one CTA per SM, FFT warps feed tensor-core mel warps through a shared-memory ring
-        const size_t smem = a->moments ? fe->tc_smem_bytes_moments : fe->tc_smem_bytes;
-        auto launch = [&](auto kernel) { kernel<<<fe->tc_grid, kTcThreads, smem, st>>>(p); };
-        if (a->moments) { if (p.out_bf16) launch(logmel_tc_kernel<true, __nv_bfloat16>); else launch(logmel_tc_kernel<true, float>); }
-        else { if (p.out_bf16) launch(logmel_tc_kernel<false, __nv_bfloat16>); else launch(logmel_tc_kernel<false, float>); }
-        n_parts = fe->tc_grid;
+    // The mel projection runs on the CUDA cores: measured on B200 (256 x 30 s) this kernel runs 0.466 ms against 1.80 ms for a
+    // warp-specialised variant with the projection on the tensor pipe, whose twelve FFT warps alone needed 0.437 ms
+    // (profiles/r02_tc_variant.txt) -- the FFT phase, not the mel projection, bounds this path.
+    const int threads = fe->groups * kGroupThreads;
+    const size_t smem = a->moments ? fe->smem_bytes_moments : fe->smem_bytes;
+    auto launch = [&](auto kernel) { kernel<<<grid, threads, smem, st>>>(p); };
+    if (fe->groups == 4) {
+        if (a->moments) { if (p.out_bf16) launch(logmel_fused_kernel<4, true, __nv_bfloat16>); else launch(logmel_fused_kernel<4, true, float>); }
+        else { if (p.out_bf16) launch(logmel_fused_kernel<4, false, __nv_bfloat16>); else launch(logmel_fused_kernel<4, false, float>); }
     } else {
-        const int threads = fe->groups * kGroupThreads;
-        const size_t smem = a->moments ? fe->smem_bytes_moments : fe->smem_bytes;
-        auto launch = [&](auto kernel) { kernel<<<grid, threads, smem, st>>>(p); };
-        if (fe->groups == 4) {
-            if (a->moments) { if (p.out_bf16) launch(logmel_fused_kernel<4, true, __nv_bfloat16>); else launch(logmel_fused_kernel<4, true, float>); }
-            else { if (p.out_bf16) launch(logmel_fused_kernel<4, false, __nv_bfloat16>); else launch(logmel_fused_kernel<4, false, float>); }
-        } else {
-            if (a->moments) { if (p.out_bf16) launch(logmel_fused_kernel<2, true, __nv_bfloat16>); else launch(logmel_fused_kernel<2, true, float>); }
-            else { if (p.out_bf16) launch(logmel_fused_kernel<2, false, __nv_bfloat16>); else launch(logmel_fused_kernel<2, false, float>); }
-        }
-        n_parts = grid * fe->groups;
+        if (a->moments) { if (p.out_bf16) launch(logmel_fused_kernel<2, true, __nv_bfloat16>); else launch(logmel_fused_kernel<2, true, float>); }
+        else { if (p.out_bf16) launch(logmel_fused_kernel<2, false, __nv_bfloat16>); else launch(logmel_fused_kernel<2, false, float>); }
     }
     if (a->moments) {
         const int n_vals = 2 * fe->n_mels;
-        moments_reduce_kernel<<<(n_vals + 7) / 8, 256, 0, st>>>(p.moments_partial, n_parts, n_vals, a->moments);
+        moments_reduce_kernel<<<(n_vals + 7) / 8, 256, 0, st>>>(p.moments_partial, grid * fe->groups, n_vals, a->moments);
     }
     cudaError_t e = cudaGetLastError();
     if (prev != fe->device) cudaSetDevice(prev);
@@ -2024,8 +1573,7 @@ int acb_logmel_forward(const acb_frontend* fe, const acb_logmel_args* a, void* s
 int acb_frontend_set_kernel(acb_frontend* fe, int kind) {
     if (!fe) return fail(ACB_ERR_INVALID, "acb_frontend_set_kernel: null handle");
     if (kind < 0 || kind > 2) return fail(ACB_ERR_INVALID, "acb_frontend_set_kernel: kind must be 0 (automatic), 1 (CUDA-core mel) or 2 (tensor-core mel)");
-    if (kind == 2 && !fe->tc_ok) return fail(ACB_ERR_UNSUPPORTED, "acb_frontend_set_kernel: this filterbank does not fit the tensor-core block plan");
-    fe->kernel_kind = kind;
+    if (kind == 2) return fail(ACB_ERR_UNSUPPORTED, "acb_frontend_set_kernel: this build has only the CUDA-core mel kernel (kind 0 or 1)");
     return ACB_OK;
 }
 

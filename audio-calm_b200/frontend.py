@@ -168,9 +168,9 @@ class LogMelFrontend:
         return keep
 
     def set_kernel(self, kind: str = "auto") -> None:
-        """Choose the implementation behind ``acb_logmel_forward``: ``"auto"`` (the faster one as measured: the CUDA-core kernel),
-        ``"cuda_core"`` or ``"tensor_core"`` (warp-specialised variant with the mel projection on the tensor pipe).  Same results
-        within the parity tolerance; the switch exists for A/B measurement and so that the tests can pin either."""
+        """Choose the implementation behind ``acb_logmel_forward``.  ``"auto"`` and ``"cuda_core"`` select the one this build has,
+        the kernel with the mel projection on the CUDA cores.  ``"tensor_core"`` (a warp-specialised variant with the projection on
+        the tensor pipe, measured 3.9x slower and removed) raises AcbError."""
         _lib.check(self._lib.acb_frontend_set_kernel(self._handle, {"auto": 0, "cuda_core": 1, "tensor_core": 2}[kind]),
                    "acb_frontend_set_kernel")
 

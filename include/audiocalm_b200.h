@@ -71,11 +71,10 @@ int64_t acb_plan_tiles(const int64_t* lengths_host, int32_t n_clips, int n_fft, 
 int acb_frontend_create(acb_frontend** out, int device, int n_fft, int hop, int n_mels,
                         const float* window_host, const float* fb_host, float clamp_min, int log_kind);
 int acb_frontend_destroy(acb_frontend* fe);
-/* Which of the two implementations of the fused log-mel kernel acb_logmel_forward launches: 0 = automatic (the faster one as
- * measured on B200: the CUDA-core kernel), 1 = CUDA-core mel projection, 2 = the warp-specialised kernel with the mel projection
- * on the tensor pipe (mma.sync TF32 pairs; ACB_ERR_UNSUPPORTED when the filterbank does not fit its register-resident block
- * plan).  Both compute MelExtractor.forward (preprocess/core.py:50-61); the switch exists for A/B measurement and for the
- * parity tests of both. */
+/* Which implementation of the fused log-mel kernel acb_logmel_forward launches.  This build has one, with the mel projection
+ * on the CUDA cores: 0 = automatic and 1 = CUDA-core mel projection both select it and return ACB_OK.  2 = the warp-specialised
+ * kernel with the mel projection on the tensor pipe (mma.sync TF32 pairs) returns ACB_ERR_UNSUPPORTED: it was measured on B200
+ * at 1.80 ms against 0.466 ms for the CUDA-core kernel (256 x 30 s) and removed.  Any other kind returns ACB_ERR_INVALID. */
 int acb_frontend_set_kernel(acb_frontend* fe, int kind);
 /* bytes of device workspace acb_logmel_forward needs when moments are requested */
 int64_t acb_moments_workspace_bytes(const acb_frontend* fe);

@@ -420,44 +420,14 @@ def test_pad_multiple_must_divide_the_tile(fe):
     assert fe.forward(x, pad_multiple=8).shape[-1] % 8 == 0
 
 
-# ----------------------------------------------------------------------------------- the tensor-core variant of the kernel
-def test_tensor_core_mel_variant_matches_the_goldens(golden):
-    """logmel_tc_kernel (FFT warps + mma.sync TF32-pair mel warps, selected with set_kernel) against the reference-minted goldens,
-    the oracle on a ragged batch with peak normalisation, pad-to-4 and fused moments, and the CUDA-core kernel."""
-    fe2 = acb.LogMelFrontend("cuda")
-    fe2.set_kernel("tensor_core")
-    for name in ("raw_noise_16000_s1", "raw_synth_24001_s12", "raw_synth_513_s13", "raw_zeros_4000"):
-        y = fe2.forward(dev(RAW[name]()[None]))[0].cpu().numpy()
-        assert y.shape == golden[name].shape and float(np.max(np.abs(y - golden[name]))) < EXPECT, name
-    waves = [o.synth_clip(n, 700 + i) for i, n in enumerate((8000, 24001, 777, 100001, 16000, 40000))]
-    batch = acb.pack_clips([torch.from_numpy(w) for w in waves], torch.device("cuda", torch.cuda.current_device()))
-    acc = acb.MelStatsAccumulator(80, "cuda")
-    for layout, dtype in (("mel_major", torch.float32), ("time_major", torch.float32), ("mel_major", torch.bfloat16)):
-        aff = (acb.MEL_MEAN_DEFAULT, acb.MEL_STD_DEFAULT) if dtype == torch.bfloat16 else None
-        out, frames = fe2.forward_ragged(batch, pad_multiple=4, peak=fe2.peak_abs_ragged(batch), layout=layout, out_dtype=dtype, affine=aff,
-                                         moments=acc if layout == "mel_major" and dtype == torch.float32 else None)
-        for i, w in enumerate(waves):
-            ref = o.dataset_mel(w[None], fe2.window.numpy(), fe2.fb.numpy())
-            T4 = ref.shape[1]
-            assert int(frames[i]) == T4
-            got = out[i].float().cpu().numpy()
-            got = got[:, :T4] if layout == "mel_major" else got[:T4].T
-            if dtype == torch.bfloat16:
-                assert float(np.max(np.abs(got - o.normalise_global(ref)))) < TOL_BF16
-            else:
-                assert float(np.max(np.abs(got - ref))) < EXPECT, (layout, i)
-            tail = out[i][:, T4:] if layout == "mel_major" else out[i][T4:]
-            assert not bool(tail.float().abs().max() > 0) if tail.numel() else True       # zero tail
-    mels = [o.dataset_mel(w[None], fe2.window.numpy(), fe2.fb.numpy()) for w in waves]
-    s, s2, n_frames = o.stats_per_bin(mels)
-    st = acc.finalize()
-    bm, bs = o.stats_per_bin_finalise(s, s2, n_frames)
-    assert st.frames == n_frames and np.max(np.abs(st.bin_mean - bm)) < 1e-5 and np.max(np.abs(st.bin_std - bs)) < 1e-5
-    x = _device_clips(32, 480000, 77)                                                 # config-2 sized clips: both kernels agree
-    fe1 = acb.LogMelFrontend("cuda")
-    a, b = fe1.forward(x), fe2.forward(x)
-    fe2.check()
-    assert float((a - b).abs().max()) < 1e-5
+# ----------------------------------------------------------------------------------- kernel selection
+def test_tensor_core_kind_is_unsupported(fe):
+    """Kind 2 (the tensor-core mel variant, removed) returns ACB_ERR_UNSUPPORTED from the host; kinds 0 and 1 return ACB_OK."""
+    lib = acb._lib.load()
+    assert lib.acb_frontend_set_kernel(fe._handle, 2) == -3 and b"CUDA-core" in lib.acb_last_error()
+    with pytest.raises(acb._lib.AcbError):
+        fe.set_kernel("tensor_core")
+    assert lib.acb_frontend_set_kernel(fe._handle, 0) == 0 and lib.acb_frontend_set_kernel(fe._handle, 1) == 0
 
 
 # ----------------------------------------------------------------------------------- host-buffer path

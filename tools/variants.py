@@ -33,10 +33,6 @@ VARIANTS = {
     "win00": ["-DACB_WIN_FUSE=0", "-DACB_WIN_T=0"],
     "win10": ["-DACB_WIN_FUSE=1", "-DACB_WIN_T=0"],
     "win01": ["-DACB_WIN_FUSE=0", "-DACB_WIN_T=1"],
-    "tcab1": ["-DACB_DEV", "-DACB_TC_ABLATE=1"],
-    "tcab2": ["-DACB_DEV", "-DACB_TC_ABLATE=2"],
-    "tcab3": ["-DACB_DEV", "-DACB_TC_ABLATE=3"],
-    "tcab7": ["-DACB_DEV", "-DACB_TC_ABLATE=7"],
     "dev": ["-DACB_DEV"],
     "p16": ["-DACBG_PREP_WARPS=16"],
     "band8": ["-DACBG_BAND_COST=8"],
@@ -91,7 +87,6 @@ def run_one(name, steps=50):
     from oracle import logmel_oracle as o
     acb._lib.LIB_PATH = os.path.join(OUT, f"lib_{name}.so")
     fe = acb.LogMelFrontend("cuda")
-    fe.set_kernel(os.environ.get("ACB_KIND", "auto"))
     # parity: ragged pair of clips, peak-normalised, pad-to-4, fused moments
     clips = [o.synth_clip(48000 + 777, 5), o.hash_noise(16000, 1)]
     worst = 0.0
@@ -120,7 +115,7 @@ def run_one(name, steps=50):
     ref_clip = o.normalise_global(o.logmel(x[3].cpu().numpy(), fe.window.numpy(), fe.fb.numpy()))
     d2 = float(np.max(np.abs(out[3].cpu().numpy() - ref_clip)))
     fe.check()
-    print(json.dumps({"variant": name, "kind": os.environ.get("ACB_KIND", "auto"), "flags": VARIANTS[name], "ms": ms, "gframes_s": 256 * 1876 / ms / 1e6,
+    print(json.dumps({"variant": name, "flags": VARIANTS[name], "ms": ms, "gframes_s": 256 * 1876 / ms / 1e6,
                       "frac": 256 * (4 * 480000 + 320 * 1876) / (ms * 1e-3) / 1e9 / 6537.6, "max_abs_err": worst, "cfg2_err": d2}), flush=True)
 
 
