@@ -1269,6 +1269,14 @@ int acb_frontend_create(acb_frontend** out, int device, int n_fft, int hop, int 
     if (n_mels < 1 || n_mels > kMaxMels) return fail(ACB_ERR_UNSUPPORTED, "acb_frontend_create: n_mels must be in [1, 128]");
     if (log_kind != ACB_LOG_NATURAL && log_kind != ACB_LOG_10) return fail(ACB_ERR_INVALID, "acb_frontend_create: bad log_kind");
     if (!(clamp_min >= 1.17549435e-38f)) return fail(ACB_ERR_INVALID, "acb_frontend_create: clamp_min must be a positive normal float");
+    // The kernel stages only w[0 .. N/2 - 1] and computes the second half as 1 - w[n] (the periodic-Hann property).  A window
+    // without that property would give wrong features silently; fp32 periodic Hann deviates by 1.8e-7.
+    for (int n = 0; n < kNfft / 2; ++n) {
+        const double dev = std::fabs((double)window_host[n + kNfft / 2] - (1.0 - (double)window_host[n]));
+        if (!(dev <= 1e-6))
+            return fail(ACB_ERR_UNSUPPORTED, "acb_frontend_create: the window must have the periodic-Hann property w[n + 512] = 1 - w[n] "
+                                             "(deviation " + std::to_string(dev) + " at n=" + std::to_string(n) + ")");
+    }
     const int n_freq = n_fft / 2 + 1;
 
     // banded form of the filterbank; the 1/4 of the packed-pair power spectrum is folded in (exact scaling)

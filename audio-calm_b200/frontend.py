@@ -83,6 +83,11 @@ class LogMelFrontend:
 
     Defaults reproduce ``MelExtractor()`` (preprocess/core.py:33-48,60): 16 kHz, n_fft 1024, periodic Hann,
     hop 256, 80 slaney mels over 0-8000 Hz, power 2, ``log(clamp(., 1e-5))``.
+
+    ``fb`` may be any ``[513, n_mels]`` bank with 1 <= n_mels <= 128, no weight on the Nyquist bin and at most 4096 weights between
+    each band's first and last non-zero bin.  ``window`` must have the periodic-Hann property ``w[n + 512] = 1 - w[n]`` to within
+    1e-6: the kernel stages only the first half of the window and computes the second.  ``torch.hann_window(1024)`` has it; a
+    Hamming, a symmetric Hann or a scaled Hann window does not and raises ``AcbError``.
     """
 
     def __init__(self, device: Union[str, torch.device, int] = "cuda", sample_rate: int = 16000, n_fft: int = 1024,

@@ -291,3 +291,37 @@ def test_peak_norm_affine_and_moments(gw):
     assert acc8.finalize().frames == n and np.max(np.abs(acc8.finalize().bin_mean - bm8)) < 1e-5
     with pytest.raises(ValueError):
         acb.WhisperLogMel("cuda").forward_ragged([dev(waves[0])], moments=acb.MelStatsAccumulator(80, "cuda"))
+
+
+# ----------------------------------------------------------------------------------- windows and small or sparse banks
+def test_symmetric_window_other_than_hann():
+    """The route needs only w[n] = w[400 - n]: a periodic Hamming window matches the oracle computed with it."""
+    w = torch.hamming_window(400)
+    fe2 = acb.WhisperLogMel("cuda", window=w)
+    x = o.synth_clip(40000, 91)
+    y = fe2.forward(dev(x)[None], check=True)[0].cpu().numpy()
+    assert np.abs(y - wo.whisper_logmel(x, w.numpy(), fe2.fb.numpy())).max() < EXPECT
+
+
+def test_asymmetric_window_raises():
+    n = torch.arange(400, dtype=torch.float64)
+    w = (0.5 - 0.5 * torch.cos(2 * np.pi * n / 400) + 0.05 * torch.sin(6 * np.pi * n / 400)).float()
+    with pytest.raises(acb._lib.AcbError, match="symmetric"):
+        acb.WhisperLogMel("cuda", window=w)
+
+
+@pytest.mark.parametrize("bank", ["slaney2", "slaney3", "zero_bands"])
+def test_banks_that_leave_worker_warps_without_a_band(bank):
+    """With 2 or 3 bands most of the 8 worker warps get no band to project; all-zero bands (first, middle, last) sit on the clamp."""
+    from audio_calm_b200.whisper import whisper_tables
+    if bank == "zero_bands":
+        fb = whisper_tables(80)[1].clone()
+        fb[:, [0, 40, 79]] = 0.0
+    else:
+        fb = whisper_tables(int(bank[-1]))[1]
+    fe2 = acb.WhisperLogMel("cuda", n_mels=fb.shape[1], fb=fb)
+    xs = np.stack([o.synth_clip(40000, 92), o.hash_noise(40000, 93)])
+    y = fe2.forward(dev(xs), check=True).cpu().numpy()
+    for i in range(2):
+        ref = wo.whisper_logmel(xs[i], fe2.window.numpy(), fe2.fb.numpy())
+        assert y[i].shape == ref.shape and np.abs(y[i] - ref).max() < EXPECT, (bank, i)
