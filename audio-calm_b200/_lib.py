@@ -127,8 +127,7 @@ def build(force: bool = False, verbose: bool = False) -> str:
     """Compile the CUDA sources for sm_100a into ``csrc/libaudiocalm_b200.so`` (cross-compiles without a GPU)."""
     if not force and not needs_build():
         return LIB_PATH
-    extra = os.environ.get("ACB_NVCC_EXTRA", "").split()      # development: e.g. -DACBG_WORKER_WARPS=8
-    cmd = [_nvcc()] + NVCC_FLAGS + extra + ["-I", INCLUDE, "-o", LIB_PATH + ".tmp"] + [os.path.join(CSRC, s) for s in SOURCES]
+    cmd = [_nvcc()] + NVCC_FLAGS + ["-I", INCLUDE, "-o", LIB_PATH + ".tmp"] + [os.path.join(CSRC, s) for s in SOURCES]
     if verbose:
         cmd.insert(1, "-Xptxas")
         cmd.insert(2, "-v")

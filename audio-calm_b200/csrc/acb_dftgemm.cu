@@ -57,28 +57,9 @@ constexpr int kNfft = 400;
 constexpr int kHop = 160;
 constexpr int kBinsAll = 201;
 constexpr int kTileFrames = 128;
-// Development-only hooks, compiled in only with -DACB_DEV: the ablation switch (tools/ablate_dftgemm.sh prices each part of the K loop
-// in situ; results are wrong for n != 0) and the in-kernel timeline (tools/whisper_trace.py).  The shipped library has neither.
-#if !defined(ACB_DEV) || !defined(ACBG_ABLATE)
-#undef ACBG_ABLATE
-#define ACBG_ABLATE 0
-#endif
-#ifndef ACBG_CHK
-#define ACBG_CHK 1
-#endif
-#ifndef ACBG_PRESCALE
-#define ACBG_PRESCALE 1
-#endif
-#ifndef ACBG_A_HI_TMEM
-#define ACBG_A_HI_TMEM 1        // 1: the A_hi slices live in the 64 TMEM columns the accumulators leave free (.ts MMAs); 0: all operands in shared memory
-#endif
-constexpr int kAhiCols = 448;                       // first TMEM column of the A_hi stages: [stage][gemm][8 columns = 16 fp16]
+constexpr int kAhiCols = 448;                       // first TMEM column of the A_hi stages (the 64 the accumulators leave free): [stage][gemm][8 columns = 16 fp16]
 constexpr int kWorkerWarps = 16;                    // all of them run the epilogue (4 per TMEM lane quarter)
-#ifndef ACBG_PREP_WARPS
-#define ACBG_PREP_WARPS 8
-#endif
-constexpr int kPrepWarps = ACBG_PREP_WARPS;         // 8: the first 8 warps build the A slices, thread = (frame row, k-half), 16-byte stores;
-                                                    // 16 (experiment): all of them, thread = (frame row, quarter of the K step), 8-byte stores
+constexpr int kPrepWarps = 8;                       // the first 8 build the A slices, thread = (frame row, k-half), 16-byte stores
 constexpr int kWorkerThreads = kWorkerWarps * 32;
 constexpr int kThreads = kWorkerThreads + 64;      // + one MMA issuer warp + one B-slice loader warp (one elected lane each)
 constexpr int kKpad = 112;                       // K of every GEMM (n = 0..100 used)
@@ -97,10 +78,7 @@ constexpr int kPowBins = 224;                    // 7 chunks of 32 bins of |X|^2
 constexpr int kMaxWeights = 3072;                // packed non-zero filterbank weights (banded form)
 constexpr int kTmemCols = 512;
 constexpr int kMaxMels = 128;
-#ifndef ACBG_BAND_COST
-#define ACBG_BAND_COST 16
-#endif
-constexpr int kBandCost = ACBG_BAND_COST;          // fixed cost of a band (logs, stores) in units of one weight, for balancing the band groups
+constexpr int kBandCost = 16;                      // fixed cost of a band (logs, stores) in units of one weight, for balancing the band groups
 constexpr float kPrescale = 4096.f;                // power-of-two scale of the A operands (see acb_dftgemm_create)
 
 // shared memory carve-up (bytes)
@@ -153,22 +131,13 @@ __device__ __forceinline__ void mbar_arrive_expect_tx(uint32_t bar, uint32_t byt
 // sleeps in hardware until the phase completes (or the hint expires) instead of polling.  Without it 45 % of the kernel's issued
 // instructions were mbarrier polls of idle warps, each one an access to shared memory next to the K loop's operand traffic:
 // 0.480 -> 0.463 ms per 256 x 30 s (hint 100 ns: 0.465, 1 us: 0.4634, 10 us: 0.4629).  Returns false after ~10 s.
-#ifndef ACBG_WAIT_HINT_NS
-#define ACBG_WAIT_HINT_NS 10000
-#endif
+constexpr uint32_t kWaitHintNs = 10000;
 __device__ __forceinline__ bool mbar_wait(uint32_t bar, uint32_t parity) {
     uint32_t ok = 0;
-#if ACBG_WAIT_HINT_NS > 0
     for (int spin = 0; spin < (1 << 20) && !ok; ++spin) {
         asm volatile("{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2, %3;\n\tselp.u32 %0, 1, 0, p;\n\t}\n"
-                     : "=r"(ok) : "r"(bar), "r"(parity), "r"((uint32_t)ACBG_WAIT_HINT_NS) : "memory");
+                     : "=r"(ok) : "r"(bar), "r"(parity), "r"(kWaitHintNs) : "memory");
     }
-#else
-    for (int spin = 0; spin < (1 << 26) && !ok; ++spin) {
-        asm volatile("{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\tselp.u32 %0, 1, 0, p;\n\t}\n"
-                     : "=r"(ok) : "r"(bar), "r"(parity) : "memory");
-    }
-#endif
     return ok != 0;
 }
 __device__ __forceinline__ void bulk_copy_g2s(uint32_t dst, const void* src, uint32_t bytes, uint32_t bar) {
@@ -205,9 +174,6 @@ __device__ __forceinline__ void mma_f16_ts(uint32_t tmem_d, uint32_t tmem_a, uin
 }
 __device__ __forceinline__ void tmem_st4(uint32_t taddr, uint32_t r0, uint32_t r1, uint32_t r2, uint32_t r3) {
     asm volatile("tcgen05.st.sync.aligned.32x32b.x4.b32 [%0], {%1, %2, %3, %4};" ::"r"(taddr), "r"(r0), "r"(r1), "r"(r2), "r"(r3) : "memory");
-}
-__device__ __forceinline__ void tmem_st2(uint32_t taddr, uint32_t r0, uint32_t r1) {
-    asm volatile("tcgen05.st.sync.aligned.32x32b.x2.b32 [%0], {%1, %2};" ::"r"(taddr), "r"(r0), "r"(r1) : "memory");
 }
 __device__ __forceinline__ void tmem_st_wait() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
 __device__ __forceinline__ void mma_commit(uint32_t bar) {
@@ -301,7 +267,6 @@ struct Params {
     double* moments_partial;   // [gridDim.x][2][n_mels] per-CTA sums of v and v^2 over the frames that exist, or nullptr
     int* error_flag;           // set to 1 when a barrier wait timed out
     int use_tma;               // the batch is 128-byte row addressable (16-byte aligned base, clip_stride % 32 == 0): tensor copies
-    long long* trace;          // development: clock64 stamps of CTA 0 ([role][tile < 48][event < 16]), or nullptr
 };
 
 // A-operand values of one thread for one K step: 8 consecutive n of its frame row, for the 4 GEMMs
@@ -313,36 +278,17 @@ __device__ __forceinline__ uint32_t pack_half2(__half a, __half b) {
     return (uint32_t)__half_as_ushort(a) | ((uint32_t)__half_as_ushort(b) << 16);
 }
 
-// split 8 fp32 values into fp16 (hi, lo) and store them as one 16-byte core-matrix row each (packed conversions: F2FP / HADD2.F32)
-__device__ __forceinline__ void split_store(const float (&v)[8], uint8_t* dst_hi, uint8_t* dst_lo) {
-    uint32_t hi[4], lo[4];
-#pragma unroll
-    for (int i = 0; i < 4; ++i) {
-        const __half2 h = __floats2half2_rn(v[2 * i], v[2 * i + 1]);
-        const float2 hf = __half22float2(h);
-        const __half2 l = __floats2half2_rn(v[2 * i] - hf.x, v[2 * i + 1] - hf.y);
-        hi[i] = *reinterpret_cast<const uint32_t*>(&h);
-        lo[i] = *reinterpret_cast<const uint32_t*>(&l);
-    }
-    *reinterpret_cast<uint4*>(dst_hi) = make_uint4(hi[0], hi[1], hi[2], hi[3]);
-    *reinterpret_cast<uint4*>(dst_lo) = make_uint4(lo[0], lo[1], lo[2], lo[3]);
-}
-
-// Same, with the hi halves going to tensor memory: 4 columns (8 packed halves) of this thread's lane at `t_hi`
+// split 8 fp32 values into fp16 (hi, lo) (packed conversions: F2FP / HADD2.F32); the hi halves go to tensor memory, 4 columns
+// (8 packed halves) of this thread's lane at `t_hi`, the lo halves to shared memory as one 16-byte core-matrix row
 __device__ __forceinline__ void split_store_tmem(const float (&v)[8], uint32_t t_hi, uint8_t* dst_lo) {
     uint32_t hi[4], lo[4];
 #pragma unroll
     for (int i = 0; i < 4; ++i) {
-#if ACBG_ABLATE == 5   // byte permutes instead of the split conversions
-        hi[i] = __byte_perm(__float_as_uint(v[2 * i]), __float_as_uint(v[2 * i + 1]), 0x7632) & 0x3fff3fffu;
-        lo[i] = __byte_perm(__float_as_uint(v[2 * i]), __float_as_uint(v[2 * i + 1]), 0x5410) & 0x3fff3fffu;
-#else
         const __half2 h = __floats2half2_rn(v[2 * i], v[2 * i + 1]);
         const float2 hf = __half22float2(h);
         const __half2 l = __floats2half2_rn(v[2 * i] - hf.x, v[2 * i + 1] - hf.y);
         hi[i] = *reinterpret_cast<const uint32_t*>(&h);
         lo[i] = *reinterpret_cast<const uint32_t*>(&l);
-#endif
     }
     tmem_st4(t_hi, hi[0], hi[1], hi[2], hi[3]);
     *reinterpret_cast<uint4*>(dst_lo) = make_uint4(lo[0], lo[1], lo[2], lo[3]);
@@ -377,17 +323,13 @@ __device__ __forceinline__ void build_a_slices(const float* __restrict__ srow, i
         const float4 e0 = *reinterpret_cast<const float4*>(pe), e1 = *reinterpret_cast<const float4*>(srow + (staged_index(base + 392 - n0) ^ 4));
         xe[0] = *pe8; xe[1] = e1.w; xe[2] = e1.z; xe[3] = e1.y; xe[4] = e1.x; xe[5] = e0.w; xe[6] = e0.z; xe[7] = e0.y;
     }
-#if ACBG_ABLATE == 2   // no sample loads
-#pragma unroll
-    for (int i = 0; i < 8; ++i) { xa[i] = 0.25f * i + n0; xb[i] = 0.5f; xc[i] = 1.f + n0; xe[i] = 0.125f * i; }
-#endif
     Fold8 f;
     {
         const float4 wf0 = *reinterpret_cast<const float4*>(s_wf + n0), wf1 = *reinterpret_cast<const float4*>(s_wf + n0 + 4);
         const float4 wr0 = *reinterpret_cast<const float4*>(s_wr + n0), wr1 = *reinterpret_cast<const float4*>(s_wr + n0 + 4);
         float wa[8] = {wf0.x, wf0.y, wf0.z, wf0.w, wf1.x, wf1.y, wf1.z, wf1.w};
         float wb[8] = {wr0.x, wr0.y, wr0.z, wr0.w, wr1.x, wr1.y, wr1.z, wr1.w};
-        if (ACBG_PRESCALE && pre != 1.f) {      // warp-uniform: the clip's power-of-two pre-scale (exact), folded into the window
+        if (pre != 1.f) {      // warp-uniform: the clip's power-of-two pre-scale (exact), folded into the window
 #pragma unroll
             for (int i = 0; i < 8; ++i) { wa[i] *= pre; wb[i] *= pre; }
         }
@@ -402,62 +344,10 @@ __device__ __forceinline__ void build_a_slices(const float* __restrict__ srow, i
             f.dd[i] = dn + dr;
         }
     }
-#if ACBG_ABLATE == 3   // no operand stores (and, as dead code, no conversions)
-    if (f.se[0] == 1234.5f && f.so[1] == 3.25f && f.de[2] == 7.f && f.dd[3] == 1.f) dst[0] = 1;
-    (void)t_hi;
-#elif ACBG_A_HI_TMEM
     split_store_tmem(f.se, t_hi + 0, dst + 1 * kASliceBytes);
     split_store_tmem(f.so, t_hi + 8, dst + 3 * kASliceBytes);
     split_store_tmem(f.de, t_hi + 16, dst + 5 * kASliceBytes);
     split_store_tmem(f.dd, t_hi + 24, dst + 7 * kASliceBytes);
-    tmem_st_wait();
-#else
-    (void)t_hi;
-    split_store(f.se, dst + 0 * kASliceBytes, dst + 1 * kASliceBytes);
-    split_store(f.so, dst + 2 * kASliceBytes, dst + 3 * kASliceBytes);
-    split_store(f.de, dst + 4 * kASliceBytes, dst + 5 * kASliceBytes);
-    split_store(f.dd, dst + 6 * kASliceBytes, dst + 7 * kASliceBytes);
-#endif
-}
-
-// Experiment (ACBG_PREP_WARPS == 16): 4 consecutive n per thread; hi halves -> 2 TMEM columns, lo halves -> one 8-byte store
-__device__ __forceinline__ void split_store_tmem4(const float (&v)[4], uint32_t t_hi, uint8_t* dst_lo) {
-    uint32_t hi[2], lo[2];
-#pragma unroll
-    for (int i = 0; i < 2; ++i) {
-        const __half2 h = __floats2half2_rn(v[2 * i], v[2 * i + 1]);
-        const float2 hf = __half22float2(h);
-        const __half2 l = __floats2half2_rn(v[2 * i] - hf.x, v[2 * i + 1] - hf.y);
-        hi[i] = *reinterpret_cast<const uint32_t*>(&h);
-        lo[i] = *reinterpret_cast<const uint32_t*>(&l);
-    }
-    tmem_st2(t_hi, hi[0], hi[1]);
-    *reinterpret_cast<uint2*>(dst_lo) = make_uint2(lo[0], lo[1]);
-}
-__device__ __forceinline__ void build_a_slices4(const float* __restrict__ srow, int base, int n0, const float* __restrict__ s_wf,
-                                                const float* __restrict__ s_wr, uint8_t* dst, uint32_t t_hi, float pre) {
-    const float4 a = *reinterpret_cast<const float4*>(srow + staged_index(base + n0));              // x[n0 .. n0+3]
-    const float4 c = *reinterpret_cast<const float4*>(srow + staged_index(base + 200 + n0));        // x[200+n0 .. 200+n0+3]
-    const float4 b = *reinterpret_cast<const float4*>(srow + staged_index(base + 196 - n0));        // x[196-n0 .. 199-n0]
-    const float b4 = srow[staged_index(base + 200 - n0)];                                            // x[200-n0]
-    const float4 e = *reinterpret_cast<const float4*>(srow + staged_index(base + 396 - n0));        // x[396-n0 .. 399-n0]
-    const float e4 = srow[staged_index(base + (n0 == 0 ? 0 : 400 - n0))];                            // x[400-n0], index taken mod 400
-    const float4 wf = *reinterpret_cast<const float4*>(s_wf + n0), wr = *reinterpret_cast<const float4*>(s_wr + n0);
-    const float xa[4] = {a.x, a.y, a.z, a.w}, xc[4] = {c.x, c.y, c.z, c.w};
-    const float xb[4] = {b4, b.w, b.z, b.y}, xe[4] = {e4, e.w, e.z, e.y};
-    const float wa[4] = {wf.x * pre, wf.y * pre, wf.z * pre, wf.w * pre}, wb[4] = {wr.x * pre, wr.y * pre, wr.z * pre, wr.w * pre};
-    float se[4], so[4], de[4], dd[4];
-#pragma unroll
-    for (int i = 0; i < 4; ++i) {
-        const float pa = wa[i] * xa[i], pe = wa[i] * xe[i];
-        const float pb = wb[i] * xb[i], pc = wb[i] * xc[i];
-        const float sn = pa + pc, sr = pb + pe, dn = pa - pc, dr = pb - pe;
-        se[i] = sn + sr; so[i] = sn - sr; de[i] = dn - dr; dd[i] = dn + dr;
-    }
-    split_store_tmem4(se, t_hi + 0, dst + 1 * kASliceBytes);
-    split_store_tmem4(so, t_hi + 8, dst + 3 * kASliceBytes);
-    split_store_tmem4(de, t_hi + 16, dst + 5 * kASliceBytes);
-    split_store_tmem4(dd, t_hi + 24, dst + 7 * kASliceBytes);
     tmem_st_wait();
 }
 
@@ -538,15 +428,6 @@ __global__ void __launch_bounds__(kThreads, 1) dftgemm_logmel_kernel(const Param
     const int n_tiles = p.n_clips * p.tiles_per_clip;
     bool ok = (smem_u32(smem) & 1023u) == 0;       // the swizzled sample tile needs a 1 KB aligned base
 
-    // development timeline (acb_dftgemm_set_trace): role 0 = worker warp 0, 1 = issuer, 2 = loader; CTA 0, first 8 tiles
-    auto stamp = [&](int role, uint32_t tile_iter, int event) {
-#ifdef ACB_DEV
-        if (p.trace && blockIdx.x == 0 && lane == 0 && tile_iter < 48 && event < 16) p.trace[(role * 48 + tile_iter) * 16 + event] = clock64();
-#else
-        (void)role; (void)tile_iter; (void)event;
-#endif
-    };
-
     if (warp == kWorkerWarps + 1) {
         // ======================================= B-slice loader =======================================
         // Streams the 28 KB of DFT-matrix slices of every K step from L2 as soon as the stage's previous MMAs have completed,
@@ -574,7 +455,6 @@ __global__ void __launch_bounds__(kThreads, 1) dftgemm_logmel_kernel(const Param
                     if (gs + ks >= 2) ok = mbar_wait(bar_mma0 + 8 * st, (use - 1) & 1u) && ok;      // the stage's previous MMAs are complete
                     // the epilogue of the previous tile keeps |X|^2 in the operand stages: wait until it is done with them
                     if (ks == 0 && tile_iter > 0) ok = mbar_wait(bar_tfree, (tile_iter - 1) & 1u) && ok;
-                    stamp(2, tile_iter, ks);        // B copy of step ks issued
                     mbar_arrive_expect_tx(bar_bfull0 + 8 * st, kBStageBytes);
                     bulk_copy_g2s(smem_u32(s_b + st * kBStageBytes), p.b_slices + (size_t)ks * kBStageBytes, kBStageBytes, bar_bfull0 + 8 * st);
                 }
@@ -582,7 +462,6 @@ __global__ void __launch_bounds__(kThreads, 1) dftgemm_logmel_kernel(const Param
             gs += kKsteps;
             __syncwarp();
             ok = mbar_wait(bar_sfree, tile_iter & 1u) && ok;      // every worker is past its last read of the sample tile
-            stamp(2, tile_iter, 8);
             if (tile + (int)gridDim.x < n_tiles) fetch_samples(tile + gridDim.x);
         }
     } else if (warp == kWorkerWarps) {
@@ -594,31 +473,19 @@ __global__ void __launch_bounds__(kThreads, 1) dftgemm_logmel_kernel(const Param
                 for (int ks = 0; ks < kKsteps; ++ks, ++gs) {
                     const uint32_t st = gs & 1u, use = gs >> 1;
                     ok = mbar_wait(bar_afull0 + 8 * st, use & 1u) && ok;      // A slices written by the worker warps
-                    stamp(1, tile_iter, 2 * ks);
                     ok = mbar_wait(bar_bfull0 + 8 * st, use & 1u) && ok;      // B slices landed (implies: accumulators drained, see the loader)
-                    stamp(1, tile_iter, 2 * ks + 1);
                     tc_fence_after();
                     const uint32_t a_base = smem_u32(s_a + st * kAStageBytes), b_base = smem_u32(s_b + st * kBStageBytes);
 #pragma unroll
                     for (int g = 0; g < kGemms; ++g) {
-                        const uint64_t a_hi = make_desc(a_base + (2 * g) * kASliceBytes, kTileFrames * 16, 128);
+                        const uint32_t a_hi = tmem + (uint32_t)(kAhiCols + st * 32 + g * 8);
                         const uint64_t a_lo = make_desc(a_base + (2 * g + 1) * kASliceBytes, kTileFrames * 16, 128);
                         const uint64_t b_hi = make_desc(b_base + (2 * g) * kBSliceBytes, 128, 256);
                         const uint64_t b_lo = make_desc(b_base + (2 * g + 1) * kBSliceBytes, 128, 256);
                         const uint32_t d = tmem + (uint32_t)(g * kNpad);
-#if ACBG_ABLATE == 4   // no MMAs (the commits still arrive)
-                        (void)a_hi; (void)a_lo; (void)b_hi; (void)b_lo; (void)d;
-#elif ACBG_A_HI_TMEM
-                        const uint32_t a_hi_t = tmem + (uint32_t)(kAhiCols + st * 32 + g * 8);
-                        (void)a_hi;
-                        mma_f16_ts(d, a_hi_t, b_hi, idesc, ks > 0);
+                        mma_f16_ts(d, a_hi, b_hi, idesc, ks > 0);
                         mma_f16_ss(d, a_lo, b_hi, idesc, 1);
-                        mma_f16_ts(d, a_hi_t, b_lo, idesc, 1);
-#else
-                        mma_f16_ss(d, a_hi, b_hi, idesc, ks > 0);
-                        mma_f16_ss(d, a_lo, b_hi, idesc, 1);
-                        mma_f16_ss(d, a_hi, b_lo, idesc, 1);
-#endif
+                        mma_f16_ts(d, a_hi, b_lo, idesc, 1);
                     }
                     mma_commit(bar_mma0 + 8 * st);
                     if (ks == kKsteps - 1) mma_commit(bar_tile);
@@ -699,7 +566,6 @@ __global__ void __launch_bounds__(kThreads, 1) dftgemm_logmel_kernel(const Param
             } else {
                 worker_sync();   // gathered samples visible
             }
-            if (warp == 0) stamp(0, tile_iter, 0);      // samples ready
             // ---------------- K loop: build the A slices of each step ----------------
             const int base = kHop * row + 120;
             if (warp < kPrepWarps) {
@@ -707,19 +573,13 @@ __global__ void __launch_bounds__(kThreads, 1) dftgemm_logmel_kernel(const Param
                 for (int ks = 0; ks < kKsteps; ++ks) {
                     const uint32_t st = (gs + ks) & 1u, use = (gs + ks) >> 1;
                     if (gs + ks >= 2) ok = mbar_wait(bar_mma0 + 8 * st, (use - 1) & 1u) && ok;   // MMAs that read this stage are complete
-                    if (kPrepWarps == 8)
-                        build_a_slices(s_samples, base, 16 * ks + 8 * hsel, s_wf, s_wr,
-                                       s_a + st * kAStageBytes + hsel * (kTileFrames * 16) + row * 16,
-                                       tmem + ((uint32_t)((warp & 3) << 5) << 16) + (uint32_t)(kAhiCols + st * 32 + hsel * 4), pre);
-                    else
-                        build_a_slices4(s_samples, base, 16 * ks + 4 * qsel, s_wf, s_wr,
-                                        s_a + st * kAStageBytes + (qsel >> 1) * (kTileFrames * 16) + row * 16 + (qsel & 1) * 8,
-                                        tmem + ((uint32_t)((warp & 3) << 5) << 16) + (uint32_t)(kAhiCols + st * 32 + qsel * 2), pre);
-                    if (ACBG_ABLATE != 1) fence_async_smem();      // generic-proxy writes of A -> visible to the tensor core's async proxy
+                    build_a_slices(s_samples, base, 16 * ks + 8 * hsel, s_wf, s_wr,
+                                   s_a + st * kAStageBytes + hsel * (kTileFrames * 16) + row * 16,
+                                   tmem + ((uint32_t)((warp & 3) << 5) << 16) + (uint32_t)(kAhiCols + st * 32 + hsel * 4), pre);
+                    fence_async_smem();      // generic-proxy writes of A -> visible to the tensor core's async proxy
                     tc_fence_before();       // (and the tensor-memory stores of A_hi, completed by tcgen05.wait::st, ordered before the arrive)
                     __syncwarp();
                     if (lane == 0) mbar_arrive(bar_afull0 + 8 * st);
-                    if (warp == 0) stamp(0, tile_iter, 1 + ks);
                 }
                 // this warp is past its last read of the sample tile: tell the loader, which prefetches an interior next tile
                 __syncwarp();
@@ -742,7 +602,6 @@ __global__ void __launch_bounds__(kThreads, 1) dftgemm_logmel_kernel(const Param
             // ---------------- epilogue: |X|^2 -> shared memory, banded mel, log, store ----------------
             ok = mbar_wait(bar_tile, tile_iter & 1u) && ok;      // every MMA of the tile is complete: accumulators ready, stages idle
             tc_fence_after();
-            if (warp == 0) stamp(0, tile_iter, 8);
             {
                 // power pass: the 4 warps of a lane quarter share the 14 units of 8 accumulator columns (16 bins); s_pow[bin][row]
                 // (a warp writes 32 consecutive rows: conflict-free)
@@ -764,7 +623,6 @@ __global__ void __launch_bounds__(kThreads, 1) dftgemm_logmel_kernel(const Param
                 }
                 tc_fence_before();
                 worker_sync();       // the whole power tile is in shared memory; the accumulators are drained
-                if (warp == 0) stamp(0, tile_iter, 9);
 
                 // mel pass: lane = 4 consecutive frames (one 16-byte load per bin), warp = one group of bands (weights are
                 // warp-uniform broadcast loads); a warp stores 32 x 4 consecutive frames of one band = 512 contiguous bytes
@@ -794,7 +652,7 @@ __global__ void __launch_bounds__(kThreads, 1) dftgemm_logmel_kernel(const Param
                         a.z = fmaf(w, q.z, a.z);
                         a.w = fmaf(w, q.w, a.w);
                     }
-                    if (ACBG_CHK) chk += (a.x + a.y) + (a.z + a.w);          // inf / NaN powers (operand overflow) must not hide behind the clamp
+                    chk += (a.x + a.y) + (a.z + a.w);          // inf / NaN powers (operand overflow) must not hide behind the clamp
                     // the factor that undoes the pre-scale / applies the peak gain moves through the log: log(a post) = log a + log post,
                     // and the clamp is compared against clamp_min / post
                     float4 v;
@@ -860,9 +718,7 @@ __global__ void __launch_bounds__(kThreads, 1) dftgemm_logmel_kernel(const Param
                     for (int o = 16; o >= 1; o >>= 1) vmin = fminf(vmin, __shfl_xor_sync(0xffffffffu, vmin, o));
                     if (lane == 0 && vmin < 3.0e38f) atomicMax(p.tile_min + tile, float_key(-vmin));   // key of -min: same initial pattern as clip_max
                 }
-                if (warp == 0) stamp(0, tile_iter, 10);
                 worker_sync();       // nobody reads the power tile any more: the operand stages may be refilled
-                if (warp == 0) stamp(0, tile_iter, 11);
                 if (lane == 0) mbar_arrive(bar_tfree);
             }
             smp_async = next_async;
@@ -967,7 +823,6 @@ struct acb_dftgemm {
     const float* d_melw = nullptr;
     int n_mel_w = 0;
     int* d_err = nullptr;
-    long long* d_trace = nullptr;   // development timeline buffer (acb_dftgemm_set_trace)
 };
 
 using namespace acbg;
@@ -1211,7 +1066,6 @@ int acb_dftgemm_forward(const acb_dftgemm* fe, const acb_dftgemm_args* a, void* 
     p.drop_last_frame = a->drop_last_frame;
     p.fill_value = a->fill_value;
     p.error_flag = fe->d_err;
-    p.trace = fe->d_trace;
     if (p.clip_max)   // one fill for both arrays: keys below every float (tile_min holds keys of the negated minimum)
         ACBG_CUDA(cudaMemsetAsync(p.clip_max, 0x80, sizeof(int) * (size_t)a->n_clips * (size_t)(1 + tiles_per_clip), s));
     const int64_t n_tiles = tiles_per_clip * a->n_clips;
@@ -1249,15 +1103,6 @@ int acb_dftgemm_forward(const acb_dftgemm* fe, const acb_dftgemm_args* a, void* 
     }
     return ACB_OK;
 }
-
-#ifdef ACB_DEV
-/* development only (not in the public header, -DACB_DEV builds): device buffer of 3 * 48 * 16 int64 clock stamps written by CTA 0, or NULL */
-int acb_dftgemm_set_trace(acb_dftgemm* fe, long long* device_buffer) {
-    if (!fe) return fail(ACB_ERR_INVALID, "acb_dftgemm_set_trace: null handle");
-    fe->d_trace = device_buffer;
-    return ACB_OK;
-}
-#endif
 
 int acb_dftgemm_check(const acb_dftgemm* fe, void* stream) {
     if (!fe) return fail(ACB_ERR_INVALID, "acb_dftgemm_check: null handle");

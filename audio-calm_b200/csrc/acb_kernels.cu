@@ -9,9 +9,10 @@
 // Every input sample is read from HBM once (plus a 3/16 halo served by L2) and every output value is
 // written once.
 //
-// Structure: a CTA (256 threads, 2 CTAs per SM) holds TWO independent groups of 4 warps; a group owns a contiguous range
-// of 8-frame tiles, its own sample buffer, scratch and named barrier, so four groups per SM run out of phase and the
-// FMA-heavy and the shared-memory-heavy parts of different groups overlap.  Per tile a group does:
+// Structure: a CTA holds G independent groups of 4 warps: 4 groups in one 512-thread CTA per SM by default, or 2 groups in
+// each of 2 CTAs per SM when a large filterbank plan does not leave room for four groups' buffers.  A group owns a contiguous
+// range of 8-frame tiles, its own sample buffer, scratch and named barrier, so the four groups of an SM run out of phase and
+// the FMA-heavy and the shared-memory-heavy parts of different groups overlap.  Per tile a group does:
 //   1. one bulk async copy (cp.async.bulk + mbarrier) brings the tile's (8+3)*256 samples into shared memory (edge tiles,
 //      which need reflection, are gathered by the group);
 //   2. each warp takes one pair of adjacent frames (A, B) and runs ONE complex 1024-point FFT of
@@ -38,20 +39,6 @@
 #include <numeric>
 #include <string>
 #include <vector>
-
-// Development-only ablation switch, compiled in only with -DACB_DEV (tools/ablate.py builds variants with
-// -DACB_DEV -DACB_ABLATE=n to price each part of the kernel in situ; results are wrong for n != 0).
-#if !defined(ACB_DEV) || !defined(ACB_ABLATE)
-#undef ACB_ABLATE
-#define ACB_ABLATE 0
-#endif
-
-#ifndef ACB_WIN_FUSE
-#define ACB_WIN_FUSE 1
-#endif
-#ifndef ACB_WIN_T
-#define ACB_WIN_T 1
-#endif
 
 namespace acb {
 
@@ -457,10 +444,8 @@ __global__ void __launch_bounds__(G * kGroupThreads, G == 4 ? 1 : 2) logmel_fuse
 
     // ---- one-time table staging (whole CTA) ----
     for (int i = tid; i < 5 * 32; i += kThreads) s_tw4[i] = p.twiddle[i];
-    for (int i = tid; i < kNfft / 2; i += kThreads) {
-        if (ACB_WIN_T) s_win[(i & 31) * 20 + (i >> 5)] = p.window[i];      // [lane][row], 20-float pitch: conflict-free 16-byte loads
-        else s_win[i] = p.window[i];
-    }
+    for (int i = tid; i < kNfft / 2; i += kThreads)
+        s_win[(i & 31) * 20 + (i >> 5)] = p.window[i];      // [lane][row], 20-float pitch: conflict-free 16-byte loads
     for (int i = tid; i < p.n_plan_w; i += kThreads) s_pw[i] = p.plan_w[i];
     for (int i = tid; i < kGroupWarps * kMaxRounds * kSlots; i += kThreads) {
         const int slot = i / kSlots, qq = i - slot * kSlots;
@@ -512,7 +497,7 @@ __global__ void __launch_bounds__(G * kGroupThreads, G == 4 ? 1 : 2) logmel_fuse
 
         const int f0 = cur.tile_in_clip * kTileFrames;
         const bool has_frames = f0 < cur.frames;  // false for pure tail-fill tiles
-        const bool active = has_frames && f0 + 2 * gw < cur.frames && ACB_ABLATE != 7;   // this warp's frame pair exists
+        const bool active = has_frames && f0 + 2 * gw < cur.frames;   // this warp's frame pair exists
 
         // ================= phase 1: one frame pair per warp =================
         // The first FFT-32 needs only the samples and registers, so it runs BEFORE the barrier that frees the scratch: a warp that
@@ -527,33 +512,21 @@ __global__ void __launch_bounds__(G * kGroupThreads, G == 4 ? 1 : 2) logmel_fuse
                 float2 v[20];
 #pragma unroll
                 for (int r = 0; r < 20; ++r) v[r] = make_float2(sp[32 * (2 * r)], sp[32 * (2 * r + 1)]);
+                // the lane's 16 window values, stored per lane: four 16-byte loads instead of sixteen 4-byte ones
                 float4 w4[4];
-                if (ACB_WIN_T) {   // the lane's 16 window values, stored per lane: four 16-byte loads instead of sixteen 4-byte ones
-                    const float4* wq = reinterpret_cast<const float4*>(s_win + lane * 20);
+                const float4* wq = reinterpret_cast<const float4*>(s_win + lane * 20);
 #pragma unroll
-                    for (int u = 0; u < 4; ++u) w4[u] = wq[u];
-                }
+                for (int u = 0; u < 4; ++u) w4[u] = wq[u];
 #pragma unroll
                 for (int j = 0; j < 8; ++j) {
                     const int t = brev5(2 * j) >> 1;      // sample rows n1 = 2t, 2t + 1 (n1 < 16)
-                    const float2 wa = ACB_WIN_T ? ((t & 1) ? make_float2(w4[t >> 1].z, w4[t >> 1].w) : make_float2(w4[t >> 1].x, w4[t >> 1].y))
-                                                : make_float2(s_win[32 * (2 * t) + lane], s_win[32 * (2 * t + 1) + lane]);
-#if ACB_WIN_FUSE
+                    const float2 wa = (t & 1) ? make_float2(w4[t >> 1].z, w4[t >> 1].w) : make_float2(w4[t >> 1].x, w4[t >> 1].y);
                     // periodic Hann: w[n + N/2] = 1 - w[n], so b (1 - w) = b - b w is one FMA, and a w +- that another
                     const float2 br = __ffma2_rn(neg2(v[t + 8]), wa, v[t + 8]), bi = __ffma2_rn(neg2(v[t + 12]), wa, v[t + 12]);
                     pr[2 * j] = __ffma2_rn(v[t], wa, br);
                     pr[2 * j + 1] = __ffma2_rn(v[t], wa, neg2(br));
                     pi[2 * j] = __ffma2_rn(v[t + 4], wa, bi);
                     pi[2 * j + 1] = __ffma2_rn(v[t + 4], wa, neg2(bi));
-#else
-                    const float2 wb = __fadd2_rn(bcast2(1.f), neg2(wa));   // periodic Hann: w[n + N/2] = 1 - w[n]
-                    const float2 ar = __fmul2_rn(v[t], wa), br = __fmul2_rn(v[t + 8], wb);
-                    const float2 ai = __fmul2_rn(v[t + 4], wa), bi = __fmul2_rn(v[t + 12], wb);
-                    pr[2 * j] = __fadd2_rn(ar, br);
-                    pr[2 * j + 1] = __fadd2_rn(ar, neg2(br));
-                    pi[2 * j] = __fadd2_rn(ai, bi);
-                    pi[2 * j + 1] = __fadd2_rn(ai, neg2(bi));
-#endif
                 }
             }
             fft32_packed_from_stage2(pr, pi);  // over n1 -> k1 (natural order)
@@ -650,7 +623,7 @@ __global__ void __launch_bounds__(G * kGroupThreads, G == 4 ? 1 : 2) logmel_fuse
         const bool direct = !p.time_major && (f0 + kTileFrames - 1 <= cur.frames - 2 - pad);
 
         // ================= phase 2: banded mel projection, clamp, log, affine, moments =================
-        if (has_frames && ACB_ABLATE != 8) {
+        if (has_frames) {
             const int fA = f0 + 2 * pl;
             OutT* out_clip = reinterpret_cast<OutT*>(p.out) + cur.out_base;
             const bool pair_store = ((cur.cap & 1) == 0) && ((reinterpret_cast<uintptr_t>(out_clip) & (2 * sizeof(OutT) - 1)) == 0);
@@ -664,7 +637,7 @@ __global__ void __launch_bounds__(G * kGroupThreads, G == 4 ? 1 : 2) logmel_fuse
                 const float4* p4 = reinterpret_cast<const float4*>(pair_scratch) + rec.x;   // two bins x (A, B)
                 const float2* w2 = reinterpret_cast<const float2*>(s_pw) + rec.y;
                 float acc0 = 0.f, acc1 = 0.f, acc2 = 0.f, acc3 = 0.f;
-                const int half_trip = ACB_ABLATE == 4 ? 0 : (trip >> 1);
+                const int half_trip = trip >> 1;
 #pragma unroll 4
                 for (int i = 0; i < half_trip; ++i) {
                     const float4 pw = p4[i];

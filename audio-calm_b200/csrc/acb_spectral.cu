@@ -21,27 +21,15 @@ namespace acb {
 int fail(int code, const std::string& msg);   // acb_kernels.cu: sets the thread-local message behind acb_last_error()
 }
 
-#ifndef ACB_STFT_RPC
-#define ACB_STFT_RPC 32      // rows staged per CTA (upper bound)
-#endif
-#ifndef ACB_STFTC_FPC
-#define ACB_STFTC_FPC 4      // frames per CTA of the complex STFT (Griffin-Lim), upper bound
-#endif
-#ifndef ACB_ISTFT_FPC
-#define ACB_ISTFT_FPC 4      // frames per CTA of the inverse STFT, upper bound
-#endif
-#ifndef ACB_STFT_BWD_RPC
-#define ACB_STFT_BWD_RPC 16  // rows per CTA of the backward kernel
-#endif
-#ifndef ACB_STFT_DIRECT
-#define ACB_STFT_DIRECT 1    // 1: magnitudes go straight to global memory (L2 merges the 4-byte stores of a row block); 0: staged in shared memory
-#endif
-
 namespace acb_spectral {
 
 using namespace acb;
 
 constexpr int kThreads = 128;
+constexpr int kStftRowsPerCta = 32;          // rows staged per CTA (upper bound)
+constexpr int kStftComplexFramesPerCta = 4;  // frames per CTA of the complex STFT (Griffin-Lim), upper bound
+constexpr int kIstftFramesPerCta = 4;        // frames per CTA of the inverse STFT, upper bound
+constexpr int kStftBwdRowsPerCta = 16;       // rows per CTA of the backward kernel
 
 __host__ __device__ constexpr int brev_bits(int x, int bits) {
     int r = 0;
@@ -200,18 +188,17 @@ __device__ __forceinline__ void load_pair_windowed(const float* s_x, int base_a,
 }
 
 struct SpectralSmem {
-    int x, win, tw, buf, out, total_bytes;
+    int x, win, tw, buf, total_bytes;
 };
 
-__host__ __device__ inline SpectralSmem spectral_smem(int R, int rows_per_cta, int T, int n_frames) {
-    const int N = 32 * R, n_freq = N / 2 + 1;
+__host__ __device__ inline SpectralSmem spectral_smem(int R, int rows_per_cta, int T) {
+    const int N = 32 * R;
     SpectralSmem L;
     int off = 0;   // 4-byte words
     L.x = off; off += (rows_per_cta * T + 255) & ~255;           // the swizzle permutes inside aligned 256-float blocks
     L.win = off; off += N;
     L.tw = off; off += 2 * N;
     L.buf = off; off += (kThreads / R) * (2 * 33 * R);           // per lane group: N complex values, index k1 + 33 * k2
-    L.out = off; if (!ACB_STFT_DIRECT) off += rows_per_cta * n_freq * n_frames;
     L.total_bytes = off * 4;
     return L;
 }
@@ -221,11 +208,10 @@ __global__ void __launch_bounds__(kThreads) stft_mag_kernel(const float* __restr
                                                             const float* __restrict__ window, float* __restrict__ out, int rows_per_cta) {
     constexpr int N = 32 * R, kFreq = N / 2 + 1, kGroups = kThreads / R, kPerLane = 32 / R;
     extern __shared__ __align__(16) float smem[];
-    const SpectralSmem L = spectral_smem(R, rows_per_cta, T, n_frames);
+    const SpectralSmem L = spectral_smem(R, rows_per_cta, T);
     float* s_x = smem + L.x;
     float* s_win = smem + L.win;
     float2* s_tw = reinterpret_cast<float2*>(smem + L.tw);
-    float* s_out = smem + L.out;
     const int tid = threadIdx.x;
     const long long row0 = (long long)blockIdx.x * rows_per_cta;
     const int n_rows = (int)min((long long)rows_per_cta, rows - row0);
@@ -272,7 +258,7 @@ __global__ void __launch_bounds__(kThreads) stft_mag_kernel(const float* __restr
         if (valid) group_fft_stage2<R>(buf, r);
         __syncwarp();
         if (valid) {                                    // separate the two real spectra, magnitudes
-            float* obase = ACB_STFT_DIRECT ? out + row0 * kFreq * n_frames : s_out;
+            float* obase = out + row0 * kFreq * n_frames;
             float* oa = obase + (size_t)row_a * kFreq * n_frames + fa;
             float* ob = obase + (size_t)row_b * kFreq * n_frames + fb;
             for (int k = r; k < kFreq; k += R) {
@@ -285,18 +271,6 @@ __global__ void __launch_bounds__(kThreads) stft_mag_kernel(const float* __restr
         }
         __syncwarp();
     }
-    if (ACB_STFT_DIRECT) return;
-    __syncthreads();
-    {   // the CTA's rows are one contiguous span of the output
-        float* dst = out + row0 * kFreq * n_frames;
-        const int n = n_rows * kFreq * n_frames;
-        if ((reinterpret_cast<uintptr_t>(dst) & 15) == 0 && (L.out & 3) == 0) {
-            for (int i = tid; i < n / 4; i += kThreads) reinterpret_cast<float4*>(dst)[i] = reinterpret_cast<const float4*>(s_out)[i];
-            for (int i = (n & ~3) + tid; i < n; i += kThreads) dst[i] = s_out[i];
-        } else {
-            for (int i = tid; i < n; i += kThreads) dst[i] = s_out[i];
-        }
-    }
 }
 
 template <int R>
@@ -306,10 +280,10 @@ static int launch(const float* x, int64_t rows, int T, int hop, int n_frames, co
         return fail(ACB_ERR_CUDA, "acb_stft_mag: cannot query the device");
     // rows per CTA: 16 (measured best for 5-13 frames per row), doubled while a CTA's frame pairs would leave lane groups idle
     // (one frame per row at n_fft = T), halved while the footprint is large
-    int rpc = (int)std::max<int64_t>(1, std::min<int64_t>(std::min<int64_t>(16, ACB_STFT_RPC), 16384 / T));
-    while (rpc < ACB_STFT_RPC && (rpc * n_frames + 1) / 2 < kThreads / R && 2 * rpc <= 16384 / T) rpc <<= 1;
-    while (rpc > 1 && spectral_smem(R, rpc, T, n_frames).total_bytes > std::min(optin, 160 * 1024)) rpc >>= 1;
-    const SpectralSmem L = spectral_smem(R, rpc, T, n_frames);
+    int rpc = (int)std::max<int64_t>(1, std::min<int64_t>(std::min<int64_t>(16, kStftRowsPerCta), 16384 / T));
+    while (rpc < kStftRowsPerCta && (rpc * n_frames + 1) / 2 < kThreads / R && 2 * rpc <= 16384 / T) rpc <<= 1;
+    while (rpc > 1 && spectral_smem(R, rpc, T).total_bytes > std::min(optin, 160 * 1024)) rpc >>= 1;
+    const SpectralSmem L = spectral_smem(R, rpc, T);
     if (L.total_bytes > optin)
         return fail(ACB_ERR_UNSUPPORTED, "acb_stft_mag: a row of " + std::to_string(T) + " frames does not fit in shared memory");
     cudaError_t e = cudaFuncSetAttribute(stft_mag_kernel<R>, cudaFuncAttributeMaxDynamicSharedMemorySize, optin);
@@ -477,7 +451,7 @@ static int launch_backward(const float* x, const float* grad_mag, int64_t rows, 
         return fail(ACB_ERR_CUDA, "acb_stft_mag_backward: cannot query the device");
     // rows per CTA: 16, or 8 when a row has many frames (measured at T = 256: 13 frames per row run 25 % faster in one pass over 8 rows than
     // in two passes over 16 with twice the shared memory)
-    int rpc = (int)std::max<int64_t>(1, std::min<int64_t>(n_frames >= 8 ? ACB_STFT_BWD_RPC / 2 : ACB_STFT_BWD_RPC, 16384 / T));
+    int rpc = (int)std::max<int64_t>(1, std::min<int64_t>(n_frames >= 8 ? kStftBwdRowsPerCta / 2 : kStftBwdRowsPerCta, 16384 / T));
     while (rpc > 1 && spectral_bwd_smem(R, rpc, T, n_frames).total_bytes > std::min(optin, 160 * 1024)) rpc >>= 1;
     const SpectralBwdSmem L = spectral_bwd_smem(R, rpc, T, n_frames);
     if (L.total_bytes > optin)
@@ -743,7 +717,7 @@ static int launch_stft_complex(const float* x, int64_t rows, int64_t length, int
     int dev = 0, optin = 0;
     if (cudaGetDevice(&dev) != cudaSuccess || cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev) != cudaSuccess)
         return fail(ACB_ERR_CUDA, "acb_stft_complex: cannot query the device");
-    int fpc = chunk_frames(ACB_STFTC_FPC, n_frames, rows);
+    int fpc = chunk_frames(kStftComplexFramesPerCta, n_frames, rows);
     while (fpc > 2 && chunk_smem(R, fpc, hop, false).total_bytes > std::min(optin, 160 * 1024)) fpc >>= 1;
     const ChunkSmem L = chunk_smem(R, fpc, hop, false);
     if (L.total_bytes > optin) return fail(ACB_ERR_UNSUPPORTED, "acb_stft_complex: hop too large for shared memory");
@@ -761,7 +735,7 @@ static int launch_istft(const float2* spec, int64_t rows, int n_frames, int hop,
     int dev = 0, optin = 0;
     if (cudaGetDevice(&dev) != cudaSuccess || cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev) != cudaSuccess)
         return fail(ACB_ERR_CUDA, "acb_istft: cannot query the device");
-    int fpc = chunk_frames(ACB_ISTFT_FPC, n_frames, rows);
+    int fpc = chunk_frames(kIstftFramesPerCta, n_frames, rows);
     while (fpc > 2 && chunk_smem(R, fpc, hop, true).total_bytes > std::min(optin, 160 * 1024)) fpc >>= 1;
     const ChunkSmem L = chunk_smem(R, fpc, hop, true);
     if (L.total_bytes > optin) return fail(ACB_ERR_UNSUPPORTED, "acb_istft: transform too large for shared memory");

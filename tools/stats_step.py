@@ -1,5 +1,5 @@
-"""Development: the config-2 launch and a 512-clip ragged statistics-only launch, timed for one build (ACB_LIB = a variant of
-tools/variants.py, default the in-tree library)."""
+"""Development: the config-2 launch and a 512-clip ragged statistics-only launch, timed for one build (ACB_LIB = the path of
+another build of the library, default the in-tree library)."""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch
