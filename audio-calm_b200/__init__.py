@@ -15,17 +15,22 @@ directory as that package.  Layout:
     collate.py               training-feed collation on the device (crop / zero-pad to 256 frames; ragged pad + transpose)
     spectral.py              VAE-side STFT magnitudes over the mel time axis (AcousticVAE._stft_mag / stft_loss forward)
     csrc/acb_spectral.cu     its kernel (shares the in-register FFT-32 of csrc/acb_fft32.cuh)
+    resample.py              Resampler: torchaudio.transforms.Resample (sinc_interp_hann) on the device, uniform and ragged
+    csrc/acb_resample.cu     its polyphase kernel (banded per-phase coefficients in registers)
     preprocess/              drop-in mirrors of the reference's preprocess/{core,compute_mel_stats,process_dataset}.py
 """
 from . import _lib, tables  # noqa: F401
-from .frontend import (LogMelFrontend, MEL_MEAN_DEFAULT, MEL_STD_DEFAULT, RaggedBatch, frames_for_length,  # noqa: F401
-                       pack_clips, padded_frames)
+from .frontend import (LogMelFrontend, MEL_MEAN_DEFAULT, MEL_STD_DEFAULT, RaggedBatch, empty_ragged,  # noqa: F401
+                       frames_for_length, pack_clips, padded_frames)
 from .stats import MelStats, MelStatsAccumulator, finalize_moments, normalize_per_utterance  # noqa: F401
 from . import collate, frontend, stats, sharding  # noqa: F401
 from .collate import crop_collate, pad_collate, pad_collate_packed  # noqa: F401
 from . import spectral, whisper  # noqa: F401
 from .whisper import WhisperLogMel, whisper_tables  # noqa: F401
+from . import resample  # noqa: F401
+from .resample import Resampler, resampled_length  # noqa: F401
 
 __all__ = ["LogMelFrontend", "MelStatsAccumulator", "MelStats", "RaggedBatch", "pack_clips", "frames_for_length",
-           "padded_frames", "finalize_moments", "normalize_per_utterance", "MEL_MEAN_DEFAULT", "MEL_STD_DEFAULT", "WhisperLogMel", "whisper_tables"]
+           "padded_frames", "finalize_moments", "normalize_per_utterance", "MEL_MEAN_DEFAULT", "MEL_STD_DEFAULT", "WhisperLogMel", "whisper_tables",
+           "Resampler", "resampled_length", "empty_ragged"]
 __version__ = "0.1.0"

@@ -18,7 +18,7 @@ CSRC = os.path.join(_HERE, "csrc")
 INCLUDE = os.path.join(os.path.dirname(_HERE), "include")
 LIB_NAME = "libaudiocalm_b200.so"
 LIB_PATH = os.path.join(CSRC, LIB_NAME)
-SOURCES = ["acb_kernels.cu", "acb_dftgemm.cu", "acb_spectral.cu"]
+SOURCES = ["acb_kernels.cu", "acb_dftgemm.cu", "acb_spectral.cu", "acb_resample.cu"]
 HEADERS = ["acb_fft32.cuh"]
 
 NVCC_FLAGS = [
@@ -28,7 +28,7 @@ NVCC_FLAGS = [
 ]
 
 ACB_OK = 0
-ACB_F32, ACB_BF16 = 0, 1
+ACB_F32, ACB_BF16, ACB_I16 = 0, 1, 2
 ACB_MEL_MAJOR, ACB_TIME_MAJOR = 0, 1
 ACB_LOG_NATURAL, ACB_LOG_10 = 0, 1
 
@@ -41,6 +41,7 @@ EXPORTED_SYMBOLS = [
     "acb_moments_accumulate_workspace_bytes", "acb_pcm16_to_float", "acb_logmel_forward_host_pcm16",
     "acb_stft_mag_frames", "acb_stft_mag", "acb_stft_mag_backward", "acb_stft_complex", "acb_istft",
     "acb_dftgemm_frames", "acb_dftgemm_workspace_ints", "acb_dftgemm_create", "acb_dftgemm_destroy", "acb_dftgemm_forward", "acb_dftgemm_check", "acb_dftgemm_moments_workspace_bytes",
+    "acb_resampled_length", "acb_resampler_create", "acb_resampler_destroy", "acb_resample",
 ]
 
 
@@ -227,6 +228,14 @@ def load() -> ctypes.CDLL:
         lib.acb_dftgemm_moments_workspace_bytes.argtypes = [vp]
         lib.acb_dftgemm_check.restype = ctypes.c_int
         lib.acb_dftgemm_check.argtypes = [vp, vp]
+        lib.acb_resampled_length.restype = i64
+        lib.acb_resampled_length.argtypes = [i64, ctypes.c_int, ctypes.c_int]
+        lib.acb_resampler_create.restype = ctypes.c_int
+        lib.acb_resampler_create.argtypes = [ctypes.POINTER(vp), ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_int, vp]
+        lib.acb_resampler_destroy.restype = ctypes.c_int
+        lib.acb_resampler_destroy.argtypes = [vp]
+        lib.acb_resample.restype = ctypes.c_int
+        lib.acb_resample.argtypes = [vp, vp, i32, vp, vp, i64, i64, i32, vp, vp, i64, vp]
         if lib.acb_abi_version() != 2:
             raise RuntimeError(f"{LIB_PATH}: ABI version {lib.acb_abi_version()} != 2; rebuild")
         _lib = lib

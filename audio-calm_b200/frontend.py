@@ -64,18 +64,38 @@ class RaggedBatch:
     plans: dict = field(default_factory=dict, repr=False, compare=False)
 
 
+def packed_layout(lengths: Sequence[int]) -> Tuple[np.ndarray, np.ndarray, int]:
+    """(lengths, starts, buffer size) of the packed layout: every clip starts at a multiple of 4 samples."""
+    lens = np.array([int(n) for n in lengths], dtype=np.int64)
+    starts = np.zeros(len(lens), dtype=np.int64)
+    if len(lens):
+        starts[1:] = np.cumsum((lens[:-1] + 3) & ~3)
+    total = max(int(starts[-1] + ((lens[-1] + 3) & ~3)) if len(lens) else 0, 4)
+    return lens, starts, total
+
+
+def empty_ragged(lengths: Sequence[int], device: torch.device, dtype: torch.dtype = torch.float32,
+                 buffer: Optional[torch.Tensor] = None) -> RaggedBatch:
+    """An uninitialised packed batch for clips of known ``lengths``: clip starts at multiples of 4 samples (16-byte aligned for
+    float32), lengths and offsets already on the device.  ``buffer``: a flat device tensor of ``dtype`` with at least the packed size
+    to lay the clips out at the start of (a caller can keep scratch rows behind them); ``None`` allocates one."""
+    lens, starts, total = packed_layout(lengths)
+    if buffer is None:
+        flat = torch.empty(total, dtype=dtype, device=device)
+    else:
+        if buffer.dim() != 1 or buffer.dtype != dtype or buffer.numel() < total or buffer.device != torch.device(device):
+            raise ValueError(f"buffer must be a flat {dtype} device tensor of at least {total} elements")
+        flat = buffer[:total]
+    return RaggedBatch(flat, torch.from_numpy(starts).to(device), torch.from_numpy(lens).to(device), lens)
+
+
 def pack_clips(clips: Sequence[torch.Tensor], device: torch.device) -> RaggedBatch:
     """Pack 1-D fp32 clips (host or device) into one flat device buffer with 16-byte aligned clip starts."""
-    lens = np.array([int(c.shape[-1]) for c in clips], dtype=np.int64)
-    starts = np.zeros(len(clips), dtype=np.int64)
-    pos = 0
-    for i, n in enumerate(lens):
-        starts[i] = pos
-        pos += (int(n) + 3) & ~3
-    flat = torch.empty(max(pos, 4), dtype=torch.float32, device=device)
+    lens, starts, _ = packed_layout([int(c.shape[-1]) for c in clips])
+    batch = empty_ragged(lens, device)
     for c, s, n in zip(clips, starts, lens):
-        flat[s:s + n].copy_(c.reshape(-1), non_blocking=True)
-    return RaggedBatch(flat, torch.from_numpy(starts).to(device), torch.from_numpy(lens).to(device), lens)
+        batch.wav[s:s + n].copy_(c.reshape(-1), non_blocking=True)
+    return batch
 
 
 class LogMelFrontend:

@@ -29,16 +29,18 @@ from typing import Callable, Dict, List, NamedTuple, Optional, Sequence, Tuple
 import torch
 
 try:
-    from ..frontend import LogMelFrontend, pack_clips
+    from ..frontend import LogMelFrontend, empty_ragged, packed_layout
     from .._lib import check as _lib_check
+    from ..resample import Resampler, resampled_length
     from ..sharding import contiguous_shard
     from .core import load_vae, process_audio_chunk  # noqa: F401
 except ImportError:  # run as a script / as top-level `preprocess.process_dataset`
     _root = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
     if _root not in sys.path:
         sys.path.insert(0, _root)
-    from audio_calm_b200.frontend import LogMelFrontend, pack_clips
+    from audio_calm_b200.frontend import LogMelFrontend, empty_ragged, packed_layout
     from audio_calm_b200._lib import check as _lib_check
+    from audio_calm_b200.resample import Resampler, resampled_length
     from audio_calm_b200.sharding import contiguous_shard
     from audio_calm_b200.preprocess.core import load_vae, process_audio_chunk  # noqa: F401
 
@@ -104,11 +106,12 @@ def transcript_for(wav_path: str, args, cv_mapping: Dict[str, str]) -> Optional[
     return None
 
 
-def load_audio(path: str) -> torch.Tensor:
-    """Decode (+ resample to 16 kHz) on the host: ``[C, L]`` (process_dataset.py:135-137).  I/O, not on the hot path.
+def decode_audio(path: str) -> Tuple[torch.Tensor, int]:
+    """Decode on the host without resampling: ``(wav [C, L], sample_rate)``.  I/O, not on the hot path.
 
-    16-bit files that already are 16 kHz come back as **int16**: the driver ships them as PCM (half the PCIe bytes) and widens them
-    on the device to ``x / 32768`` -- exactly what ``torchaudio.load`` (normalize=True) would have produced.  Everything else is float32."""
+    16-bit files come back as **int16** at any rate: the driver ships them as PCM (half the PCIe bytes of float32) and widens them on
+    the device to ``x / 32768`` -- exactly what ``torchaudio.load`` (normalize=True) would have produced.  Everything else is
+    float32, normalised like ``torchaudio.load``."""
     try:
         import torchaudio
         wav, sr = torchaudio.load(path, normalize=False)
@@ -117,20 +120,45 @@ def load_audio(path: str) -> torch.Tensor:
         import numpy as np
         sr, data = wavfile.read(path)
         wav = torch.from_numpy(np.ascontiguousarray(np.atleast_2d(data.T if data.ndim == 2 else data)))
-    if wav.dtype == torch.int16 and sr == TARGET_SR:
-        return wav.contiguous()
     if wav.dtype == torch.int16:
-        wav = wav.to(torch.float32) / 32768.0
-    elif wav.dtype == torch.int32:
+        return wav.contiguous(), int(sr)
+    if wav.dtype == torch.int32:
         wav = wav.to(torch.float32) / 2147483648.0
     elif wav.dtype == torch.uint8:
         wav = (wav.to(torch.float32) - 128.0) / 128.0
     else:
         wav = wav.to(torch.float32)
+    return wav, int(sr)
+
+
+def load_audio(path: str) -> torch.Tensor:
+    """Decode and resample to 16 kHz on the host: ``[C, L]`` (process_dataset.py:135-137).  The driver resamples on the device
+    instead (``decode_audio`` + :class:`~audio_calm_b200.resample.Resampler`); this is the reference's host path, kept as a
+    ``load_fn`` for comparisons.
+
+    16-bit files that already are 16 kHz come back as **int16** (PCM transport, widened on the device); everything else is float32."""
+    wav, sr = decode_audio(path)
+    if wav.dtype == torch.int16 and sr == TARGET_SR:
+        return wav
+    if wav.dtype == torch.int16:
+        wav = wav.to(torch.float32) / 32768.0
     if sr != TARGET_SR:
         import torchaudio
         wav = torchaudio.transforms.Resample(sr, TARGET_SR)(wav)
     return wav
+
+
+def clip_samples(wav: torch.Tensor, sr: int, n_fft: int = 1024) -> Tuple[int, Optional[str]]:
+    """(16 kHz samples of a decoded ``[C, L]`` clip at ``sr``, or 0; the reason it cannot be processed, or None).  The length is the
+    resampled one: a 24 kHz clip of 700 samples becomes 467 <= n_fft / 2 and is too short for the reflect padding, one of 780
+    samples becomes 520 and is processed."""
+    if wav.dim() != 2 or sr <= 0:
+        return 0, f"clip of {tuple(wav.shape)} samples at {sr} Hz is not a [channels, samples] waveform"
+    n16 = resampled_length(int(wav.shape[-1]), int(sr), TARGET_SR)
+    if n16 <= n_fft // 2:
+        return 0, (f"clip of {tuple(wav.shape)} samples" + (f" at {sr} Hz ({n16} at {TARGET_SR} Hz)" if sr != TARGET_SR else "") +
+                   " is too short for reflect padding")
+    return n16, None
 
 
 # ------------------------------------------------------------------------------------------- the per-GPU engine
@@ -141,12 +169,18 @@ class Clip(NamedTuple):
     save_path: str
     text: Optional[str]
     wav: torch.Tensor
+    sr: int = TARGET_SR           # the decoded rate: clips at another rate are resampled on the device
 
 
 class ShardRunner:
-    """Processes one shard of files on one GPU in ragged batches."""
+    """Processes one shard of files on one GPU in ragged batches.
 
-    def __init__(self, args, gpu_id: int, cv_mapping: Optional[Dict[str, str]] = None, load_fn: Callable = load_audio,
+    ``load_fn(path)`` returns ``(wav [C, L], sample_rate)`` (``decode_audio``, the default) or a bare ``[C, L]`` tensor, which means
+    16 kHz (``load_audio``).  Clips at another rate travel to the device at their native rate and dtype and are resampled there
+    (torchaudio.transforms.Resample semantics) straight into the packed 16 kHz batch: one launch per source rate and dtype per
+    batch, one ``Resampler`` kept per rate.  Batch sizes and the too-short check count 16 kHz samples."""
+
+    def __init__(self, args, gpu_id: int, cv_mapping: Optional[Dict[str, str]] = None, load_fn: Callable = decode_audio,
                  batch_samples: int = 64 * 30 * TARGET_SR, decode_threads: int = 4, report: Optional[Callable[[int], None]] = None):
         self.args, self.cv_mapping, self.load_fn = args, cv_mapping or {}, load_fn
         self.device = torch.device("cuda", gpu_id)
@@ -156,32 +190,65 @@ class ShardRunner:
         self.vae = None
         if not args.mel_only:
             self.vae = load_vae(args.vae_ckpt, self.device)  # needs the reference's models/ on sys.path (out of scope here)
+        self.resamplers: Dict[int, Resampler] = {}
         self.errors: List[Tuple[str, str]] = []
         self.trans_buffer: Dict[str, List[str]] = {}
         self.done = 0
 
-    # -- one ragged batch: peak -> fused log-mel (+ peak norm, + pad-to-4) -> D2H -> save
+    def _resampler(self, sr: int) -> Resampler:
+        rs = self.resamplers.get(sr)
+        if rs is None:
+            rs = self.resamplers[sr] = Resampler(sr, TARGET_SR, device=self.device)
+        return rs
+
+    # -- one ragged batch: [resample] -> peak -> fused log-mel (+ peak norm, + pad-to-4) -> D2H -> save
     def _flush(self, items: List[Clip], writer: ThreadPoolExecutor) -> None:
         if not items:
             return
         lib = self.fe._lib
         with torch.inference_mode(), torch.cuda.device(self.device):
-            # Peak normalisation is fused into the log-mel kernel (per-clip gain from acb_peak_abs).  Multi-channel clips are
-            # mixed down first (acb_mixdown_peak: channel mean only) and then take the same fused route.
-            clips = []
-            for it in items:
+            stream = torch.cuda.current_stream(self.device).cuda_stream
+            # The packed 16 kHz batch is allocated for the clips' 16 kHz lengths up front.  Multi-channel clips at another rate are
+            # resampled channel by channel into scratch rows behind the packed clips, then mixed down into their slot.
+            lens16 = [resampled_length(int(it.wav.shape[-1]), it.sr, TARGET_SR) for it in items]
+            _, starts, total = packed_layout(lens16)
+            scratch, pos = {}, total
+            for i, it in enumerate(items):
+                if it.sr != TARGET_SR and it.wav.shape[0] > 1:
+                    scratch[i] = pos
+                    pos += (int(it.wav.shape[0]) * lens16[i] + 3) & ~3
+            buf = torch.empty(pos, dtype=torch.float32, device=self.device)
+            batch = empty_ragged(lens16, self.device, buffer=buf)
+            groups: Dict[Tuple[int, torch.dtype], List[int]] = {}
+            for i, it in enumerate(items):
+                s, n = int(starts[i]), lens16[i]
+                if it.sr != TARGET_SR:
+                    groups.setdefault((it.sr, it.wav.dtype), []).append(i)
+                    continue
+                # Peak normalisation is fused into the log-mel kernel (per-clip gain from acb_peak_abs).  Multi-channel clips are
+                # mixed down first (acb_mixdown_peak: channel mean only) and then take the same fused route.
                 w = it.wav.to(self.device, non_blocking=True)
                 if w.dtype == torch.int16:
                     w = self.fe.pcm16_to_float(w)          # 16-bit PCM transport, widened on the device
                 if w.shape[0] == 1:
-                    clips.append(w[0])
+                    batch.wav[s:s + n].copy_(w[0])
                 else:
                     w = w.contiguous()
-                    mono = torch.empty(w.shape[1], dtype=torch.float32, device=self.device)
-                    _lib_check(lib.acb_mixdown_peak(w.data_ptr(), int(w.shape[0]), int(w.shape[1]), mono.data_ptr(), None,
-                                                    torch.cuda.current_stream(self.device).cuda_stream), "acb_mixdown_peak")
-                    clips.append(mono)
-            batch = pack_clips(clips, self.device)
+                    _lib_check(lib.acb_mixdown_peak(w.data_ptr(), int(w.shape[0]), n, batch.wav[s:].data_ptr(), None, stream),
+                               "acb_mixdown_peak")
+            for (sr, dtype), idx in groups.items():
+                # every channel row of this rate, packed at its native rate and dtype; one launch writes them all
+                rows = [(i, c) for i in idx for c in range(int(items[i].wav.shape[0]))]
+                lens, src_starts, _ = packed_layout([int(items[i].wav.shape[-1]) for i, _ in rows])
+                src = empty_ragged(lens, self.device, dtype=dtype)
+                offs = []
+                for (i, c), so, n_in in zip(rows, src_starts, lens):
+                    src.wav[so:so + n_in].copy_(items[i].wav[c], non_blocking=True)
+                    offs.append(int(starts[i]) if i not in scratch else scratch[i] + c * lens16[i])
+                self._resampler(sr).ragged(src, out=buf, out_offsets=offs)
+            for i, base in scratch.items():                 # resample, then mix down: the reference's order (core.py:102)
+                C, s, n = int(items[i].wav.shape[0]), int(starts[i]), lens16[i]
+                _lib_check(lib.acb_mixdown_peak(buf[base:].data_ptr(), C, n, batch.wav[s:].data_ptr(), None, stream), "acb_mixdown_peak")
             peak = self.fe.peak_abs_ragged(batch)
             feats, frames = self.fe.forward_ragged(batch, pad_multiple=PAD_TO, peak=peak)      # [B, 80, Tmax], frames[B] = T4
             frames_h = frames.cpu().tolist()
@@ -240,28 +307,31 @@ class ShardRunner:
         def decode(job):
             wav_path = job[0]
             try:
-                return job, self.load_fn(wav_path), None
+                got = self.load_fn(wav_path)
+                wav, sr = got if isinstance(got, tuple) else (got, TARGET_SR)
+                return job, wav, int(sr), None
             except Exception as e:  # noqa: BLE001
-                return job, None, f"{type(e).__name__}: {e}"
+                return job, None, 0, f"{type(e).__name__}: {e}"
 
         pending: List[Clip] = []
         pending_samples = 0
         self._inflight: List[Tuple[Future, Clip]] = []
         with ThreadPoolExecutor(self.decode_threads) as decoders, ThreadPoolExecutor(2) as writer:
-            for job, wav, err in decoders.map(decode, todo):
+            for job, wav, sr, err in decoders.map(decode, todo):
                 wav_path, save_dir, file_id, save_path = job
-                if err is None and (wav.dim() != 2 or wav.shape[-1] <= self.fe.n_fft // 2):
-                    err = f"clip of {tuple(wav.shape)} samples is too short for reflect padding"
+                n16 = 0
+                if err is None:
+                    n16, err = clip_samples(wav, sr, self.fe.n_fft)
                 if err is not None:
                     self.errors.append((wav_path, err))
                     self._tick()
                     continue
-                if pending and pending_samples + wav.shape[-1] > self.batch_samples:
+                if pending and pending_samples + n16 > self.batch_samples:
                     self._flush_safe(pending, writer)
                     pending, pending_samples = [], 0
                     self._collect(wait=False)
-                pending.append(Clip(wav_path, save_dir, file_id, save_path, transcript_for(wav_path, args, self.cv_mapping), wav))
-                pending_samples += int(wav.shape[-1])
+                pending.append(Clip(wav_path, save_dir, file_id, save_path, transcript_for(wav_path, args, self.cv_mapping), wav, sr))
+                pending_samples += n16
             self._flush_safe(pending, writer)
             self._collect(wait=True)
         if self.done:

@@ -114,6 +114,34 @@ def band_filterbank(fb: torch.Tensor) -> BandedFilterbank:
     return BandedFilterbank(start, length, offset, weights, n_freq)
 
 
+def sinc_resample_kernel(orig_freq: int, new_freq: int, lowpass_filter_width: int = 6, rolloff: float = 0.99,
+                         resampling_method: str = "sinc_interp_hann") -> Tuple[torch.Tensor, int]:
+    """``(kernel [N, K] fp32, width)`` of ``torchaudio.transforms.Resample(orig_freq, new_freq, ...)`` with ``(O, N)`` the rates over
+    their gcd and ``K = 2 * width + O``: the same torch operations in fp64, cast to fp32 at the end, as the transform computes its
+    buffer (``dtype=None``), so the table is bit-identical to ``Resample(...).kernel[:, 0, :]``.  ``functional.resample`` computes
+    it in the waveform's dtype instead, which gives other bits; the reference calls the transform."""
+    if resampling_method != "sinc_interp_hann":
+        raise NotImplementedError(f"resampling method {resampling_method!r}: only 'sinc_interp_hann' is implemented")
+    if int(orig_freq) != orig_freq or int(new_freq) != new_freq or orig_freq <= 0 or new_freq <= 0:
+        raise ValueError("resampling rates must be positive integers")
+    if lowpass_filter_width <= 0:
+        raise ValueError("Low pass filter width should be positive.")
+    gcd = math.gcd(int(orig_freq), int(new_freq))
+    orig, new = int(orig_freq) // gcd, int(new_freq) // gcd
+    base_freq = min(orig, new) * rolloff
+    width = math.ceil(lowpass_filter_width * orig / base_freq)
+    idx = torch.arange(-width, width + orig, dtype=torch.float64)[None, None] / orig
+    t = torch.arange(0, -new, -1)[:, None, None] / new + idx      # torchaudio passes dtype=None here: the default dtype (fp32)
+    t *= base_freq
+    t = t.clamp_(-lowpass_filter_width, lowpass_filter_width)
+    window = torch.cos(t * math.pi / lowpass_filter_width / 2) ** 2
+    t *= math.pi
+    scale = base_freq / orig
+    kernels = torch.where(t == 0, torch.tensor(1.0).to(t), t.sin() / t)
+    kernels *= window * scale
+    return kernels.to(torch.float32)[:, 0, :].contiguous(), width
+
+
 def calm_tables(sample_rate: int = 16000, n_fft: int = 1024, n_mels: int = 80,
                 f_min: float = 0.0, f_max: float = 8000.0) -> Tuple[torch.Tensor, torch.Tensor]:
     """(window ``[n_fft]``, fb ``[n_fft//2+1, n_mels]``) for ``MelExtractor``'s constructor arguments

@@ -288,6 +288,33 @@ int acb_stft_complex(const float* x, int64_t rows, int64_t length, int n_fft, in
                      const float* gl_magnitude, float gl_momentum, void* stream);
 int acb_istft(const float* spec, int64_t rows, int64_t n_frames, int n_fft, int hop, const float* window, float* out, int64_t length, void* stream);
 
+/* ---------------------------------------------------------------------------------------------
+ * Resampling to the front-end's rate: torchaudio.transforms.Resample(orig_freq, new_freq) with the default "sinc_interp_hann"
+ * method, which the reference runs on the host for every file that is not 16 kHz (preprocess/process_dataset.py:135-137).
+ * With (O, N) = (orig_freq, new_freq) / gcd, output y[b * N + j] = sum_k kernel[j][k] * xpad[b * O + k], xpad = the clip zero-padded
+ * by `width` samples on the left and width + O on the right (at each clip's own ends), over the band of non-zero coefficients of
+ * each phase.  Skipped coefficients are exact zeros, so finite input gives torchaudio's result up to fp32 summation order; a
+ * non-finite sample does not reach outputs through zero coefficients, as it does through torchaudio's dense conv1d.
+ * ------------------------------------------------------------------------------------------------------------------ */
+#define ACB_I16 2                 /* input element type of acb_resample: int16 samples, widened on the device to x / 32768 */
+
+typedef struct acb_resampler acb_resampler; /* opaque: banded per-phase coefficient table for one (device, O, N) */
+
+/* torchaudio's output length for `length` input samples: ceil(torch.as_tensor(N * length / O)) -- the quotient is rounded to fp32
+ * before the ceiling, so beyond 2^24 outputs it can differ from the exact ceiling (24 kHz -> 16 kHz: 30000001 -> 20000000) -- capped
+ * by the conv1d length (length / O + 1) * N.  orig_freq == new_freq returns length.  Host only; -1 for a negative length or rate. */
+int64_t acb_resampled_length(int64_t length, int orig_freq, int new_freq);
+/* kernel_host[N * (2 * width + O)]: the fp32 table transforms.Resample holds (row-major [N][K]).  Tables with more than 32768 banded
+ * coefficients or a band wider than 512 taps return ACB_ERR_UNSUPPORTED (8-192 kHz <-> 16 kHz at lowpass_filter_width <= 16 fit). */
+int acb_resampler_create(acb_resampler** out, int device, int orig_freq, int new_freq, int width, const float* kernel_host);
+int acb_resampler_destroy(acb_resampler* rs);
+/* Resamples n_rows rows in one launch.  in: device samples of in_dtype (ACB_F32 | ACB_I16); row i starts at element in_offset[i]
+ * (device; NULL => i * in_stride) and has in_length[i] samples (device; NULL => uniform_length).  out: device fp32; row i's
+ * acb_resampled_length(len_i) outputs start at out_offset[i] (device; NULL => i * out_stride).  Nothing outside a row is read. */
+int acb_resample(const acb_resampler* rs, const void* in, int32_t in_dtype, const int64_t* in_offset, const int64_t* in_length,
+                 int64_t in_stride, int64_t uniform_length, int32_t n_rows, float* out, const int64_t* out_offset,
+                 int64_t out_stride, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
