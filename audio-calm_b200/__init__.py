@@ -17,6 +17,8 @@ directory as that package.  Layout:
     csrc/acb_spectral.cu     its kernel (shares the in-register FFT-32 of csrc/acb_fft32.cuh)
     resample.py              Resampler: torchaudio.transforms.Resample (sinc_interp_hann) on the device, uniform and ragged
     csrc/acb_resample.cu     its polyphase kernel (banded per-phase coefficients in registers)
+    flac.py                  FlacDecoder: FLAC (RFC 9639) streams decoded bit-exact on the device, many per launch
+    csrc/acb_flac.cu         its frame-parallel decoder (sync search + CRC-8, one thread per frame, CRC-16, coverage check)
     preprocess/              drop-in mirrors of the reference's preprocess/{core,compute_mel_stats,process_dataset}.py
 """
 from . import _lib, tables  # noqa: F401
@@ -29,8 +31,10 @@ from . import spectral, whisper  # noqa: F401
 from .whisper import WhisperLogMel, whisper_tables  # noqa: F401
 from . import resample  # noqa: F401
 from .resample import Resampler, resampled_length  # noqa: F401
+from . import flac  # noqa: F401
+from .flac import FlacDecoder, FlacError, FlacInfo, parse_flac  # noqa: F401
 
 __all__ = ["LogMelFrontend", "MelStatsAccumulator", "MelStats", "RaggedBatch", "pack_clips", "frames_for_length",
            "padded_frames", "finalize_moments", "normalize_per_utterance", "MEL_MEAN_DEFAULT", "MEL_STD_DEFAULT", "WhisperLogMel", "whisper_tables",
-           "Resampler", "resampled_length", "empty_ragged"]
+           "Resampler", "resampled_length", "empty_ragged", "FlacDecoder", "FlacError", "FlacInfo", "parse_flac"]
 __version__ = "0.1.0"

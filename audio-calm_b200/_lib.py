@@ -18,7 +18,7 @@ CSRC = os.path.join(_HERE, "csrc")
 INCLUDE = os.path.join(os.path.dirname(_HERE), "include")
 LIB_NAME = "libaudiocalm_b200.so"
 LIB_PATH = os.path.join(CSRC, LIB_NAME)
-SOURCES = ["acb_kernels.cu", "acb_dftgemm.cu", "acb_spectral.cu", "acb_resample.cu"]
+SOURCES = ["acb_kernels.cu", "acb_dftgemm.cu", "acb_spectral.cu", "acb_resample.cu", "acb_flac.cu"]
 HEADERS = ["acb_fft32.cuh"]
 
 NVCC_FLAGS = [
@@ -31,6 +31,8 @@ ACB_OK = 0
 ACB_F32, ACB_BF16, ACB_I16 = 0, 1, 2
 ACB_MEL_MAJOR, ACB_TIME_MAJOR = 0, 1
 ACB_LOG_NATURAL, ACB_LOG_10 = 0, 1
+ACB_ERR_INVALID, ACB_ERR_CUDA, ACB_ERR_UNSUPPORTED = -1, -2, -3
+ACB_FLAC_OK, ACB_FLAC_BAD_CLIP, ACB_FLAC_TOO_MANY_CANDIDATES, ACB_FLAC_NOT_TILED = 0, 1, 2, 3
 
 # every symbol include/audiocalm_b200.h declares (tests check the built library exports all of them)
 EXPORTED_SYMBOLS = [
@@ -42,6 +44,7 @@ EXPORTED_SYMBOLS = [
     "acb_stft_mag_frames", "acb_stft_mag", "acb_stft_mag_backward", "acb_stft_complex", "acb_istft",
     "acb_dftgemm_frames", "acb_dftgemm_workspace_ints", "acb_dftgemm_create", "acb_dftgemm_destroy", "acb_dftgemm_forward", "acb_dftgemm_check", "acb_dftgemm_moments_workspace_bytes",
     "acb_resampled_length", "acb_resampler_create", "acb_resampler_destroy", "acb_resample",
+    "acb_flac_candidate_capacity", "acb_flac_workspace_bytes", "acb_flac_decode",
 ]
 
 
@@ -236,6 +239,12 @@ def load() -> ctypes.CDLL:
         lib.acb_resampler_destroy.argtypes = [vp]
         lib.acb_resample.restype = ctypes.c_int
         lib.acb_resample.argtypes = [vp, vp, i32, vp, vp, i64, i64, i32, vp, vp, i64, vp]
+        lib.acb_flac_candidate_capacity.restype = i64
+        lib.acb_flac_candidate_capacity.argtypes = [i64]
+        lib.acb_flac_workspace_bytes.restype = i64
+        lib.acb_flac_workspace_bytes.argtypes = [i64, i32]
+        lib.acb_flac_decode.restype = ctypes.c_int
+        lib.acb_flac_decode.argtypes = [vp, vp, i32, i32, vp, vp, vp, i64, vp]
         if lib.acb_abi_version() != 2:
             raise RuntimeError(f"{LIB_PATH}: ABI version {lib.acb_abi_version()} != 2; rebuild")
         _lib = lib

@@ -26,10 +26,12 @@ import time
 from concurrent.futures import Future, ThreadPoolExecutor
 from typing import Callable, Dict, List, NamedTuple, Optional, Sequence, Tuple
 
+import numpy as np
 import torch
 
 try:
-    from ..frontend import LogMelFrontend, empty_ragged, packed_layout
+    from ..flac import FlacDecoder, FlacInfo, STATUS_TEXT, parse_flac
+    from ..frontend import LogMelFrontend, RaggedBatch, empty_ragged, packed_layout
     from .._lib import check as _lib_check
     from ..resample import Resampler, resampled_length
     from ..sharding import contiguous_shard
@@ -38,7 +40,8 @@ except ImportError:  # run as a script / as top-level `preprocess.process_datase
     _root = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
     if _root not in sys.path:
         sys.path.insert(0, _root)
-    from audio_calm_b200.frontend import LogMelFrontend, empty_ragged, packed_layout
+    from audio_calm_b200.flac import FlacDecoder, FlacInfo, STATUS_TEXT, parse_flac
+    from audio_calm_b200.frontend import LogMelFrontend, RaggedBatch, empty_ragged, packed_layout
     from audio_calm_b200._lib import check as _lib_check
     from audio_calm_b200.resample import Resampler, resampled_length
     from audio_calm_b200.sharding import contiguous_shard
@@ -131,6 +134,26 @@ def decode_audio(path: str) -> Tuple[torch.Tensor, int]:
     return wav, int(sr)
 
 
+class FlacSource:
+    """A FLAC file read but not decoded: its bytes and parsed header.  The driver decodes every FLAC clip of a batch on the device
+    in one launch (:class:`~audio_calm_b200.flac.FlacDecoder`); ``shape`` is the ``[channels, samples]`` it decodes to."""
+
+    def __init__(self, data: bytes, info: FlacInfo):
+        self.data, self.info = data, info
+        self.shape = (info.channels, info.total_samples)
+
+    def dim(self) -> int:
+        return 2
+
+
+def read_flac(path: str) -> Tuple[FlacSource, int]:
+    """The decode-thread half of a ``.flac`` file: read the bytes and parse the header (no sample is decoded on the host)."""
+    with open(path, "rb") as f:
+        data = f.read()
+    info = parse_flac(data)
+    return FlacSource(data, info), info.sample_rate
+
+
 def load_audio(path: str) -> torch.Tensor:
     """Decode and resample to 16 kHz on the host: ``[C, L]`` (process_dataset.py:135-137).  The driver resamples on the device
     instead (``decode_audio`` + :class:`~audio_calm_b200.resample.Resampler`); this is the reference's host path, kept as a
@@ -178,7 +201,13 @@ class ShardRunner:
     ``load_fn(path)`` returns ``(wav [C, L], sample_rate)`` (``decode_audio``, the default) or a bare ``[C, L]`` tensor, which means
     16 kHz (``load_audio``).  Clips at another rate travel to the device at their native rate and dtype and are resampled there
     (torchaudio.transforms.Resample semantics) straight into the packed 16 kHz batch: one launch per source rate and dtype per
-    batch, one ``Resampler`` kept per rate.  Batch sizes and the too-short check count 16 kHz samples."""
+    batch, one ``Resampler`` kept per rate.  Batch sizes and the too-short check count 16 kHz samples.
+
+    With the default ``load_fn``, ``.flac`` files are only read and header-parsed on the decode threads (``read_flac``); each batch's
+    FLAC clips are decoded on the device in one launch, as float32 ``x / 2^(bps - 1)`` (the values ``torchaudio.load`` gives):
+    16 kHz mono clips straight into their slot of the packed batch, multi-channel 16 kHz clips into scratch rows that are then mixed
+    down, and clips at other rates into native-rate rows that the resampler reads.  A clip that fails to decode is reported in
+    ``errors``; the rest of its batch is saved."""
 
     def __init__(self, args, gpu_id: int, cv_mapping: Optional[Dict[str, str]] = None, load_fn: Callable = decode_audio,
                  batch_samples: int = 64 * 30 * TARGET_SR, decode_threads: int = 4, report: Optional[Callable[[int], None]] = None):
@@ -191,6 +220,7 @@ class ShardRunner:
         if not args.mel_only:
             self.vae = load_vae(args.vae_ckpt, self.device)  # needs the reference's models/ on sys.path (out of scope here)
         self.resamplers: Dict[int, Resampler] = {}
+        self.flac: Optional[FlacDecoder] = None
         self.errors: List[Tuple[str, str]] = []
         self.trans_buffer: Dict[str, List[str]] = {}
         self.done = 0
@@ -212,16 +242,28 @@ class ShardRunner:
             # resampled channel by channel into scratch rows behind the packed clips, then mixed down into their slot.
             lens16 = [resampled_length(int(it.wav.shape[-1]), it.sr, TARGET_SR) for it in items]
             _, starts, total = packed_layout(lens16)
-            scratch, pos = {}, total
+            # FLAC clips are decoded on the device into the same buffer: 16 kHz multi-channel clips into scratch rows, clips at
+            # another rate into native-rate rows (flac_src) behind them.
+            flac = [i for i, it in enumerate(items) if isinstance(it.wav, FlacSource)]
+            scratch, flac_src, pos = {}, {}, total
             for i, it in enumerate(items):
-                if it.sr != TARGET_SR and it.wav.shape[0] > 1:
+                if it.wav.shape[0] > 1 and (it.sr != TARGET_SR or isinstance(it.wav, FlacSource)):
                     scratch[i] = pos
                     pos += (int(it.wav.shape[0]) * lens16[i] + 3) & ~3
+            for i in flac:
+                if items[i].sr != TARGET_SR:
+                    flac_src[i] = pos
+                    pos += int(items[i].wav.shape[0]) * ((int(items[i].wav.shape[1]) + 3) & ~3)
             buf = torch.empty(pos, dtype=torch.float32, device=self.device)
             batch = empty_ragged(lens16, self.device, buffer=buf)
-            groups: Dict[Tuple[int, torch.dtype], List[int]] = {}
+            failed = self._decode_flac(items, flac, buf, starts, scratch, flac_src, lens16)
+            groups: Dict[Tuple[int, object], List[int]] = {}
             for i, it in enumerate(items):
                 s, n = int(starts[i]), lens16[i]
+                if isinstance(it.wav, FlacSource):
+                    if it.sr != TARGET_SR and i not in failed:
+                        groups.setdefault((it.sr, "flac"), []).append(i)
+                    continue
                 if it.sr != TARGET_SR:
                     groups.setdefault((it.sr, it.wav.dtype), []).append(i)
                     continue
@@ -237,16 +279,24 @@ class ShardRunner:
                     _lib_check(lib.acb_mixdown_peak(w.data_ptr(), int(w.shape[0]), n, batch.wav[s:].data_ptr(), None, stream),
                                "acb_mixdown_peak")
             for (sr, dtype), idx in groups.items():
-                # every channel row of this rate, packed at its native rate and dtype; one launch writes them all
                 rows = [(i, c) for i in idx for c in range(int(items[i].wav.shape[0]))]
+                offs = [int(starts[i]) if i not in scratch else scratch[i] + c * lens16[i] for i, c in rows]
+                if dtype == "flac":
+                    # decoded rows already in `buf` at their native rate: channel c of clip i at flac_src[i] + c * pitch
+                    lens = np.array([int(items[i].wav.shape[1]) for i, _ in rows], dtype=np.int64)
+                    src_offs = np.array([flac_src[i] + c * ((int(items[i].wav.shape[1]) + 3) & ~3) for i, c in rows], dtype=np.int64)
+                    src = RaggedBatch(buf, torch.from_numpy(src_offs).to(self.device), torch.from_numpy(lens).to(self.device), lens)
+                    self._resampler(sr).ragged(src, out=buf, out_offsets=offs)
+                    continue
+                # every channel row of this rate, packed at its native rate and dtype; one launch writes them all
                 lens, src_starts, _ = packed_layout([int(items[i].wav.shape[-1]) for i, _ in rows])
                 src = empty_ragged(lens, self.device, dtype=dtype)
-                offs = []
                 for (i, c), so, n_in in zip(rows, src_starts, lens):
                     src.wav[so:so + n_in].copy_(items[i].wav[c], non_blocking=True)
-                    offs.append(int(starts[i]) if i not in scratch else scratch[i] + c * lens16[i])
                 self._resampler(sr).ragged(src, out=buf, out_offsets=offs)
             for i, base in scratch.items():                 # resample, then mix down: the reference's order (core.py:102)
+                if i in failed:
+                    continue
                 C, s, n = int(items[i].wav.shape[0]), int(starts[i]), lens16[i]
                 _lib_check(lib.acb_mixdown_peak(buf[base:].data_ptr(), C, n, batch.wav[s:].data_ptr(), None, stream), "acb_mixdown_peak")
             peak = self.fe.peak_abs_ragged(batch)
@@ -255,13 +305,44 @@ class ShardRunner:
             if self.vae is None:
                 host = feats.cpu()
                 for i, it in enumerate(items):
+                    if i in failed:
+                        continue
                     mel = host[i, :, :frames_h[i]].clone()                                     # logical [80, T4] float32
                     self._inflight.append((writer.submit(self._save, it.save_dir, it.save_path, {"mel": mel}), it))
             else:
                 for i, it in enumerate(items):
+                    if i in failed:
+                        continue
                     mu, _ = self.vae.encode(feats[i:i + 1, :, :frames_h[i]])                   # process_dataset.py:159-163
                     payload = {"latent": mu.squeeze(0).cpu(), "vae_path": self.args.vae_ckpt}
                     self._inflight.append((writer.submit(self._save, it.save_dir, it.save_path, payload), it))
+
+    def _decode_flac(self, items: List[Clip], flac: List[int], buf: torch.Tensor, starts, scratch: Dict[int, int],
+                     flac_src: Dict[int, int], lens16: List[int]) -> set:
+        """Decode the batch's FLAC clips into ``buf`` in one launch; report the ones that fail and return their indices."""
+        if not flac:
+            return set()
+        if self.flac is None:
+            self.flac = FlacDecoder(self.device)
+        offs, strides = [], []
+        for i in flac:
+            w = items[i].wav
+            if i in flac_src:
+                offs.append(flac_src[i])
+                strides.append((int(w.shape[1]) + 3) & ~3)
+            else:
+                offs.append(scratch[i] if i in scratch else int(starts[i]))
+                strides.append(lens16[i])
+        status = self.flac.decode([items[i].wav.data for i in flac], torch.float32, infos=[items[i].wav.info for i in flac],
+                                  out=buf, out_offsets=offs, out_strides=strides)
+        failed = set()
+        for i, st in zip(flac, status.tolist()):
+            if st:
+                failed.add(i)
+                buf[int(starts[i]):int(starts[i]) + lens16[i]].zero_()                    # its slot holds no stale samples
+                self.errors.append((items[i].wav_path, f"FLAC decode failed: {STATUS_TEXT.get(st, st)}"))
+                self._tick()
+        return failed
 
     @staticmethod
     def _save(save_dir: str, save_path: str, payload: dict) -> None:
@@ -307,7 +388,10 @@ class ShardRunner:
         def decode(job):
             wav_path = job[0]
             try:
-                got = self.load_fn(wav_path)
+                if self.load_fn is decode_audio and wav_path.lower().endswith(".flac"):
+                    got = read_flac(wav_path)                                                  # decoded on the device per batch
+                else:
+                    got = self.load_fn(wav_path)
                 wav, sr = got if isinstance(got, tuple) else (got, TARGET_SR)
                 return job, wav, int(sr), None
             except Exception as e:  # noqa: BLE001

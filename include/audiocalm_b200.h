@@ -315,6 +315,49 @@ int acb_resample(const acb_resampler* rs, const void* in, int32_t in_dtype, cons
                  int64_t in_stride, int64_t uniform_length, int32_t n_rows, float* out, const int64_t* out_offset,
                  int64_t out_stride, void* stream);
 
+/* ---------------------------------------------------------------------------------------------
+ * FLAC decoding (RFC 9639) for the dataset driver: LibriSpeech ships as 16 kHz, 16-bit mono FLAC.  The host parses the stream
+ * header (section 8: "fLaC", STREAMINFO first, the other metadata blocks skipped); the device decodes the audio frames of many
+ * streams in one call, bit-exact:
+ *   - frame headers (9.1): both blocking strategies, block-size codes 1-15 including the 8- and 16-bit uncommon forms, sample-rate
+ *     codes 0-14 including the uncommon forms, channel assignments 0-10, bit-depth codes, coded numbers of up to 7 bytes, CRC-8;
+ *   - subframes (9.2): CONSTANT, VERBATIM, FIXED orders 0-4, LPC orders 1-32, wasted bits, residual coding methods 0 and 1 with
+ *     partition orders 0-15 and escaped partitions; left/side, side/right and mid/side stereo (9.2 / 4.2);
+ *   - the frame footer (9.3): byte-alignment padding and CRC-16.
+ * Rejected: 32-bit samples (the host parse returns ACB_ERR_UNSUPPORTED), negative LPC shifts, coefficient precision 16, reserved
+ * codes.  The STREAMINFO MD5 is not verified (it is sequential over the whole stream); every frame's CRC-16 is.
+ * Frames are found by searching every byte of a clip's region for a sync whose header has a valid CRC-8 and agrees with STREAMINFO;
+ * a candidate is accepted only when it decodes and its CRC-16 matches, and the accepted frames must tile [0, total_samples) in byte
+ * order with contiguous byte ranges.  A clip that fails any of this gets a non-zero status; the other clips of the call are decoded.
+ * ------------------------------------------------------------------------------------------------------------------ */
+#define ACB_FLAC_OK 0
+#define ACB_FLAC_BAD_CLIP 1               /* descriptor out of range (channels 1-8, bps 4-24, max_block 1-65536, region < 2 GiB) */
+#define ACB_FLAC_TOO_MANY_CANDIDATES 2    /* more sync candidates than acb_flac_candidate_capacity(byte_length) */
+#define ACB_FLAC_NOT_TILED 3              /* accepted frames do not tile [0, total_samples): corrupt, truncated or missing frames */
+
+typedef struct acb_flac_clip {     /* one stream, in device memory (72 bytes) */
+    int64_t byte_offset;           /* first byte of the stream's audio-frame region in `data` */
+    int64_t byte_length;           /* bytes of the region; nothing outside [byte_offset, byte_offset + byte_length) is read */
+    int64_t total_samples;         /* samples per channel (STREAMINFO, or recovered by the host when STREAMINFO says 0) */
+    int64_t out_offset;            /* element of `out` where channel 0 starts */
+    int64_t out_stride;            /* elements between channel rows */
+    int64_t cand_offset;           /* first candidate slot: exclusive prefix over clips of acb_flac_candidate_capacity(byte_length) */
+    int32_t channels, bps, sample_rate, max_block;   /* STREAMINFO */
+    int32_t variable;              /* blocking strategy of the stream's frames: 0 fixed (0xFFF8), 1 variable (0xFFF9) */
+    int32_t reserved;
+} acb_flac_clip;
+
+/* Candidate slots one clip needs: byte_length / 8 + 16 (a frame takes at least 9 bytes). */
+int64_t acb_flac_candidate_capacity(int64_t byte_length);
+/* Bytes of device workspace for total_candidates slots (the sum of the capacities) and n_clips clips. */
+int64_t acb_flac_workspace_bytes(int64_t total_candidates, int32_t n_clips);
+/* Decodes n_clips streams: data (device bytes), clips (device [n_clips]).  out: device int16 (ACB_I16, only for bps = 16 streams:
+ * the samples themselves) or fp32 (ACB_F32: x / 2^(bps - 1), exact for bps <= 24 and what torchaudio.load returns).  status: device
+ * int32 [n_clips], ACB_FLAC_*.  Only frames that pass their CRC-16 are written; a clip with a non-zero status may be partly written.
+ * workspace: 16-byte aligned, acb_flac_workspace_bytes(total_candidates, n_clips) bytes.  Three launches on `stream`. */
+int acb_flac_decode(const uint8_t* data, const acb_flac_clip* clips, int32_t n_clips, int32_t out_dtype, void* out, int32_t* status,
+                    void* workspace, int64_t total_candidates, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

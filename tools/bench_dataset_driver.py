@@ -2,12 +2,16 @@
 GPU batches -> {"mel"} payloads on disk.  One JSON line.
 
     python tools/bench_dataset_driver.py [--files 2000] [--seconds 10] [--decode-threads 8] [--sample-rate 24000 [--host-resample]]
+                                         [--format flac]
 
 Synthetic 16-bit PCM .wav files (what LibriSpeech-style corpora hold once decoded) are written to a scratch directory first; the
 timed region is ShardRunner.run over them, i.e. what `python preprocess/process_dataset.py --mel_only` does per GPU process.
 --sample-rate writes the files at another rate (LibriTTS is 24 kHz): the driver resamples them on the device.  --host-resample
 runs the same files through the reference's host path instead (load_fn=load_audio: torchaudio.transforms.Resample in every
-decode thread), so the two arms compare device and host resampling on the same files."""
+decode thread), so the two arms compare device and host resampling on the same files.  --format flac writes the files as FLAC
+(16-bit, LPC order 8, 4096-sample blocks; eight distinct encoded clips, copied to every file name) and --format wav the same eight
+PCM clips as 16-bit .wav, so the two arms compare device FLAC decoding with the host .wav path on the same audio; the report adds
+the host-to-device bytes per audio-second (the file's audio bytes: compressed frames for FLAC, PCM for .wav)."""
 import argparse
 import json
 import os
@@ -50,6 +54,9 @@ def main():
     ap.add_argument("--procs", type=int, default=1, help="driver processes sharing the GPU (--procs_per_gpu of the driver)")
     ap.add_argument("--sample-rate", type=int, default=16000, help="rate of the synthetic files")
     ap.add_argument("--host-resample", action="store_true", help="resample on the host (load_fn=load_audio), the reference's path")
+    ap.add_argument("--format", choices=["wav", "flac", "wav-distinct"], default="wav-distinct",
+                    help="wav-distinct: every file its own slice of one noise signal (the default, as before); wav / flac: eight "
+                         "distinct speech-like clips copied to every file, as 16-bit .wav or as FLAC")
     args = ap.parse_args()
     from scipy.io import wavfile
     from audio_calm_b200.preprocess import process_dataset as pd
@@ -61,15 +68,37 @@ def main():
         n = int(args.seconds * sr)
         rng = np.random.default_rng(0)
         base = (hash_noise(n + 4096, 5) * 0.8 * 32767).astype(np.int16)
-        for i in range(args.files):
-            d = os.path.join(in_dir, f"spk{i % 40:03d}", f"chap{i % 7}")
-            os.makedirs(d, exist_ok=True)
-            off = int(rng.integers(0, 4096))
-            wavfile.write(os.path.join(d, f"utt{i:06d}.wav"), sr, base[off:off + n - int(rng.integers(0, n // 2))])
-        files = pd.scan_files(in_dir)
-        audio_s = sum(os.path.getsize(f) - 44 for f in files) / 2 / sr
+        if args.format == "wav-distinct":
+            for i in range(args.files):
+                d = os.path.join(in_dir, f"spk{i % 40:03d}", f"chap{i % 7}")
+                os.makedirs(d, exist_ok=True)
+                off = int(rng.integers(0, 4096))
+                wavfile.write(os.path.join(d, f"utt{i:06d}.wav"), sr, base[off:off + n - int(rng.integers(0, n // 2))])
+            files = pd.scan_files(in_dir)
+            audio_s = sum(os.path.getsize(f) - 44 for f in files) / 2 / sr
+            h2d = 2.0 * sr
+        else:
+            from oracle import flac_oracle as fo
+            from oracle.gen_golden_flac import speech_like
+            clips = [speech_like(n - int(rng.integers(0, n // 2)), 1, 16, 200 + k, sr) for k in range(8)]
+            blobs = [fo.encode(c, sr, 16, kind="lpc", order=8, block_size=4096) if args.format == "flac" else None for c in clips]
+            for i in range(args.files):
+                d = os.path.join(in_dir, f"spk{i % 40:03d}", f"chap{i % 7}")
+                os.makedirs(d, exist_ok=True)
+                if args.format == "flac":
+                    with open(os.path.join(d, f"utt{i:06d}.flac"), "wb") as f:
+                        f.write(blobs[i % 8])
+                else:
+                    wavfile.write(os.path.join(d, f"utt{i:06d}.wav"), sr, clips[i % 8][0].astype(np.int16))
+            files = pd.scan_files(in_dir)
+            audio_s = sum(clips[i % 8].shape[1] for i in range(args.files)) / sr
+            if args.format == "flac":
+                from audio_calm_b200.flac import parse_flac
+                h2d = sum(parse_flac(blobs[i % 8]).audio_length for i in range(args.files)) / audio_s
+            else:
+                h2d = 2.0 * sr
         load_fn = pd.load_audio if args.host_resample else pd.decode_audio
-        arm = {"sample_rate": sr, "resampling": "none" if sr == 16000 else ("host (torchaudio, decode threads)" if args.host_resample
+        arm = {"format": args.format, "h2d_bytes_per_audio_s": h2d, "sample_rate": sr, "resampling": "none" if sr == 16000 else ("host (torchaudio, decode threads)" if args.host_resample
                                                                               else "device (acb_resample)")}
         a = types.SimpleNamespace(dataset_name="librispeech", in_dir=in_dir, out_dir=out_dir, vae_ckpt=None, mel_only=True, cv_tsv=None,
                                   num_gpus=1, workers_per_gpu=args.decode_threads, force=False)
