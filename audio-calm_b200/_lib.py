@@ -18,8 +18,8 @@ CSRC = os.path.join(_HERE, "csrc")
 INCLUDE = os.path.join(os.path.dirname(_HERE), "include")
 LIB_NAME = "libaudiocalm_b200.so"
 LIB_PATH = os.path.join(CSRC, LIB_NAME)
-SOURCES = ["acb_kernels.cu", "acb_dftgemm.cu", "acb_spectral.cu", "acb_resample.cu", "acb_flac.cu"]
-HEADERS = ["acb_fft32.cuh"]
+SOURCES = ["acb_kernels.cu", "acb_logmel_stft.cu", "acb_dftgemm.cu", "acb_spectral.cu", "acb_resample.cu", "acb_flac.cu"]
+HEADERS = ["acb_fft32.cuh", "acb_logmel_common.cuh"]
 
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",

@@ -27,6 +27,7 @@
 // frees the scratch, so a warp never waits for its group with nothing to do.
 #include "audiocalm_b200.h"
 #include "acb_fft32.cuh"
+#include "acb_logmel_common.cuh"
 
 #include <cuda_bf16.h>
 #include <cuda_runtime.h>
@@ -45,9 +46,6 @@ namespace acb {
 constexpr int kNfft = 1024;
 constexpr int kHop = 256;
 constexpr int kBins = 512;                                   // bins 0..511 are produced; 512 (Nyquist) has zero weight
-constexpr int kTileFrames = 8;                               // one tile = 4 frame pairs = one pair per warp of a group
-constexpr int kGroupWarps = 4;
-constexpr int kGroupThreads = kGroupWarps * 32;
 // Groups per CTA are a template parameter G: 4 groups in ONE 512-thread CTA per SM (the tables are staged once per SM and
 // the 16 warps share one instruction footprint; measured 7 % faster than 2 CTAs of 2 groups), or 2 groups x 2 CTAs per SM when
 // a large filterbank plan does not leave room for four groups' buffers.
@@ -57,7 +55,6 @@ constexpr int kRowStride = 36;                               // floats per row o
 constexpr int kPlaneFloats = 32 * kRowStride;                // the real and the imaginary parts are transposed in separate planes
 constexpr int kScratchFloats = 2 * kPlaneFloats + 8;         // 2312 floats / warp; == 8 (mod 32): see the mel phase
 constexpr int kSlots = 8;                                    // band slots per mel round: lanes = 8 slots x 4 frame pairs
-constexpr int kMaxMels = 128;
 constexpr int kMaxRounds = 4;                                // mel plan: rounds of (8 bands) per warp
 constexpr int kMaxWeights = 4096;
 constexpr int kOutStageOffset = 2 * kBins;                   // the staged output tile lives above pair 0's power spectrum
@@ -112,59 +109,9 @@ __device__ __forceinline__ void bulk_copy_g2s(void* smem, const void* gmem, unsi
 // --------------------------------------------------------------------------------------------
 // fused log-mel kernel
 // --------------------------------------------------------------------------------------------
-struct LogmelParams {
-    // tables (device)
-    const float* window;       // [1024]
-    const float4* twiddle;     // [5][32]  seeds of the twiddle chains per lane l, W = exp(-2*pi*i/1024):
-                               //          [k][l] = (Re W^kl, Re W^(k+16)l, Im W^kl, Im W^(k+16)l), k = 0..3;  [4][l] = (Re, Im W^4l, 0, 0)
-    // mel plan: per (group warp, round) eight band slots with a common even trip count; weights zero-padded to the trip
-    // and interleaved as [i/2][slot][2] so that a lane fetches two consecutive weights with one 8-byte load
-    const float* plan_w;       // [n_plan_w]
-    const int* plan_woff;      // [kGroupWarps][kMaxRounds] offset (floats) of the round's weights in plan_w
-    const short* plan_trip;    // [kGroupWarps][kMaxRounds] bins per round (even, 0 = no more rounds)
-    const short* plan_band;    // [kGroupWarps][kMaxRounds][kSlots] band id or -1
-    const short* plan_astart;  // [kGroupWarps][kMaxRounds][kSlots] first bin (even) of the slot's run
-    int n_plan_w;
-    int n_mels;
-    float clamp_min;
-    float log_scale;           // ln(2) for ln, log10(2) for log10 (applied to log2)
-    float log_floor;           // log(clamp_min) computed on the host: clamped values are exactly the reference's floor
-    // batch
-    const float* wav;
-    const long long* clip_offset;
-    const long long* clip_length;
-    long long clip_stride;
-    long long uniform_length;
-    const int* tile_start;
-    int n_clips;
-    int n_tiles;
-    int uniform_tiles_per_clip;
-    const float* clip_peak;
-    // output
-    void* out;
-    int out_bf16;
-    int time_major;
-    const long long* out_offset;
-    long long out_clip_stride;
-    long long frame_capacity;
-    const long long* frame_capacity_per_clip;
-    int pad_multiple;
-    int fill_tail;
-    float fill_value;
-    int affine;
-    float affine_mean;
-    float affine_inv_std;
-    const float* bin_mean;
-    const float* bin_std;
-    double* moments_partial;   // [gridDim.x * G][2][n_mels] or nullptr
-    int* error_flag;           // set to 1 when a sample-tile barrier timed out (results invalid)
-};
-
 struct SmemLayout {
     int samples, scratch, twiddle, window, plan_w, affine, plan_rec, mbar, moments, total_bytes;
 };
-
-__host__ __device__ inline int out_row_stride(int n_mels) { return n_mels | 1; }   // odd: conflict-free both ways
 
 // Kernels without the moment accumulators: every offset is a compile-time constant of the kernel -- the regions whose size depends on
 // the filterbank are sized for kMaxMels (the per-band affine pairs) or placed last (the plan's weights) -- so that no shared-memory
@@ -197,63 +144,6 @@ __host__ __device__ inline SmemLayout make_smem_layout(int kGroups, int n_mels, 
     }
     L.total_bytes = off * 4;
     return L;
-}
-
-// Position of a group in its contiguous tile range: which clip, which tile of the clip, and the clip's geometry.
-struct ClipCursor {
-    long long wav_base;    // element index of the clip's first sample in wav
-    long long length;      // samples in the clip
-    long long out_base;    // element offset of the clip in out
-    int cap;               // frame capacity (row pitch of the mel-major layout)
-    int frames;            // T
-    int frames_padded;     // T4
-    int clip;
-    int tile_in_clip;
-    int tiles_in_clip;
-    float gain;            // squared waveform scale (fused peak normalisation), 1 otherwise
-};
-
-__device__ __forceinline__ void cursor_load_clip(const LogmelParams& p, ClipCursor& c) {
-    const int i = c.clip;
-    c.wav_base = p.clip_offset ? p.clip_offset[i] : (long long)i * p.clip_stride;
-    c.length = p.clip_length ? p.clip_length[i] : p.uniform_length;
-    c.out_base = p.out_offset ? p.out_offset[i] : (long long)i * p.out_clip_stride;
-    c.cap = (int)(p.frame_capacity_per_clip ? p.frame_capacity_per_clip[i] : p.frame_capacity);
-    c.frames = 1 + (int)(c.length / kHop);
-    const int rem = c.frames % p.pad_multiple;
-    c.frames_padded = rem ? c.frames + (p.pad_multiple - rem) : c.frames;
-    c.tiles_in_clip = p.tile_start ? (__ldg(p.tile_start + i + 1) - __ldg(p.tile_start + i)) : p.uniform_tiles_per_clip;
-    c.gain = 1.f;
-    if (p.clip_peak) {
-        const float peak = __ldg(p.clip_peak + i);
-        if (peak > 0.f) {
-            const float s = 0.95f / (peak + 1e-8f);
-            c.gain = s * s;
-        }
-    }
-}
-
-__device__ __forceinline__ void cursor_init(const LogmelParams& p, ClipCursor& c, long long tile) {
-    if (p.tile_start == nullptr) {
-        c.clip = (int)(tile / p.uniform_tiles_per_clip);
-        c.tile_in_clip = (int)(tile - (long long)c.clip * p.uniform_tiles_per_clip);
-    } else {  // largest clip with tile_start[clip] <= tile
-        int lo = 0, hi = p.n_clips;
-        while (hi - lo > 1) {
-            const int mid = (lo + hi) >> 1;
-            if ((long long)__ldg(p.tile_start + mid) <= tile) lo = mid; else hi = mid;
-        }
-        c.clip = lo;
-        c.tile_in_clip = (int)(tile - __ldg(p.tile_start + lo));
-    }
-    cursor_load_clip(p, c);
-}
-
-__device__ __forceinline__ void cursor_advance(const LogmelParams& p, ClipCursor& c) {
-    if (++c.tile_in_clip >= c.tiles_in_clip) {
-        c.tile_in_clip = 0;
-        do { ++c.clip; cursor_load_clip(p, c); } while (c.tiles_in_clip == 0 && c.clip + 1 < p.n_clips);
-    }
 }
 
 __device__ __forceinline__ void group_sync(int grp) {   // named barrier of one 4-warp group (barrier 0 is __syncthreads)
@@ -297,123 +187,6 @@ __device__ __forceinline__ void load_tile_samples(const LogmelParams& p, const C
     gather_edge_tile(src, g0, t.length, s_samples, gt);
     group_sync(grp);
     if (gt == 0) mbar_arrive(full);
-}
-
-template <typename OutT>
-__device__ __forceinline__ OutT to_out(float v);
-template <>
-__device__ __forceinline__ float to_out<float>(float v) { return v; }
-template <>
-__device__ __forceinline__ __nv_bfloat16 to_out<__nv_bfloat16>(float v) { return __float2bfloat16_rn(v); }
-
-template <typename OutT>
-__device__ __forceinline__ void store_pair(OutT* dst, float a, float b);
-template <>
-__device__ __forceinline__ void store_pair<float>(float* dst, float a, float b) { *reinterpret_cast<float2*>(dst) = make_float2(a, b); }
-template <>
-__device__ __forceinline__ void store_pair<__nv_bfloat16>(__nv_bfloat16* dst, float a, float b) {
-    *reinterpret_cast<__nv_bfloat162*>(dst) = __floats2bfloat162_rn(a, b);
-}
-
-// Store one staged tile.  Interior tiles (every frame exists and none is a pad-to-4 source) take loops without
-// per-element conditions; the last tiles of a clip take the general path (masking, reflected columns, tail fill).
-template <typename OutT>
-__device__ __forceinline__ void store_tile(const LogmelParams& p, const ClipCursor& c, const float* s_out, int n_mels, int S, int tid) {
-    OutT* out = reinterpret_cast<OutT*>(p.out) + c.out_base;
-    const int lane = tid & 31, warp = tid >> 5;   // thread / warp index inside the group
-    const int f0 = c.tile_in_clip * kTileFrames;
-    const int T = c.frames, T4 = c.frames_padded, pad = T4 - T;
-    const bool interior = (f0 + kTileFrames - 1 <= T - 2 - pad);
-    if (interior) {
-        if (p.time_major) {
-            OutT* row0 = out + (size_t)f0 * n_mels;
-            for (int f = warp; f < kTileFrames; f += kGroupWarps) {
-                OutT* row = row0 + f * n_mels;
-                const float* srow = s_out + f * S;
-                for (int b = lane; b < n_mels; b += 32) row[b] = to_out<OutT>(srow[b]);
-            }
-        } else {
-            OutT* col0 = out + f0;
-            const int f = tid & (kTileFrames - 1);
-            for (int b = tid / kTileFrames; b < n_mels; b += kGroupThreads / kTileFrames)
-                col0[(unsigned)b * (unsigned)c.cap + f] = to_out<OutT>(s_out[f * S + b]);
-        }
-        return;
-    }
-    const int n_out = kTileFrames * n_mels;
-    for (int idx = tid; idx < n_out; idx += kGroupThreads) {
-        int f, b;
-        if (p.time_major) { f = idx / n_mels; b = idx - f * n_mels; }
-        else { b = idx / kTileFrames; f = idx - b * kTileFrames; }
-        const int fr = f0 + f;
-        if (fr >= c.cap) continue;
-        float v;
-        bool dup = false;
-        if (fr < T) {
-            v = s_out[f * S + b];
-            dup = (fr <= T - 2) && (fr > T - 2 - pad);
-        } else if (fr >= T4 && p.fill_tail) {
-            v = p.fill_value;
-        } else {
-            continue;
-        }
-        const size_t e0 = p.time_major ? ((size_t)fr * n_mels + b) : ((size_t)b * c.cap + fr);
-        out[e0] = to_out<OutT>(v);
-        if (dup) {
-            const int fd = 2 * T - 2 - fr;  // column T + j with j = T-2-fr  (out[T+j] = mel[T-2-j])
-            const size_t e1 = p.time_major ? ((size_t)fd * n_mels + b) : ((size_t)b * c.cap + fd);
-            out[e1] = to_out<OutT>(v);
-        }
-    }
-}
-
-// Fill `n` elements at `ptr` with `fv`: scalar head / tail around 16-byte stores, `nt` cooperating threads (index t)
-template <typename OutT>
-__device__ __forceinline__ void fill_span(OutT* ptr, long long n, OutT fv, int t, int nt) {
-    constexpr int per16 = 16 / (int)sizeof(OutT);
-    const long long head = min(n, (long long)(((16 - (reinterpret_cast<uintptr_t>(ptr) & 15)) & 15) / sizeof(OutT)));
-    for (long long i = t; i < head; i += nt) ptr[i] = fv;
-    const long long body = (n - head) / per16;
-    unsigned w;
-    if (sizeof(OutT) == 4) w = *reinterpret_cast<const unsigned*>(&fv);
-    else { const unsigned short h = *reinterpret_cast<const unsigned short*>(&fv); w = (unsigned)h | ((unsigned)h << 16); }
-    uint4* q = reinterpret_cast<uint4*>(ptr + head);
-    for (long long i = t; i < body; i += nt) q[i] = make_uint4(w, w, w, w);
-    for (long long i = head + body * per16 + t; i < n; i += nt) ptr[i] = fv;
-}
-
-// Padded batches with a tile plan (tiles cover only the frames that exist): the group that stores a clip's last tile also sets the
-// rest of the clip's row, frames [end of the tile, frame_capacity), to the fill value -- one vectorised sweep instead of one
-// near-empty tile per 8 frames.
-template <typename OutT>
-__device__ __forceinline__ void fill_row_tail(const LogmelParams& p, const ClipCursor& c, int n_mels, int tid) {
-    const int f_begin = (c.tile_in_clip + 1) * kTileFrames;
-    const long long n_fill = (long long)c.cap - f_begin;
-    if (n_fill <= 0) return;
-    OutT* out = reinterpret_cast<OutT*>(p.out) + c.out_base;
-    const OutT fv = to_out<OutT>(p.fill_value);
-    if (p.time_major) {
-        fill_span<OutT>(out + (size_t)f_begin * n_mels, n_fill * n_mels, fv, tid, kGroupThreads);
-    } else {
-        const int lane = tid & 31, warp = tid >> 5;
-        for (int b = warp; b < n_mels; b += kGroupWarps) fill_span<OutT>(out + (size_t)b * c.cap + f_begin, n_fill, fv, lane, 32);
-    }
-}
-
-// log2 of a value known to be a normal float (it is above the clamp): the bare MUFU.LG2, without __log2f's denormal rescue
-__device__ __forceinline__ float lg2_normal(float x) {
-    float y;
-    asm("lg2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));
-    return y;
-}
-
-// (hi, lo) += x with the rounding error of hi + x carried in lo (Knuth two-sum; no fast-math reassociation is enabled)
-__device__ __forceinline__ void two_sum_add(float2& acc, float x) {
-    const float t = __fadd_rn(acc.x, x);
-    const float bb = __fsub_rn(t, acc.x);
-    const float e = __fadd_rn(__fsub_rn(acc.x, __fsub_rn(t, bb)), __fsub_rn(x, bb));
-    acc.y = __fadd_rn(acc.y, e);
-    acc.x = t;
 }
 
 template <int G, bool kMoments, typename OutT>
@@ -474,7 +247,7 @@ __global__ void __launch_bounds__(G * kGroupThreads, G == 4 ? 1 : 2) logmel_fuse
     bool staged = false;          // group-uniform: a sample tile was requested for the current tile
     unsigned full_parity = 0;
     if (t_begin < t_end) {
-        cursor_init(p, cur, t_begin);
+        cursor_init(p, cur, t_begin, kHop);
         staged = cur.tile_in_clip * kTileFrames < cur.frames;
         if (staged) load_tile_samples(p, cur, s_samples, gt, grp, s_full);
     }
@@ -611,7 +384,7 @@ __global__ void __launch_bounds__(G * kGroupThreads, G == 4 ? 1 : 2) logmel_fuse
         ClipCursor nxt = cur;
         staged = false;
         if (tile + 1 < t_end) {
-            cursor_advance(p, nxt);
+            cursor_advance(p, nxt, kHop);
             staged = nxt.tile_in_clip * kTileFrames < nxt.frames;
             if (staged) load_tile_samples(p, nxt, s_samples, gt, grp, s_full);
         }
@@ -1168,32 +941,6 @@ __global__ void __launch_bounds__(256) pad_transpose_kernel(const T* __restrict_
 // ==============================================================================================
 // host side: handle, planning, launches
 // ==============================================================================================
-struct acb_frontend {
-    int device = 0;
-    int n_fft = 0, hop = 0, n_mels = 0, n_weights = 0, log_kind = 0;
-    float clamp_min = 0.f;
-    int num_sms = 0;
-    int groups = 0;        // groups per CTA (template parameter G of the kernel): 4, or 2 when four do not fit in shared memory
-    int grid = 0;          // persistent grid (CTAs)
-    int smem_bytes = 0;
-    int smem_bytes_moments = 0;
-    // one device allocation holding every table
-    void* d_blob = nullptr;
-    const float* d_window = nullptr;
-    const float4* d_twiddle = nullptr;
-    const float* d_plan_w = nullptr;
-    const int* d_plan_woff = nullptr;
-    const short* d_plan_trip = nullptr;
-    const short* d_plan_band = nullptr;
-    const short* d_plan_astart = nullptr;
-    int n_plan_w = 0;
-    int* d_err = nullptr;  // in-kernel barrier timeout flag
-    // host-path streams/events (created lazily)
-    cudaStream_t s_in = nullptr, s_out = nullptr;
-    std::vector<cudaEvent_t> ev;
-    std::mutex mu;
-};
-
 using namespace acb;
 
 extern "C" {
@@ -1236,12 +983,15 @@ int64_t acb_plan_tiles(const int64_t* lengths_host, int32_t n_clips, int n_fft, 
 int acb_frontend_create(acb_frontend** out, int device, int n_fft, int hop, int n_mels, const float* window_host,
                         const float* fb_host, float clamp_min, int log_kind) {
     if (!out || !window_host || !fb_host) return fail(ACB_ERR_INVALID, "acb_frontend_create: null argument");
-    if (n_fft != kNfft || hop != kHop)
-        return fail(ACB_ERR_UNSUPPORTED, "acb_frontend_create: this build has kernels for n_fft=1024, hop=256 only (got n_fft=" +
+    // (1024, 256) runs the tuned kernel below; every other supported (n_fft, hop) the general STFT kernel (acb_logmel_stft.cu)
+    const bool tuned = n_fft == kNfft && hop == kHop;
+    if (!tuned && !stft_logmel_supported(n_fft, hop))
+        return fail(ACB_ERR_UNSUPPORTED, "acb_frontend_create: this build has kernels for n_fft 256, 512 or 1024 with 1 <= hop <= n_fft (got n_fft=" +
                                              std::to_string(n_fft) + ", hop=" + std::to_string(hop) + ")");
     if (n_mels < 1 || n_mels > kMaxMels) return fail(ACB_ERR_UNSUPPORTED, "acb_frontend_create: n_mels must be in [1, 128]");
     if (log_kind != ACB_LOG_NATURAL && log_kind != ACB_LOG_10) return fail(ACB_ERR_INVALID, "acb_frontend_create: bad log_kind");
     if (!(clamp_min >= 1.17549435e-38f)) return fail(ACB_ERR_INVALID, "acb_frontend_create: clamp_min must be a positive normal float");
+    if (!tuned) return stft_frontend_create(out, device, n_fft, hop, n_mels, window_host, fb_host, clamp_min, log_kind);
     // The kernel stages only w[0 .. N/2 - 1] and computes the second half as 1 - w[n] (the periodic-Hann property).  A window
     // without that property would give wrong features silently; fp32 periodic Hann deviates by 1.8e-7.
     for (int n = 0; n < kNfft / 2; ++n) {
@@ -1534,7 +1284,9 @@ int acb_logmel_forward(const acb_frontend* fe, const acb_logmel_args* a, void* s
     const int threads = fe->groups * kGroupThreads;
     const size_t smem = a->moments ? fe->smem_bytes_moments : fe->smem_bytes;
     auto launch = [&](auto kernel) { kernel<<<grid, threads, smem, st>>>(p); };
-    if (fe->groups == 4) {
+    if (fe->stft_r) {
+        stft_logmel_launch(fe, p, a->moments != nullptr, st);
+    } else if (fe->groups == 4) {
         if (a->moments) { if (p.out_bf16) launch(logmel_fused_kernel<4, true, __nv_bfloat16>); else launch(logmel_fused_kernel<4, true, float>); }
         else { if (p.out_bf16) launch(logmel_fused_kernel<4, false, __nv_bfloat16>); else launch(logmel_fused_kernel<4, false, float>); }
     } else {

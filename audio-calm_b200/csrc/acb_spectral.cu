@@ -31,68 +31,6 @@ constexpr int kStftComplexFramesPerCta = 4;  // frames per CTA of the complex ST
 constexpr int kIstftFramesPerCta = 4;        // frames per CTA of the inverse STFT, upper bound
 constexpr int kStftBwdRowsPerCta = 16;       // rows per CTA of the backward kernel
 
-__host__ __device__ constexpr int brev_bits(int x, int bits) {
-    int r = 0;
-    for (int i = 0; i < bits; ++i) r |= ((x >> i) & 1) << (bits - 1 - i);
-    return r;
-}
-__host__ __device__ constexpr int ilog2(int x) { return x <= 1 ? 0 : 1 + ilog2(x >> 1); }
-
-// In-register complex FFT of R points (R a power of two <= 32), natural order in and out: the cross-lane factor of the transform.
-template <int R>
-__device__ __forceinline__ void small_fft(float2 (&v)[R]) {
-    constexpr int kLog = ilog2(R);
-#pragma unroll
-    for (int i = 0; i < R; ++i) {
-        const int j = brev_bits(i, kLog);
-        if (i < j) { const float2 t = v[i]; v[i] = v[j]; v[j] = t; }
-    }
-#pragma unroll
-    for (int half = 1; half < R; half <<= 1) {
-#pragma unroll
-        for (int base = 0; base < R; base += 2 * half) {
-#pragma unroll
-            for (int j = 0; j < half; ++j) {
-                const int tw = j * (16 / half);                       // W_(2 half)^j = W_32^tw, tw < 16
-                const float wr = kCos32[tw], wi = -kSin32[tw];
-                const float2 u = v[base + j], w = v[base + j + half];
-                const float tr = fmaf(wr, w.x, -wi * w.y), ti = fmaf(wr, w.y, wi * w.x);
-                v[base + j] = make_float2(u.x + tr, u.y + ti);
-                v[base + j + half] = make_float2(u.x - tr, u.y - ti);
-            }
-        }
-    }
-}
-
-// The complex FFT of N = 32 R points that a group of R lanes computes together.  Stage 1: the lane's 32 stride-R inputs (packed,
-// bit-reversed order: see fft32_packed) -> in-register FFT-32, twiddle W_N^(r k1), hand-over to the group's exchange buffer at index
-// k1 + 33 r.  Stage 2 (after a __syncwarp): an R-point FFT across the group's lanes, in place; Z[k1 + 32 k2] ends up at index k1 + 33 k2.
-template <int R>
-__device__ __forceinline__ void group_fft_stage1(float2 (&pr)[16], float2 (&pi)[16], float2* buf, const float2* s_tw, int r) {
-    fft32_packed(pr, pi);
-#pragma unroll
-    for (int k = 0; k < 16; ++k) {
-        const float2 t0 = s_tw[k * R + r], t1 = s_tw[(k + 16) * R + r];     // table laid out [k][r]: a group's lanes read consecutive entries
-        buf[k + 33 * r] = make_float2(fmaf(pr[k].x, t0.x, -pi[k].x * t0.y), fmaf(pr[k].x, t0.y, pi[k].x * t0.x));
-        buf[k + 16 + 33 * r] = make_float2(fmaf(pr[k].y, t1.x, -pi[k].y * t1.y), fmaf(pr[k].y, t1.y, pi[k].y * t1.x));
-    }
-}
-template <int R>
-__device__ __forceinline__ void group_fft_stage2(float2* buf, int r) {
-    constexpr int kPerLane = 32 / R;
-#pragma unroll
-    for (int t = 0; t < kPerLane; ++t) {
-        const int k1 = r + R * t;             // interleaved over the lanes: the group's lanes touch consecutive 8-byte slots (a blocked r * kPerLane + t
-                                              // put the 32 lanes of a warp on 4 of the 16 bank pairs)
-        float2 v[R];
-#pragma unroll
-        for (int rr = 0; rr < R; ++rr) v[rr] = buf[k1 + 33 * rr];
-        small_fft<R>(v);
-#pragma unroll
-        for (int rr = 0; rr < R; ++rr) buf[k1 + 33 * rr] = v[rr];
-    }
-}
-__device__ __forceinline__ int buf_index(int k) { return (k & 31) + 33 * (k >> 5); }
 // sqrt / reciprocal sqrt as ONE special-function instruction each (about 1 ulp / 2 ulp; the correctly rounded sqrtf and the IEEE
 // division are 8-10 instructions apiece, paid twice per bin): the parity tolerance of these kernels is 1e-4 of the magnitudes
 __device__ __forceinline__ float sqrt_fast(float x) {

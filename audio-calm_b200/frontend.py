@@ -5,7 +5,7 @@
 reference's ``MelExtractor`` / ``process_audio_chunk`` signatures.
 
 torch is used for device memory, streams and (elsewhere) ``torch.distributed``; all arithmetic on the
-path runs in ``csrc/acb_kernels.cu``.
+path runs in ``csrc/acb_kernels.cu`` and ``csrc/acb_logmel_stft.cu``.
 """
 from __future__ import annotations
 
@@ -104,10 +104,17 @@ class LogMelFrontend:
     Defaults reproduce ``MelExtractor()`` (preprocess/core.py:33-48,60): 16 kHz, n_fft 1024, periodic Hann,
     hop 256, 80 slaney mels over 0-8000 Hz, power 2, ``log(clamp(., 1e-5))``.
 
-    ``fb`` may be any ``[513, n_mels]`` bank with 1 <= n_mels <= 128, no weight on the Nyquist bin and at most 4096 weights between
-    each band's first and last non-zero bin.  ``window`` must have the periodic-Hann property ``w[n + 512] = 1 - w[n]`` to within
-    1e-6: the kernel stages only the first half of the window and computes the second.  ``torch.hann_window(1024)`` has it; a
-    Hamming, a symmetric Hann or a scaled Hann window does not and raises ``AcbError``.
+    ``n_fft`` is 256, 512 or 1024 and ``1 <= hop_length <= n_fft``; the kernel is chosen from the pair, and others raise ``AcbError``.
+    ``window`` is ``[n_fft]`` and ``fb`` ``[n_fft // 2 + 1, n_mels]`` with 1 <= n_mels <= 128.  A window shorter than n_fft (torchaudio's
+    ``win_length``) is passed zero-padded and centred, as torch.stft pads it: ``F.pad(w, (left, n_fft - win_length - left))`` with
+    ``left = (n_fft - win_length) // 2``.
+
+    * n_fft 1024 with hop 256 runs the tuned kernel.  There ``fb`` may have no weight on the Nyquist bin and at most 4096 weights
+      between each band's first and last non-zero bin, and ``window`` must have the periodic-Hann property ``w[n + 512] = 1 - w[n]``
+      to within 1e-6: the kernel stages only the first half of the window and computes the second.  ``torch.hann_window(1024)`` has
+      it; a Hamming, a symmetric Hann or a scaled Hann window does not and raises ``AcbError``.
+    * Every other (n_fft, hop) runs the general STFT kernel: any window, weights on any bin including DC and Nyquist, up to 16384
+      banded weights.
     """
 
     def __init__(self, device: Union[str, torch.device, int] = "cuda", sample_rate: int = 16000, n_fft: int = 1024,

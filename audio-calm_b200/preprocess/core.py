@@ -45,7 +45,8 @@ class MelExtractor(nn.Module):
     """Log-mel extractor with the reference's constructor and forward contract (preprocess/core.py:33-61).
 
     ``forward(wav[..., L])`` -> ``[..., n_mels, 1 + L // hop_length]`` float32 on the input's device, natural log
-    of the slaney mel power spectrogram clamped at 1e-5.  The result is returned, like torchaudio's, as a
+    of the slaney mel power spectrogram (f_max 8000 Hz, as the reference hard-codes) clamped at 1e-5, for n_fft 256, 512 or
+    1024 and any hop_length in [1, n_fft] (``LogMelFrontend`` lists the kernels).  The result is returned, like torchaudio's, as a
     transposed view of a time-major buffer (strides ``(n_mels*T, 1, n_mels)`` for ``[B, n_mels, T]``).
     Buffers ``mel_transform.spectrogram.window`` and ``mel_transform.mel_scale.fb`` exist under the reference's
     state-dict keys and hold bit-identical values.

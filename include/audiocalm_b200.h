@@ -66,10 +66,15 @@ int64_t acb_plan_tiles(const int64_t* lengths_host, int32_t n_clips, int n_fft, 
 
 /* Build the device tables (replaces MelExtractor.__init__, preprocess/core.py:33-48).
  * window_host[n_fft] and fb_host[(n_fft/2+1) * n_mels] (row-major [freq][mel]) are the fp32 tables the
- * host derived with the reference's torch calls.  This build has kernels for n_fft = 1024, hop = 256,
- * n_mels <= 128; anything else returns ACB_ERR_UNSUPPORTED.  So does a window without the periodic-Hann property
- * |w[n + 512] - (1 - w[n])| <= 1e-6 (the kernel computes the second half of the window from the first), a filterbank with
- * weight on the Nyquist bin, or one with more than 4096 banded weights. */
+ * host derived with the reference's torch calls.  This build has kernels for n_fft in {256, 512, 1024} with
+ * 1 <= hop <= n_fft and 1 <= n_mels <= 128; anything else (n_fft 128, 400 or 2048, hop 0, hop > n_fft, n_mels 0 or 129)
+ * returns ACB_ERR_UNSUPPORTED.  The kernel is chosen from (n_fft, hop) alone:
+ *   - (1024, 256) runs the tuned kernel, which also returns ACB_ERR_UNSUPPORTED for a window without the periodic-Hann
+ *     property |w[n + 512] - (1 - w[n])| <= 1e-6 (it computes the second half of the window from the first), a filterbank
+ *     with weight on the Nyquist bin, or one with more than 4096 banded weights;
+ *   - every other pair runs the general STFT kernel: any fp32 window (a shorter window zero-padded and centred, as torch.stft
+ *     pads it), weights on any bin 0..n_fft/2 including DC and Nyquist, up to 16384 banded weights (each band's run from
+ *     its first to its last non-zero bin); a denser filterbank returns ACB_ERR_UNSUPPORTED ("too dense"). */
 int acb_frontend_create(acb_frontend** out, int device, int n_fft, int hop, int n_mels,
                         const float* window_host, const float* fb_host, float clamp_min, int log_kind);
 int acb_frontend_destroy(acb_frontend* fe);
