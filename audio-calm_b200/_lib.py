@@ -31,13 +31,15 @@ ACB_OK = 0
 ACB_F32, ACB_BF16, ACB_I16 = 0, 1, 2
 ACB_MEL_MAJOR, ACB_TIME_MAJOR = 0, 1
 ACB_LOG_NATURAL, ACB_LOG_10 = 0, 1
+ACB_PAD_REFLECT, ACB_PAD_CONSTANT = 0, 1
 ACB_ERR_INVALID, ACB_ERR_CUDA, ACB_ERR_UNSUPPORTED = -1, -2, -3
 ACB_FLAC_OK, ACB_FLAC_BAD_CLIP, ACB_FLAC_TOO_MANY_CANDIDATES, ACB_FLAC_NOT_TILED = 0, 1, 2, 3
 
 # every symbol include/audiocalm_b200.h declares (tests check the built library exports all of them)
 EXPORTED_SYMBOLS = [
     "acb_abi_version", "acb_last_error", "acb_frames_per_tile", "acb_frames_for_length", "acb_padded_frames",
-    "acb_plan_tiles", "acb_frontend_create", "acb_frontend_destroy", "acb_moments_workspace_bytes",
+    "acb_plan_tiles", "acb_frontend_create", "acb_frontend_create_stft", "acb_stft_frames_for_length", "acb_stft_plan_tiles",
+    "acb_frontend_destroy", "acb_moments_workspace_bytes",
     "acb_logmel_forward", "acb_frontend_check", "acb_frontend_set_kernel", "acb_peak_abs", "acb_process_audio_chunk", "acb_mixdown_peak", "acb_moments_accumulate",
     "acb_moments_finalize", "acb_normalize_per_utterance", "acb_logmel_forward_host", "acb_crop_pad", "acb_pad_transpose",
     "acb_moments_accumulate_workspace_bytes", "acb_pcm16_to_float", "acb_logmel_forward_host_pcm16",
@@ -81,6 +83,16 @@ class LogmelArgs(ctypes.Structure):
         ("bin_std", ctypes.c_void_p),
         ("moments", ctypes.c_void_p),
         ("moments_workspace", ctypes.c_void_p),
+    ]
+
+
+class StftOptions(ctypes.Structure):
+    """Mirror of ``struct acb_stft_options`` (include/audiocalm_b200.h): the front-end's spectrogram definition."""
+    _fields_ = [
+        ("pad", ctypes.c_int32),
+        ("pad_mode", ctypes.c_int32),
+        ("power", ctypes.c_int32),
+        ("magnitude_eps", ctypes.c_float),
     ]
 
 
@@ -172,6 +184,13 @@ def load() -> ctypes.CDLL:
         lib.acb_frontend_create.restype = ctypes.c_int
         lib.acb_frontend_create.argtypes = [ctypes.POINTER(vp), ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_int,
                                             vp, vp, f32, ctypes.c_int]
+        lib.acb_frontend_create_stft.restype = ctypes.c_int
+        lib.acb_frontend_create_stft.argtypes = [ctypes.POINTER(vp), ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_int,
+                                                 vp, vp, f32, ctypes.c_int, ctypes.POINTER(StftOptions)]
+        lib.acb_stft_frames_for_length.restype = i64
+        lib.acb_stft_frames_for_length.argtypes = [i64, ctypes.c_int, ctypes.c_int, ctypes.POINTER(StftOptions)]
+        lib.acb_stft_plan_tiles.restype = i64
+        lib.acb_stft_plan_tiles.argtypes = [vp, i32, ctypes.c_int, ctypes.c_int, ctypes.POINTER(StftOptions), i64, vp]
         lib.acb_frontend_destroy.restype = ctypes.c_int
         lib.acb_frontend_destroy.argtypes = [vp]
         lib.acb_moments_workspace_bytes.restype = i64

@@ -961,15 +961,84 @@ int64_t acb_padded_frames(int64_t frames, int multiple) {
     return r ? frames + (multiple - r) : frames;
 }
 
+}  // extern "C"
+
+// ---- spectrogram definitions (acb_stft_options) ----
+static acb_stft_options stft_options_or_default(const acb_stft_options* opt, int n_fft) {
+    return opt ? *opt : acb_stft_options{n_fft / 2, ACB_PAD_REFLECT, 2, 0.f};
+}
+
+static bool stft_options_default(const acb_stft_options& o, int n_fft) {
+    return o.pad == n_fft / 2 && o.pad_mode == ACB_PAD_REFLECT && o.power == 2;
+}
+
+// ACB_OK, or the error code with the envelope in `msg`
+static int stft_options_check(const acb_stft_options& o, int n_fft, std::string& msg) {
+    if (o.pad < 0 || o.pad > n_fft / 2) {
+        msg = "pad must be in [0, n_fft/2] = [0, " + std::to_string(n_fft / 2) + "] (got " + std::to_string(o.pad) + ")";
+        return ACB_ERR_INVALID;
+    }
+    if (o.pad_mode != ACB_PAD_REFLECT && o.pad_mode != ACB_PAD_CONSTANT) {
+        msg = "pad_mode must be ACB_PAD_REFLECT (0) or ACB_PAD_CONSTANT (1); replicate and circular padding have no kernel (got " +
+              std::to_string(o.pad_mode) + ")";
+        return ACB_ERR_UNSUPPORTED;
+    }
+    if (o.power != 1 && o.power != 2) {
+        msg = "power must be 1 (magnitude) or 2 (power) (got " + std::to_string(o.power) + ")";
+        return ACB_ERR_INVALID;
+    }
+    if (!std::isfinite(o.magnitude_eps) || o.magnitude_eps < 0.f) {
+        msg = "magnitude_eps must be finite and >= 0 (got " + std::to_string(o.magnitude_eps) + ")";
+        return ACB_ERR_INVALID;
+    }
+    if (o.power == 2 && o.magnitude_eps != 0.f) {
+        msg = "magnitude_eps applies to power 1 only; it must be 0 with power 2";
+        return ACB_ERR_INVALID;
+    }
+    return ACB_OK;
+}
+
+// T = 1 + (L + 2 pad - n_fft) / hop, or -1 below the definition's minimum length (torch.stft / F.pad's limits)
+static int64_t stft_frames(int64_t length, int n_fft, int hop, const acb_stft_options& o) {
+    if (n_fft <= 0 || hop <= 0) return -1;
+    if (length + 2 * (int64_t)o.pad < n_fft) return -1;
+    if (o.pad_mode == ACB_PAD_REFLECT ? length <= o.pad : length < 1) return -1;
+    return 1 + (length + 2 * (int64_t)o.pad - n_fft) / hop;
+}
+
+static std::string stft_minimum(int n_fft, const acb_stft_options& o) {
+    if (stft_options_default(o, n_fft)) return "reflect padding needs more than " + std::to_string(n_fft / 2);
+    const int64_t need = std::max<int64_t>(n_fft - 2 * (int64_t)o.pad, o.pad_mode == ACB_PAD_REFLECT ? o.pad + 1 : 1);
+    return "n_fft=" + std::to_string(n_fft) + " with " + (o.pad_mode == ACB_PAD_REFLECT ? "reflect" : "constant") + " padding of " +
+           std::to_string(o.pad) + " needs at least " + std::to_string(need);
+}
+
+extern "C" {
+
+int64_t acb_stft_frames_for_length(int64_t length, int n_fft, int hop, const acb_stft_options* opt) {
+    const acb_stft_options o = stft_options_or_default(opt, n_fft);
+    std::string msg;
+    if (stft_options_check(o, n_fft, msg) != ACB_OK) return -1;
+    return stft_frames(length, n_fft, hop, o);
+}
+
 int64_t acb_plan_tiles(const int64_t* lengths_host, int32_t n_clips, int n_fft, int hop, int64_t frame_capacity,
                        int32_t* tile_start_host) {
+    return acb_stft_plan_tiles(lengths_host, n_clips, n_fft, hop, nullptr, frame_capacity, tile_start_host);
+}
+
+int64_t acb_stft_plan_tiles(const int64_t* lengths_host, int32_t n_clips, int n_fft, int hop, const acb_stft_options* opt,
+                            int64_t frame_capacity, int32_t* tile_start_host) {
     if (!lengths_host || !tile_start_host || n_clips < 0) return fail(ACB_ERR_INVALID, "acb_plan_tiles: null argument");
+    const acb_stft_options o = stft_options_or_default(opt, n_fft);
+    std::string msg;
+    if (stft_options_check(o, n_fft, msg) != ACB_OK) return fail(ACB_ERR_INVALID, "acb_plan_tiles: " + msg);
     int64_t total = 0;
     for (int32_t i = 0; i < n_clips; ++i) {
-        const int64_t T = acb_frames_for_length(lengths_host[i], n_fft, hop);
+        const int64_t T = stft_frames(lengths_host[i], n_fft, hop, o);
         if (T < 0) {
             return fail(ACB_ERR_INVALID, "acb_plan_tiles: clip " + std::to_string(i) + " has " + std::to_string(lengths_host[i]) +
-                                             " samples; reflect padding needs more than " + std::to_string(n_fft / 2));
+                                             " samples; " + stft_minimum(n_fft, o));
         }
         const int64_t cover = frame_capacity > 0 ? frame_capacity : T;
         tile_start_host[i] = (int32_t)total;
@@ -982,16 +1051,25 @@ int64_t acb_plan_tiles(const int64_t* lengths_host, int32_t n_clips, int n_fft, 
 
 int acb_frontend_create(acb_frontend** out, int device, int n_fft, int hop, int n_mels, const float* window_host,
                         const float* fb_host, float clamp_min, int log_kind) {
+    return acb_frontend_create_stft(out, device, n_fft, hop, n_mels, window_host, fb_host, clamp_min, log_kind, nullptr);
+}
+
+int acb_frontend_create_stft(acb_frontend** out, int device, int n_fft, int hop, int n_mels, const float* window_host,
+                             const float* fb_host, float clamp_min, int log_kind, const acb_stft_options* opt) {
     if (!out || !window_host || !fb_host) return fail(ACB_ERR_INVALID, "acb_frontend_create: null argument");
-    // (1024, 256) runs the tuned kernel below; every other supported (n_fft, hop) the general STFT kernel (acb_logmel_stft.cu)
-    const bool tuned = n_fft == kNfft && hop == kHop;
+    const acb_stft_options so = stft_options_or_default(opt, n_fft);
+    // (1024, 256) with the default definition runs the tuned kernel below; every other supported (n_fft, hop), and every one with
+    // another definition, the general STFT kernel (acb_logmel_stft.cu)
+    const bool tuned = n_fft == kNfft && hop == kHop && stft_options_default(so, n_fft);
     if (!tuned && !stft_logmel_supported(n_fft, hop))
         return fail(ACB_ERR_UNSUPPORTED, "acb_frontend_create: this build has kernels for n_fft 256, 512 or 1024 with 1 <= hop <= n_fft (got n_fft=" +
                                              std::to_string(n_fft) + ", hop=" + std::to_string(hop) + ")");
     if (n_mels < 1 || n_mels > kMaxMels) return fail(ACB_ERR_UNSUPPORTED, "acb_frontend_create: n_mels must be in [1, 128]");
     if (log_kind != ACB_LOG_NATURAL && log_kind != ACB_LOG_10) return fail(ACB_ERR_INVALID, "acb_frontend_create: bad log_kind");
     if (!(clamp_min >= 1.17549435e-38f)) return fail(ACB_ERR_INVALID, "acb_frontend_create: clamp_min must be a positive normal float");
-    if (!tuned) return stft_frontend_create(out, device, n_fft, hop, n_mels, window_host, fb_host, clamp_min, log_kind);
+    std::string msg;
+    if (const int rc = stft_options_check(so, n_fft, msg)) return fail(rc, "acb_frontend_create_stft: " + msg);
+    if (!tuned) return stft_frontend_create(out, device, n_fft, hop, n_mels, window_host, fb_host, clamp_min, log_kind, so);
     // The kernel stages only w[0 .. N/2 - 1] and computes the second half as 1 - w[n] (the periodic-Hann property).  A window
     // without that property would give wrong features silently; fp32 periodic Hann deviates by 1.8e-7.
     for (int n = 0; n < kNfft / 2; ++n) {
@@ -1112,6 +1190,7 @@ int acb_frontend_create(acb_frontend** out, int device, int n_fft, int hop, int 
     ACB_CUDA(cudaGetDevice(&prev));
     ACB_CUDA(cudaSetDevice(device));
     auto* fe = new acb_frontend();
+    fe->opt = so;
     fe->device = device; fe->n_fft = n_fft; fe->hop = hop; fe->n_mels = n_mels; fe->n_weights = (int)weights.size();
     fe->n_plan_w = (int)plan_w.size();
     fe->log_kind = log_kind; fe->clamp_min = clamp_min;
@@ -1249,9 +1328,9 @@ int acb_logmel_forward(const acb_frontend* fe, const acb_logmel_args* a, void* s
         if ((int64_t)p.uniform_tiles_per_clip * a->n_clips != a->n_tiles)
             return fail(ACB_ERR_INVALID, "acb_logmel_forward: n_tiles does not match n_clips * tiles per clip");
     } else if (!a->tile_start) {
-        const int64_t T = acb_frames_for_length(a->uniform_length, fe->n_fft, fe->hop);
+        const int64_t T = stft_frames(a->uniform_length, fe->n_fft, fe->hop, fe->opt);
         if (T < 0) return fail(ACB_ERR_INVALID, "acb_logmel_forward: clips of " + std::to_string(a->uniform_length) +
-                                                    " samples are too short for reflect padding of " + std::to_string(fe->n_fft / 2));
+                                                    " samples are too short: " + stft_minimum(fe->n_fft, fe->opt));
         const int64_t cover = a->fill_tail ? a->frame_capacity : T;
         p.uniform_tiles_per_clip = (int)((cover + kTileFrames - 1) / kTileFrames);
         if ((int64_t)p.uniform_tiles_per_clip * a->n_clips != a->n_tiles)
@@ -1512,7 +1591,7 @@ static int forward_host_impl(const acb_frontend* fe_c, const void* wav_host, int
     if (!fe_c || !wav_host || !tmpl || !dev_in || !dev_out) return fail(ACB_ERR_INVALID, "acb_logmel_forward_host: null argument");
     if (n_clips <= 0) return ACB_OK;
     auto* fe = const_cast<acb_frontend*>(fe_c);
-    const int64_t T = acb_frames_for_length(length, fe->n_fft, fe->hop);
+    const int64_t T = stft_frames(length, fe->n_fft, fe->hop, fe->opt);
     if (T < 0) return fail(ACB_ERR_INVALID, "acb_logmel_forward_host: clips too short");
     n_chunks = std::max(1, std::min(n_chunks, n_clips));
     const int64_t cap = tmpl->frame_capacity;

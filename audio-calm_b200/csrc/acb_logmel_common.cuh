@@ -85,13 +85,15 @@ struct ClipCursor {
     float gain;            // squared waveform scale (fused peak normalisation), 1 otherwise
 };
 
-__device__ __forceinline__ void cursor_load_clip(const LogmelParams& p, ClipCursor& c, int hop) {
+// T = 1 + (L + len_off) / hop with len_off = 2 pad - n_fft of the framing: 0 for torch.stft(center=True), a compile-time 0 in the
+// tuned kernel.
+__device__ __forceinline__ void cursor_load_clip(const LogmelParams& p, ClipCursor& c, int hop, int len_off = 0) {
     const int i = c.clip;
     c.wav_base = p.clip_offset ? p.clip_offset[i] : (long long)i * p.clip_stride;
     c.length = p.clip_length ? p.clip_length[i] : p.uniform_length;
     c.out_base = p.out_offset ? p.out_offset[i] : (long long)i * p.out_clip_stride;
     c.cap = (int)(p.frame_capacity_per_clip ? p.frame_capacity_per_clip[i] : p.frame_capacity);
-    c.frames = 1 + (int)(c.length / hop);
+    c.frames = 1 + (int)((c.length + len_off) / hop);
     const int rem = c.frames % p.pad_multiple;
     c.frames_padded = rem ? c.frames + (p.pad_multiple - rem) : c.frames;
     c.tiles_in_clip = p.tile_start ? (__ldg(p.tile_start + i + 1) - __ldg(p.tile_start + i)) : p.uniform_tiles_per_clip;
@@ -105,7 +107,7 @@ __device__ __forceinline__ void cursor_load_clip(const LogmelParams& p, ClipCurs
     }
 }
 
-__device__ __forceinline__ void cursor_init(const LogmelParams& p, ClipCursor& c, long long tile, int hop) {
+__device__ __forceinline__ void cursor_init(const LogmelParams& p, ClipCursor& c, long long tile, int hop, int len_off = 0) {
     if (p.tile_start == nullptr) {
         c.clip = (int)(tile / p.uniform_tiles_per_clip);
         c.tile_in_clip = (int)(tile - (long long)c.clip * p.uniform_tiles_per_clip);
@@ -118,13 +120,13 @@ __device__ __forceinline__ void cursor_init(const LogmelParams& p, ClipCursor& c
         c.clip = lo;
         c.tile_in_clip = (int)(tile - __ldg(p.tile_start + lo));
     }
-    cursor_load_clip(p, c, hop);
+    cursor_load_clip(p, c, hop, len_off);
 }
 
-__device__ __forceinline__ void cursor_advance(const LogmelParams& p, ClipCursor& c, int hop) {
+__device__ __forceinline__ void cursor_advance(const LogmelParams& p, ClipCursor& c, int hop, int len_off = 0) {
     if (++c.tile_in_clip >= c.tiles_in_clip) {
         c.tile_in_clip = 0;
-        do { ++c.clip; cursor_load_clip(p, c, hop); } while (c.tiles_in_clip == 0 && c.clip + 1 < p.n_clips);
+        do { ++c.clip; cursor_load_clip(p, c, hop, len_off); } while (c.tiles_in_clip == 0 && c.clip + 1 < p.n_clips);
     }
 }
 
@@ -248,14 +250,16 @@ __device__ __forceinline__ void two_sum_add(float2& acc, float x) {
 
 }  // namespace acb
 
-// Device-resident tables of one front-end.  Two routes share the handle: (n_fft, hop) = (1024, 256) runs logmel_fused_kernel with its
-// mel plan (acb_kernels.cu); every other supported (n_fft, hop) runs logmel_stft_kernel<R> with R = n_fft / 32 (acb_logmel_stft.cu).
+// Device-resident tables of one front-end.  Two routes share the handle: (n_fft, hop) = (1024, 256) with the default spectrogram
+// definition runs logmel_fused_kernel with its mel plan (acb_kernels.cu); every other supported (n_fft, hop), and every (n_fft, hop)
+// with another definition, runs logmel_stft_kernel<R> with R = n_fft / 32 (acb_logmel_stft.cu).
 struct acb_frontend {
     int device = 0;
     int n_fft = 0, hop = 0, n_mels = 0, n_weights = 0, log_kind = 0;
     float clamp_min = 0.f;
     int num_sms = 0;
     int stft_r = 0;        // 0: logmel_fused_kernel; 8, 16 or 32: logmel_stft_kernel<stft_r>
+    acb_stft_options opt{};   // spectrogram definition (pad, pad mode, power, magnitude eps); only the STFT kernel takes other than the default
     int groups = 0;        // groups per CTA (template parameter G of the kernel): 4, or 2 when four do not fit in shared memory; 1 for the STFT kernel
     int grid = 0;          // persistent grid (CTAs)
     int smem_bytes = 0;
@@ -283,10 +287,10 @@ struct acb_frontend {
 
 namespace acb {
 // acb_logmel_stft.cu: the general route.  stft_logmel_supported says whether (n_fft, hop) has a kernel there; stft_frontend_create
-// validates the filterbank and builds the handle (n_mels, log_kind and clamp_min are checked by the caller); stft_logmel_launch
+// validates the filterbank and builds the handle (n_mels, log_kind, clamp_min and the options are checked by the caller); stft_logmel_launch
 // enqueues one launch of the kernel for the batch `p` describes.
 bool stft_logmel_supported(int n_fft, int hop);
 int stft_frontend_create(acb_frontend** out, int device, int n_fft, int hop, int n_mels, const float* window_host, const float* fb_host,
-                         float clamp_min, int log_kind);
+                         float clamp_min, int log_kind, const acb_stft_options& opt);
 void stft_logmel_launch(const acb_frontend* fe, const LogmelParams& p, bool moments, cudaStream_t st);
 }  // namespace acb

@@ -3,18 +3,23 @@
 // (logmel_fused_kernel, acb_kernels.cu); acb_frontend_create routes every other supported pair here.  The launch contract is the
 // same acb_logmel_args: uniform and ragged batches, fused peak gain, fp32 / bf16 in both layouts, reflected pad columns, tail fill,
 // scalar / per-band affine and fp64 per-band moments, with the cursor, store and fill helpers of acb_logmel_common.cuh.
+// The handle's spectrogram definition (acb_stft_options) sets the framing pad p (T = 1 + (L + 2 p - n_fft) / hop), reflect or
+// constant padding, and power 2 or magnitude sqrt(|X|^2 + eps); a definition other than the centred power spectrogram runs here at
+// every supported (n_fft, hop), (1024, 256) included.
 //
 // Mapping: one CTA of 4 R threads works through a contiguous range of 8-frame tiles (acb_frames_per_tile), persistent over the grid.
 // Per tile:
-//   1. the tile's (8 - 1) * hop + n_fft samples are staged in shared memory by 4-byte cp.async copies issued while the previous tile's
-//      mel phase runs.  Each copy computes its own source index: reflection about sample 0 / L - 1 (torch.stft center=True,
-//      pad_mode="reflect") and zero fill beyond it come for free, no read leaves [clip_offset, clip_offset + clip_length), and a
-//      hop that is not a multiple of 4 samples needs no alignment;
+//   1. the tile's (8 - 1) * hop + n_fft samples, from sample f0 * hop - p on, are staged in shared memory by 4-byte cp.async copies
+//      issued while the previous tile's mel phase runs.  Each copy computes its own source index: reflection about sample 0 / L - 1
+//      (pad_mode="reflect"), or zeros outside [0, L) (pad_mode="constant", a cp.async of source size 0), and zero fill beyond come
+//      for free, no read leaves [clip_offset, clip_offset + clip_length), and a hop that is not a multiple of 4 samples needs no
+//      alignment;
 //   2. lane group g (R lanes) takes frames 2g and 2g + 1 of the tile and runs ONE complex n_fft-point group FFT of A + iB
 //      (acb_fft32.cuh: in-register FFT-32 per lane, twiddle, R-point FFT across the lanes through shared memory), with the whole
 //      window held in registers;
-//   3. the two real spectra are separated (Z[k], Z[N - k]) into 4 |X|^2 for bins 0..n_fft/2 and written over the FFT buffer as
-//      [bin][8 frames] (the 1/4 is folded into the weights);
+//   3. the two real spectra are separated (Z[k], Z[N - k]) into 4 |X|^2 for bins 0..n_fft/2 -- with power 1 into
+//      sqrt(s^2 4 |X|^2 + 4 eps) = 2 sqrt(|s X|^2 + eps), the peak gain s^2 taken under the root -- and written over the FFT buffer
+//      as [bin][8 frames] (the 1/4, or 1/2, is folded into the weights);
 //   4. thread (band, frame quad) sums its band's contiguous run of weights against four frames with 16-byte power loads, then
 //      clamp, log, moments and affine; the tile is staged in shared memory and stored by store_tile (masking, reflected pad-to-4
 //      columns, tail fill).
@@ -39,8 +44,14 @@ struct StftLogmelParams {
     int n_weights;
     const float* window;       // [N]
     const float2* twiddle;     // [32][R]: entry k * R + r = W_N^(r k)
-    const float* weights;      // [n_weights] band after band, each its run of bins, times 1/4
+    const float* weights;      // [n_weights] band after band, each its run of bins, times 1/4 (power 2) or 1/2 (power 1)
     const int4* band;          // [n_mels] {first bin, bins, offset in weights, 0}
+    // spectrogram definition (acb_stft_options), read by the kDefinition instantiations only
+    int pad;                   // samples padded on each side before framing
+    int len_off;               // 2 pad - N: T = 1 + (L + len_off) / hop
+    int pad_constant;          // 1: zeros outside the clip; 0: reflection about its first and last sample
+    int magnitude;             // 1: power rows hold 2 sqrt(|X|^2 + eps) (power 1); 0: 4 |X|^2 (power 2)
+    float eps4;                // 4 * magnitude_eps
 };
 
 struct StftSmem {
@@ -72,28 +83,37 @@ __device__ __forceinline__ void cp_async4(float* dst, const float* src, bool val
                  ::"r"(static_cast<unsigned>(__cvta_generic_to_shared(dst))), "l"(src), "r"(valid ? 4 : 0) : "memory");
 }
 
-// Request the tile's samples (relative index i = sample f0 * hop - N/2 + i of the clip, reflected at both ends, zero beyond).
-template <int R>
-__device__ __forceinline__ void stage_tile(const LogmelParams& p, const ClipCursor& c, int hop, float* s_samples, int tid) {
+// Request the tile's samples (relative index i = sample f0 * hop - pad + i of the clip; reflected at both ends in reflect mode, zero
+// beyond; zero outside the clip in constant mode).
+template <int R, bool kDefinition>
+__device__ __forceinline__ void stage_tile(const StftLogmelParams& sp, const ClipCursor& c, int hop, float* s_samples, int tid) {
     constexpr int N = 32 * R, kThreads = 4 * R;
-    const long long g0 = (long long)c.tile_in_clip * kTileFrames * hop - N / 2;
+    const LogmelParams& p = sp.c;
+    const bool constant = kDefinition && sp.pad_constant;
+    const long long g0 = (long long)c.tile_in_clip * kTileFrames * hop - (kDefinition ? sp.pad : N / 2);
     const int n = (kTileFrames - 1) * hop + N;
     const float* src = p.wav + c.wav_base;
     const long long L = c.length;
     for (int i = tid; i < n; i += kThreads) {
         long long idx = g0 + i;
-        if (idx < 0) idx = -idx;
-        if (idx >= L) idx = 2 * (L - 1) - idx;
+        if (!constant) {
+            if (idx < 0) idx = -idx;
+            if (idx >= L) idx = 2 * (L - 1) - idx;
+        }
         const bool ok = idx >= 0 && idx < L;
         cp_async4(s_samples + i, src + (ok ? idx : 0), ok);
     }
     asm volatile("cp.async.commit_group;" ::: "memory");
 }
 
-template <int R, bool kMoments, typename OutT>
+// kDefinition = false: the centred, reflect-padded power spectrogram (pad N/2 at compile time); true: the handle's spectrogram
+// definition (acb_stft_options), read from sp
+template <int R, bool kMoments, typename OutT, bool kDefinition>
 __global__ void __launch_bounds__(4 * R) logmel_stft_kernel(const StftLogmelParams sp) {
     constexpr int N = 32 * R, kThreads = 4 * R, kHalf = N / 2;
     const LogmelParams& p = sp.c;
+    const int len_off = kDefinition ? sp.len_off : 0;
+    const bool magnitude = kDefinition && sp.magnitude;
     extern __shared__ __align__(16) float smem[];
     const int hop = sp.hop, n_mels = p.n_mels, S = out_row_stride(n_mels);
     const StftSmem L = stft_smem(R, hop, n_mels, sp.n_weights);
@@ -133,8 +153,8 @@ __global__ void __launch_bounds__(4 * R) logmel_stft_kernel(const StftLogmelPara
     const long long t_end = (long long)p.n_tiles * (blockIdx.x + 1) / gridDim.x;
     ClipCursor cur;
     if (t_begin < t_end) {
-        cursor_init(p, cur, t_begin, hop);
-        if (cur.tile_in_clip * kTileFrames < cur.frames) stage_tile<R>(p, cur, hop, s_samples, tid);
+        cursor_init(p, cur, t_begin, hop, len_off);
+        if (cur.tile_in_clip * kTileFrames < cur.frames) stage_tile<R, kDefinition>(sp, cur, hop, s_samples, tid);
     }
 
     for (long long tile = t_begin; tile < t_end; ++tile) {
@@ -159,8 +179,8 @@ __global__ void __launch_bounds__(4 * R) logmel_stft_kernel(const StftLogmelPara
 
         ClipCursor nxt = cur;
         if (tile + 1 < t_end) {
-            cursor_advance(p, nxt, hop);
-            if (nxt.tile_in_clip * kTileFrames < nxt.frames) stage_tile<R>(p, nxt, hop, s_samples, tid);
+            cursor_advance(p, nxt, hop, len_off);
+            if (nxt.tile_in_clip * kTileFrames < nxt.frames) stage_tile<R, kDefinition>(sp, nxt, hop, s_samples, tid);
         }
 
         // ---- group FFT of the pair, separation into 4 |X_A|^2, 4 |X_B|^2 for bins k = r + R t <= N/2 ----
@@ -179,6 +199,10 @@ __global__ void __launch_bounds__(4 * R) logmel_stft_kernel(const StftLogmelPara
                     const float apc = z.x + zc.x, bmd = z.y - zc.y, amc = z.x - zc.x, bpd = z.y + zc.y;
                     pwa[t] = fmaf(apc, apc, bmd * bmd);
                     pwb[t] = fmaf(amc, amc, bpd * bpd);
+                    if (magnitude) {   // 2 sqrt(s^2 |X|^2 + eps): the peak gain s^2 goes under the root with the eps
+                        pwa[t] = sqrtf(fmaf(cur.gain, pwa[t], sp.eps4));
+                        pwb[t] = sqrtf(fmaf(cur.gain, pwb[t], sp.eps4));
+                    }
                 }
             }
         }
@@ -193,6 +217,7 @@ __global__ void __launch_bounds__(4 * R) logmel_stft_kernel(const StftLogmelPara
         __syncthreads();
 
         // ---- banded mel projection over four frames per thread, clamp, log, moments, affine -> staged tile ----
+        const float gain = magnitude ? 1.f : cur.gain;   // a magnitude spectrum took its gain before the root
         if (has_frames) {
             for (int base = 0; base < 2 * n_mels; base += kThreads) {   // uniform trip count: the moments' shuffle needs every lane
                 const int item = base + tid;
@@ -211,7 +236,7 @@ __global__ void __launch_bounds__(4 * R) logmel_stft_kernel(const StftLogmelPara
                     acc.z = fmaf(wi, v.z, acc.z);
                     acc.w = fmaf(wi, v.w, acc.w);
                 }
-                float v[4] = {acc.x * cur.gain, acc.y * cur.gain, acc.z * cur.gain, acc.w * cur.gain};
+                float v[4] = {acc.x * gain, acc.y * gain, acc.z * gain, acc.w * gain};
 #pragma unroll
                 for (int j = 0; j < 4; ++j) v[j] = (v[j] > p.clamp_min) ? lg2_normal(v[j]) * p.log_scale : p.log_floor;
                 if (kMoments) {
@@ -263,10 +288,14 @@ bool stft_logmel_supported(int n_fft, int hop) {
 
 template <int R, typename F>
 static void for_each_instantiation(F&& f) {
-    f(logmel_stft_kernel<R, false, float>);
-    f(logmel_stft_kernel<R, false, __nv_bfloat16>);
-    f(logmel_stft_kernel<R, true, float>);
-    f(logmel_stft_kernel<R, true, __nv_bfloat16>);
+    f(logmel_stft_kernel<R, false, float, false>);
+    f(logmel_stft_kernel<R, false, __nv_bfloat16, false>);
+    f(logmel_stft_kernel<R, true, float, false>);
+    f(logmel_stft_kernel<R, true, __nv_bfloat16, false>);
+    f(logmel_stft_kernel<R, false, float, true>);
+    f(logmel_stft_kernel<R, false, __nv_bfloat16, true>);
+    f(logmel_stft_kernel<R, true, float, true>);
+    f(logmel_stft_kernel<R, true, __nv_bfloat16, true>);
 }
 
 template <typename F>
@@ -277,10 +306,11 @@ static void for_each_instantiation(int R, F&& f) {
 }
 
 int stft_frontend_create(acb_frontend** out, int device, int n_fft, int hop, int n_mels, const float* window_host, const float* fb_host,
-                         float clamp_min, int log_kind) {
+                         float clamp_min, int log_kind, const acb_stft_options& opt) {
     const int R = n_fft / 32, n_freq = n_fft / 2 + 1;
     // banded form of the filterbank: each band's run from its first to its last non-zero bin; the 1/4 of the packed-pair power
-    // spectrum is folded in (exact scaling)
+    // spectrum (4 |X|^2), or the 1/2 of its magnitude (2 sqrt(|X|^2 + eps)), is folded in (exact scaling)
+    const float fold = opt.power == 1 ? 0.5f : 0.25f;
     std::vector<int4> band(n_mels);
     std::vector<float> weights;
     for (int m = 0; m < n_mels; ++m) {
@@ -288,7 +318,7 @@ int stft_frontend_create(acb_frontend** out, int device, int n_fft, int hop, int
         for (int f = 0; f < n_freq; ++f)
             if (fb_host[(size_t)f * n_mels + m] != 0.f) { if (lo < 0) lo = f; hi = f; }
         band[m] = make_int4(lo < 0 ? 0 : lo, lo < 0 ? 0 : hi - lo + 1, (int)weights.size(), 0);
-        for (int f = lo; lo >= 0 && f <= hi; ++f) weights.push_back(fb_host[(size_t)f * n_mels + m] * 0.25f);
+        for (int f = lo; lo >= 0 && f <= hi; ++f) weights.push_back(fb_host[(size_t)f * n_mels + m] * fold);
     }
     if ((int)weights.size() > kStftMaxWeights)
         return fail(ACB_ERR_UNSUPPORTED, "acb_frontend_create: filterbank too dense (" + std::to_string(weights.size()) +
@@ -310,6 +340,7 @@ int stft_frontend_create(acb_frontend** out, int device, int n_fft, int hop, int
     fe->device = device; fe->n_fft = n_fft; fe->hop = hop; fe->n_mels = n_mels; fe->n_weights = (int)weights.size();
     fe->log_kind = log_kind; fe->clamp_min = clamp_min;
     fe->stft_r = R;
+    fe->opt = opt;
     fe->groups = 1;
 
     size_t o = 0;
@@ -369,12 +400,23 @@ void stft_logmel_launch(const acb_frontend* fe, const LogmelParams& p, bool mome
     sp.twiddle = fe->d_stft_twiddle;
     sp.weights = fe->d_stft_weights;
     sp.band = fe->d_stft_band;
+    sp.pad = fe->opt.pad;
+    sp.len_off = 2 * fe->opt.pad - fe->n_fft;
+    sp.pad_constant = fe->opt.pad_mode == ACB_PAD_CONSTANT;
+    sp.magnitude = fe->opt.power == 1;
+    sp.eps4 = 4.f * fe->opt.magnitude_eps;
     const int R = fe->stft_r;
     auto launch = [&](auto kernel) { kernel<<<fe->grid, 4 * R, fe->smem_bytes, st>>>(sp); };
-    auto dispatch = [&](auto r_tag) {
+    // the centred power spectrogram runs the instantiation with its framing and power fixed at compile time
+    const bool definition = !(fe->opt.pad == fe->n_fft / 2 && fe->opt.pad_mode == ACB_PAD_REFLECT && fe->opt.power == 2);
+    auto dispatch_def = [&](auto r_tag, auto def_tag) {
         constexpr int kR = decltype(r_tag)::value;
-        if (moments) { if (p.out_bf16) launch(logmel_stft_kernel<kR, true, __nv_bfloat16>); else launch(logmel_stft_kernel<kR, true, float>); }
-        else { if (p.out_bf16) launch(logmel_stft_kernel<kR, false, __nv_bfloat16>); else launch(logmel_stft_kernel<kR, false, float>); }
+        constexpr bool kD = decltype(def_tag)::value;
+        if (moments) { if (p.out_bf16) launch(logmel_stft_kernel<kR, true, __nv_bfloat16, kD>); else launch(logmel_stft_kernel<kR, true, float, kD>); }
+        else { if (p.out_bf16) launch(logmel_stft_kernel<kR, false, __nv_bfloat16, kD>); else launch(logmel_stft_kernel<kR, false, float, kD>); }
+    };
+    auto dispatch = [&](auto r_tag) {
+        if (definition) dispatch_def(r_tag, std::true_type{}); else dispatch_def(r_tag, std::false_type{});
     };
     if (R == 8) dispatch(std::integral_constant<int, 8>{});
     else if (R == 16) dispatch(std::integral_constant<int, 16>{});

@@ -36,14 +36,22 @@ def _stream_ptr(device: torch.device) -> int:
     return torch.cuda.current_stream(device).cuda_stream
 
 
-def frames_for_length(length: int, n_fft: int = 1024, hop: int = 256) -> int:
+def frames_for_length(length: int, n_fft: int = 1024, hop: int = 256, *, frame_pad: Optional[int] = None,
+                      pad_mode: str = "reflect") -> int:
     """``1 + L // hop`` (torch.stft center=True via preprocess/core.py:55); RuntimeError when ``L <= n_fft // 2``
-    exactly like the reference's reflect padding."""
-    if length <= n_fft // 2:
+    exactly like the reference's reflect padding.
+
+    With ``frame_pad`` (samples padded on each side before framing; ``None`` is ``n_fft // 2``, center=True) the count is
+    ``1 + (L + 2 frame_pad - n_fft) // hop``, and RuntimeError is raised where torch raises: reflect padding needs
+    ``L > frame_pad``, constant padding ``L >= 1``, and every mode ``L + 2 frame_pad >= n_fft``."""
+    p = n_fft // 2 if frame_pad is None else int(frame_pad)
+    if pad_mode == "reflect" and length <= p:
         raise RuntimeError(
             f"Argument #4: Padding size should be less than the corresponding input dimension, but got: "
-            f"padding ({n_fft // 2}, {n_fft // 2}) at dimension 2 of input of length {length}")
-    return 1 + length // hop
+            f"padding ({p}, {p}) at dimension 2 of input of length {length}")
+    if length < 1 or length + 2 * p < n_fft:
+        raise RuntimeError(f"stft: a clip of {length} samples padded by {p} on each side is shorter than n_fft={n_fft}")
+    return 1 + (length + 2 * p - n_fft) // hop
 
 
 def padded_frames(frames: int, multiple: int = 4) -> int:
@@ -58,7 +66,8 @@ class RaggedBatch:
     offsets: torch.Tensor    # [B] int64 (device)
     lengths: torch.Tensor    # [B] int64 (device)
     lengths_host: np.ndarray  # [B] int64
-    # launch plans derived from the lengths alone, built on first use and kept with the batch (key: n_fft, hop, pad_multiple):
+    # launch plans derived from the lengths alone, built on first use and kept with the batch (key: n_fft, hop, framing pad, pad
+    # mode, pad_multiple):
     # frame counts (host + device) and the per-clip tile prefix sums the kernel walks.  A batch that is forwarded more than once
     # (peak pass + features, statistics + features, several epochs over cached batches) pays for them once.
     plans: dict = field(default_factory=dict, repr=False, compare=False)
@@ -115,12 +124,34 @@ class LogMelFrontend:
       it; a Hamming, a symmetric Hann or a scaled Hann window does not and raises ``AcbError``.
     * Every other (n_fft, hop) runs the general STFT kernel: any window, weights on any bin including DC and Nyquist, up to 16384
       banded weights.
+
+    The spectrogram definition follows torchaudio's ``MelSpectrogram`` arguments of the same names: ``power`` 2.0 (power) or 1.0
+    (magnitude), ``center`` and ``pad_mode`` ``"reflect"`` or ``"constant"`` (zeros).  ``frame_pad`` overrides the pad that ``center``
+    implies (``n_fft // 2`` or 0): ``(n_fft - hop_length) // 2`` is the HiFi-GAN / BigVGAN ``mel_spectrogram`` convention
+    (``F.pad`` by that much, then ``torch.stft(center=False)``).  ``magnitude_eps`` is added under the square root of a magnitude
+    spectrogram, ``sqrt(re^2 + im^2 + eps)`` (1e-9 in HiFi-GAN); it must be 0 with power 2.  With the defaults (centred, reflect, power
+    2) the kernel is chosen from (n_fft, hop) as above; any other definition runs the general STFT kernel at every supported
+    (n_fft, hop), 1024 / 256 included, with its envelope.  A clip of L samples has ``1 + (L + 2 pad - n_fft) // hop`` frames.
     """
 
     def __init__(self, device: Union[str, torch.device, int] = "cuda", sample_rate: int = 16000, n_fft: int = 1024,
                  hop_length: int = 256, n_mels: int = 80, f_min: float = 0.0, f_max: float = 8000.0,
                  clamp_min: float = 1e-5, log: str = "ln",
-                 window: Optional[torch.Tensor] = None, fb: Optional[torch.Tensor] = None):
+                 window: Optional[torch.Tensor] = None, fb: Optional[torch.Tensor] = None, power: float = 2.0,
+                 center: bool = True, pad_mode: str = "reflect", frame_pad: Optional[int] = None, magnitude_eps: float = 0.0):
+        if power not in (1, 2):
+            raise ValueError(f"power must be 1.0 (magnitude) or 2.0 (power), got {power!r}")
+        if pad_mode not in ("reflect", "constant"):
+            raise ValueError(f"pad_mode must be 'reflect' or 'constant', got {pad_mode!r}")
+        if frame_pad is None:
+            frame_pad = n_fft // 2 if center else 0
+        if isinstance(frame_pad, bool) or int(frame_pad) != frame_pad or not 0 <= frame_pad <= n_fft // 2:
+            raise ValueError(f"frame_pad must be an integer in [0, n_fft // 2] = [0, {n_fft // 2}], got {frame_pad!r}")
+        if not (math.isfinite(magnitude_eps) and magnitude_eps >= 0.0):
+            raise ValueError(f"magnitude_eps must be finite and >= 0, got {magnitude_eps!r}")
+        if power == 2 and magnitude_eps != 0.0:
+            raise ValueError("magnitude_eps applies to power 1.0 only")
+        self.power, self.pad_mode, self.frame_pad, self.magnitude_eps = float(power), pad_mode, int(frame_pad), float(magnitude_eps)
         device = torch.device(device)
         if device.type != "cuda":
             raise RuntimeError("LogMelFrontend runs on a CUDA device (sm_100a); there is no CPU fallback")
@@ -139,10 +170,12 @@ class LogMelFrontend:
         if tuple(self.window.shape) != (n_fft,) or tuple(self.fb.shape) != (n_fft // 2 + 1, n_mels):
             raise ValueError("window must be [n_fft] and fb [n_fft//2+1, n_mels]")
         self._lib = _lib.load()
+        self._options = _lib.StftOptions(self.frame_pad, {"reflect": _lib.ACB_PAD_REFLECT, "constant": _lib.ACB_PAD_CONSTANT}[pad_mode],
+                                         int(power), self.magnitude_eps)
         handle = ctypes.c_void_p()
-        _lib.check(self._lib.acb_frontend_create(ctypes.byref(handle), device.index, n_fft, hop_length, n_mels,
-                                                 self.window.data_ptr(), self.fb.data_ptr(), self.clamp_min, self.log_kind),
-                   "acb_frontend_create")
+        _lib.check(self._lib.acb_frontend_create_stft(ctypes.byref(handle), device.index, n_fft, hop_length, n_mels, self.window.data_ptr(),
+                                                      self.fb.data_ptr(), self.clamp_min, self.log_kind, ctypes.byref(self._options)),
+                   "acb_frontend_create_stft")
         self._handle = handle
         self.frames_per_tile = int(self._lib.acb_frames_per_tile())
         self._moments_ws: Optional[torch.Tensor] = None
@@ -159,7 +192,7 @@ class LogMelFrontend:
 
     # ------------------------------------------------------------------ helpers
     def frames_for_length(self, length: int) -> int:
-        return frames_for_length(length, self.n_fft, self.hop)
+        return frames_for_length(length, self.n_fft, self.hop, frame_pad=self.frame_pad, pad_mode=self.pad_mode)
 
     def _check_wav(self, wav: torch.Tensor) -> None:
         if not wav.is_cuda or wav.device != self.device:
@@ -275,14 +308,14 @@ class LogMelFrontend:
         Reflection happens at each clip's own ends.  The launch plan and ``frames`` depend on the lengths alone and are kept in
         ``batch.plans``: forwarding a batch again reuses them (the returned ``frames`` tensor is that cached one: treat it as read-only)."""
         self._check_wav(batch.wav)
-        key = (self.n_fft, self.hop, int(pad_multiple))
+        key = (self.n_fft, self.hop, self.frame_pad, self.pad_mode, int(pad_multiple))
         plan = batch.plans.get(key)
         if plan is None:
             lens = np.ascontiguousarray(batch.lengths_host, dtype=np.int64)
             B = int(lens.shape[0])
-            if B and int(lens.min()) <= self.n_fft // 2:
-                self.frames_for_length(int(lens.min()))          # raises like the reference's reflect padding
-            frames = 1 + lens // self.hop
+            if B:
+                self.frames_for_length(int(lens.min()))          # raises like torch.stft's padding for a clip below the minimum
+            frames = 1 + (lens + 2 * self.frame_pad - self.n_fft) // self.hop
             frames = (frames + pad_multiple - 1) // pad_multiple * pad_multiple
             frames_t = torch.from_numpy(frames).to(self.device, non_blocking=True)
             tile_start_t, n_tiles = None, 0
@@ -290,7 +323,8 @@ class LogMelFrontend:
                 # only the frames that exist are visited: per-clip tile counts differ -> host plan (prefix sums) shipped to the device.
                 # For padded outputs the group that stores a clip's last tile also fills the rest of the row with fill_value.
                 tile_start = np.zeros(B + 1, dtype=np.int32)
-                n_tiles = int(self._lib.acb_plan_tiles(lens.ctypes.data, B, self.n_fft, self.hop, 0, tile_start.ctypes.data))
+                n_tiles = int(self._lib.acb_stft_plan_tiles(lens.ctypes.data, B, self.n_fft, self.hop, ctypes.byref(self._options), 0,
+                                                            tile_start.ctypes.data))
                 if n_tiles < 0:
                     _lib.check(n_tiles, "acb_plan_tiles")
                 tile_start_t = torch.from_numpy(tile_start).to(self.device, non_blocking=True)

@@ -68,7 +68,8 @@ int64_t acb_plan_tiles(const int64_t* lengths_host, int32_t n_clips, int n_fft, 
  * window_host[n_fft] and fb_host[(n_fft/2+1) * n_mels] (row-major [freq][mel]) are the fp32 tables the
  * host derived with the reference's torch calls.  This build has kernels for n_fft in {256, 512, 1024} with
  * 1 <= hop <= n_fft and 1 <= n_mels <= 128; anything else (n_fft 128, 400 or 2048, hop 0, hop > n_fft, n_mels 0 or 129)
- * returns ACB_ERR_UNSUPPORTED.  The kernel is chosen from (n_fft, hop) alone:
+ * returns ACB_ERR_UNSUPPORTED.  This call computes torch.stft(center=True, pad_mode="reflect") then power 2 (acb_frontend_create_stft
+ * below takes other definitions), and the kernel is chosen from (n_fft, hop) alone:
  *   - (1024, 256) runs the tuned kernel, which also returns ACB_ERR_UNSUPPORTED for a window without the periodic-Hann
  *     property |w[n + 512] - (1 - w[n])| <= 1e-6 (it computes the second half of the window from the first), a filterbank
  *     with weight on the Nyquist bin, or one with more than 4096 banded weights;
@@ -77,6 +78,39 @@ int64_t acb_plan_tiles(const int64_t* lengths_host, int32_t n_clips, int n_fft, 
  *     its first to its last non-zero bin); a denser filterbank returns ACB_ERR_UNSUPPORTED ("too dense"). */
 int acb_frontend_create(acb_frontend** out, int device, int n_fft, int hop, int n_mels,
                         const float* window_host, const float* fb_host, float clamp_min, int log_kind);
+
+/* Spectrogram definition of a front-end.  acb_frontend_create computes torch.stft(center=True, pad_mode="reflect") then power 2;
+ * these options choose another:
+ *   pad            samples padded on each side before framing, 0 <= pad <= n_fft/2: n_fft/2 is center=True, 0 is center=False and
+ *                  (n_fft - hop)/2 the HiFi-GAN / BigVGAN convention (F.pad by that amount, then torch.stft(center=False));
+ *   pad_mode       ACB_PAD_REFLECT (reflection about the clip's first and last sample) or ACB_PAD_CONSTANT (zeros);
+ *   power          2 (|X|^2) or 1 (magnitude sqrt(|X|^2 + magnitude_eps));
+ *   magnitude_eps  >= 0 and finite, added under the square root when power is 1 (0 for torchaudio, 1e-9 for HiFi-GAN); it must be 0
+ *                  when power is 2.
+ * A clip of L samples has T = 1 + (L + 2 pad - n_fft) / hop frames; it needs L + 2 pad >= n_fft, and L > pad in reflect mode or
+ * L >= 1 in constant mode (the limits torch.stft and F.pad enforce). */
+#define ACB_PAD_REFLECT 0
+#define ACB_PAD_CONSTANT 1
+typedef struct acb_stft_options {
+    int32_t pad;
+    int32_t pad_mode;
+    int32_t power;
+    float magnitude_eps;
+} acb_stft_options;
+
+/* acb_frontend_create with a spectrogram definition; opt == NULL is acb_frontend_create's (pad n_fft/2, reflect, power 2), and
+ * acb_frontend_create is this call with NULL.  With that definition the kernel is chosen from (n_fft, hop) as described above.
+ * With any other, every supported (n_fft, hop), (1024, 256) included, runs the general STFT kernel with its envelope (any window,
+ * weights on any bin).  Options outside the ranges above return ACB_ERR_INVALID (pad, power, eps) or ACB_ERR_UNSUPPORTED (another
+ * pad mode, such as torch's replicate or circular). */
+int acb_frontend_create_stft(acb_frontend** out, int device, int n_fft, int hop, int n_mels, const float* window_host,
+                             const float* fb_host, float clamp_min, int log_kind, const acb_stft_options* opt);
+/* Host-only counterparts of acb_frames_for_length and acb_plan_tiles under a spectrogram definition (opt == NULL: the centred one):
+ * T = 1 + (L + 2 pad - n_fft) / hop, or -1 for a clip below the definition's minimum length or invalid options;
+ * acb_stft_plan_tiles returns ACB_ERR_INVALID with a message in those cases. */
+int64_t acb_stft_frames_for_length(int64_t length, int n_fft, int hop, const acb_stft_options* opt);
+int64_t acb_stft_plan_tiles(const int64_t* lengths_host, int32_t n_clips, int n_fft, int hop, const acb_stft_options* opt,
+                            int64_t frame_capacity, int32_t* tile_start_host);
 int acb_frontend_destroy(acb_frontend* fe);
 /* Which implementation of the fused log-mel kernel acb_logmel_forward launches.  This build has one, with the mel projection
  * on the CUDA cores: 0 = automatic and 1 = CUDA-core mel projection both select it and return ACB_OK.  2 = the warp-specialised
@@ -124,7 +158,8 @@ typedef struct acb_logmel_args {
 
 /* Fused reflect-pad + framing + Hann window + STFT + power + mel projection + clamp + log
  * (+ pad-to-4, + affine normalisation, + per-bin moments): replaces MelExtractor.forward
- * (preprocess/core.py:50-61) and the torchaudio/torch.stft calls below it. */
+ * (preprocess/core.py:50-61) and the torchaudio/torch.stft calls below it.  The padding, framing and power are those of the
+ * handle's spectrogram definition (acb_frontend_create_stft); frame counts follow acb_stft_frames_for_length with its options. */
 int acb_logmel_forward(const acb_frontend* fe, const acb_logmel_args* args, void* stream);
 /* Synchronises `stream` and reports (ACB_ERR_CUDA) whether a sample-tile copy failed to complete inside a launch since the last
  * check: the kernel's barrier waits are bounded so that a faulted copy cannot hang the device; the host-buffer entry points
